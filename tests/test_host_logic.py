@@ -419,14 +419,11 @@ def test_stored_oracle_is_the_plain_oracle_without_rounding():
 
 # ------------------------------------------------------------------ Keras HDF5 checkpoints (spnet_b200/hdf5_min.py)
 def test_hdf5_reader_on_a_file_written_by_libhdf5():
-    """The reader against a GENUINE HDF5 file (MATLAB v7.3 = libhdf5, shipped with scipy's test data: 512-byte user
-    block, superblock 0, symbol-table group, B-tree + local heap, version-1 object header, attribute, dataset)."""
-    import scipy.io
+    """The reader against a GENUINE HDF5 file (MATLAB v7.3 = libhdf5; a copy of scipy's test file
+    scipy/io/matlab/tests/data/testhdf5_7.4_GLNX86.mat, BSD-licensed: 512-byte user block, superblock 0, symbol-table
+    group, B-tree + local heap, version-1 object header, attribute, dataset)."""
     from spnet_b200 import hdf5_min
-    path = os.path.join(os.path.dirname(scipy.io.__file__), "matlab", "tests", "data", "testhdf5_7.4_GLNX86.mat")
-    if not os.path.exists(path):
-        pytest.skip("scipy's HDF5 test file is not installed")
-    r = hdf5_min.Reader(path)
+    r = hdf5_min.Reader(os.path.join(G, "testhdf5_7.4_GLNX86.mat"))
     assert r.base == 512 and list(r.links(r.root)) == ["testdouble"]
     a = r.resolve("testdouble")
     assert r.attrs(a) == {"MATLAB_class": b"double"}
