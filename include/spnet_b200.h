@@ -90,9 +90,6 @@ int spnet_dwconv3x3_bwd_fused(const void* gout, const void* in, const float* k, 
  *      of the K range stores its [M, N] partial product at D + s * slab_stride elements - split-K with a fixed
  *      summation order (spnet_slab_reduce), or a batch of GEMMs stacked along K in ONE launch (the weight gradients
  *      of Xception's 24 identical middle-flow layers, written straight into the flat gradient buffer). ---- */
-/* upper bound on the CTAs of the persistent tensor-core GEMM (0 = one per SM): lowered while a gradient all-reduce
- * is in flight so that NCCL's resident CTAs and the GEMM do not queue behind each other */
-int spnet_gemm_set_cta_cap(int max_ctas);
 int spnet_gemm_bf16(const void* A, long long lda, int a_mn, const void* B, long long ldb, int b_mn, void* D, long long ldd, long long slab_stride, int out_mode, int M, int N, int K, int splits, long long* colstats, cudaStream_t stream);
 int spnet_gemm_simt(const void* A, long long sa_r, long long sa_k, const void* B, long long sb_r, long long sb_k, void* D, long long ldd, long long slab_stride, int dtype, int out_mode, int M, int N, int K, int splits, long long* colstats, cudaStream_t stream);
 

@@ -1,7 +1,6 @@
 // Library-level entry points: version, last error, device check.
 #include "common.cuh"
 #include <stdarg.h>
-#include <stdlib.h>
 #include <string.h>
 
 static thread_local char g_last_error[512] = "";
@@ -20,18 +19,6 @@ int spnet_check_launch(const char* what) {
         return SPNET_ERR_CUDA;
     }
     return SPNET_OK;
-}
-
-bool spnet_pdl_enabled() {
-    static int v = -1;
-    if (v < 0) {
-        // measured on B200 inside the captured step graph: 9.94 ms with PDL edges vs 9.81 ms without (round 1); round 2,
-        // no early trigger: 7.23 vs 7.26 ms (common.cuh)
-        // (kernel boundaries in a graph are already ~1 us), so it is opt-in
-        const char* e = getenv("SPNET_B200_PDL");
-        v = (e && e[0] && e[0] != '0') ? 1 : 0;
-    }
-    return v != 0;
 }
 
 extern "C" {

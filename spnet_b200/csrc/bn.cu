@@ -15,8 +15,6 @@ __global__ void bn_finalize_kernel(long long* __restrict__ stats, double count, 
                                    float* __restrict__ a, float* __restrict__ b, float* __restrict__ save_mean,
                                    float* __restrict__ save_rstd, float* __restrict__ moving_mean,
                                    float* __restrict__ moving_var, int C) {
-    pdl_trigger();
-    pdl_wait();
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= C) return;
     const double mean = stat_get(stats, c) / count;
@@ -139,8 +137,6 @@ __global__ void __launch_bounds__(256, 3) bn_apply_kernel(const T* z, const floa
                                                           const float* __restrict__ b, int act, const T* x, T* out,
                                                           long long rows, int C, int cvb, int krows) {
     constexpr int V = VecN<T>::N, NP = RawVec<T>::NP;
-    pdl_trigger();
-    pdl_wait();
     const int CV = C / V;
     const int cvl = threadIdx.x % cvb, rl = threadIdx.x / cvb;
     const int cv = blockIdx.y * cvb + cvl;
@@ -192,8 +188,6 @@ __global__ void __launch_bounds__(512, 1) bn_bwd_reduce_kernel(T* __restrict__ g
                                                                long long* __restrict__ stats, long long rows, int C,
                                                                int cvb, int krows) {
     constexpr int V = VecN<T>::N, NP = RawVec<T>::NP;
-    pdl_trigger();
-    pdl_wait();
     const int CV = C / V;
     const int cvl = threadIdx.x % cvb, rl = threadIdx.x / cvb;
     const int cv = blockIdx.y * cvb + cvl;
@@ -283,8 +277,6 @@ template <typename T>
 __global__ void __launch_bounds__(512, 1) colstats_kernel(const T* __restrict__ z, long long* __restrict__ stats,
                                                           long long rows, int C, int cvb, int krows) {
     constexpr int V = VecN<T>::N, NP = RawVec<T>::NP;
-    pdl_trigger();
-    pdl_wait();
     const int CV = C / V;
     const int cvl = threadIdx.x % cvb, rl = threadIdx.x / cvb;
     const int cv = blockIdx.y * cvb + cvl;
@@ -340,8 +332,6 @@ __global__ void __launch_bounds__(512, 1) colstats_kernel(const T* __restrict__ 
 __global__ void bn_bwd_finalize_kernel(long long* __restrict__ stats, double count, float* __restrict__ dgamma,
                                        float* __restrict__ dbeta, float* __restrict__ c1, float* __restrict__ c2,
                                        int C) {
-    pdl_trigger();
-    pdl_wait();
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= C) return;
     const double sg = stat_get(stats, c), sgx = stat_get(stats, C + c);
@@ -365,8 +355,6 @@ __global__ void __launch_bounds__(256, 3) bn_bwd_dz_kernel(const T* g, const T* 
                                                            const float* __restrict__ c2, T* out, long long rows,
                                                            int C, int cvb, int krows) {
     constexpr int V = VecN<T>::N, NP = RawVec<T>::NP;
-    pdl_trigger();
-    pdl_wait();
     const int CV = C / V;
     const int cvl = threadIdx.x % cvb, rl = threadIdx.x / cvb;
     const int cv = blockIdx.y * cvb + cvl;
@@ -460,10 +448,9 @@ int spnet_bn_finalize(long long* stats, long long count, const float* gamma, con
                       float* save_rstd, float* moving_mean, float* moving_var, int C, cudaStream_t stream) {
     SPNET_REQUIRE(stats && a && b && save_mean && save_rstd && C > 0 && count > 0, "bn_finalize: bad args");
     SPNET_REQUIRE((moving_mean == nullptr) == (moving_var == nullptr), "bn_finalize: moving stats come in pairs");
-    cudaError_t e = spnet_launch_pdl(bn_finalize_kernel, dim3(ceil_div(C, 128)), dim3(128), 0, stream, 1, stats,
-                                     (double)count, gamma, beta, eps, momentum, unbiased_moving_var, a, b, save_mean,
-                                     save_rstd, moving_mean, moving_var, C);
-    SPNET_REQUIRE(e == cudaSuccess, "bn_finalize: launch: %s", cudaGetErrorString(e));
+    bn_finalize_kernel<<<ceil_div(C, 128), 128, 0, stream>>>(stats, (double)count, gamma, beta, eps, momentum,
+                                                             unbiased_moving_var, a, b, save_mean, save_rstd, moving_mean,
+                                                             moving_var, C);
     return spnet_check_launch("bn_finalize");
 }
 
@@ -484,9 +471,9 @@ int spnet_bn_apply(const void* z, const float* a, const float* b, int act, const
     if (rc) return rc;
     SPNET_REQUIRE(z && a && b && out && act >= 0 && act <= 3, "bn_apply: bad args");
     const ChanGrid cg = chan_grid(C / (dtype == SPNET_BF16 ? 8 : 4), rows, 3);
-    SPNET_DISPATCH_DTYPE(dtype, (spnet_launch_pdl(bn_apply_kernel<T>, cg.grid, dim3(cg.cvb * cg.krows), 0, stream, 1,
-                                                  reinterpret_cast<const T*>(z), a, b, act, reinterpret_cast<const T*>(x),
-                                                  reinterpret_cast<T*>(out), rows, C, cg.cvb, cg.krows)));
+    SPNET_DISPATCH_DTYPE(dtype, (bn_apply_kernel<T><<<cg.grid, cg.cvb * cg.krows, 0, stream>>>(
+                                    reinterpret_cast<const T*>(z), a, b, act, reinterpret_cast<const T*>(x),
+                                    reinterpret_cast<T*>(out), rows, C, cg.cvb, cg.krows)));
     return spnet_check_launch("bn_apply");
 }
 
@@ -499,15 +486,13 @@ int spnet_bn_bwd_reduce(void* g, const void* z, const float* save_mean, const fl
     SPNET_REQUIRE((relu_a == nullptr) == (relu_b == nullptr), "bn_bwd_reduce: mask affine comes in pairs");
     const ChanGrid cg = chan_grid_reduce(C / (dtype == SPNET_BF16 ? 8 : 4), rows);
     if (relu_a) {
-        SPNET_DISPATCH_DTYPE(dtype, (spnet_launch_pdl(bn_bwd_reduce_kernel<T, true>, cg.grid, dim3(cg.cvb * cg.krows), 0,
-                                                      stream, 1, reinterpret_cast<T*>(g), reinterpret_cast<const T*>(z),
-                                                      save_mean, save_rstd, relu_a, relu_b, act, stats, rows, C, cg.cvb,
-                                                      cg.krows)));
+        SPNET_DISPATCH_DTYPE(dtype, (bn_bwd_reduce_kernel<T, true><<<cg.grid, cg.cvb * cg.krows, 0, stream>>>(
+                                        reinterpret_cast<T*>(g), reinterpret_cast<const T*>(z), save_mean, save_rstd,
+                                        relu_a, relu_b, act, stats, rows, C, cg.cvb, cg.krows)));
     } else {
-        SPNET_DISPATCH_DTYPE(dtype, (spnet_launch_pdl(bn_bwd_reduce_kernel<T, false>, cg.grid, dim3(cg.cvb * cg.krows), 0,
-                                                      stream, 1, reinterpret_cast<T*>(g), reinterpret_cast<const T*>(z),
-                                                      save_mean, save_rstd, relu_a, relu_b, act, stats, rows, C, cg.cvb,
-                                                      cg.krows)));
+        SPNET_DISPATCH_DTYPE(dtype, (bn_bwd_reduce_kernel<T, false><<<cg.grid, cg.cvb * cg.krows, 0, stream>>>(
+                                        reinterpret_cast<T*>(g), reinterpret_cast<const T*>(z), save_mean, save_rstd,
+                                        relu_a, relu_b, act, stats, rows, C, cg.cvb, cg.krows)));
     }
     return spnet_check_launch("bn_bwd_reduce");
 }
@@ -518,17 +503,15 @@ int spnet_colstats(const void* z, long long* stats, int dtype, long long rows, i
     if (rc) return rc;
     SPNET_REQUIRE(z && stats, "colstats: null pointer");
     const ChanGrid cg = chan_grid_reduce(C / (dtype == SPNET_BF16 ? 8 : 4), rows);
-    SPNET_DISPATCH_DTYPE(dtype, (spnet_launch_pdl(colstats_kernel<T>, cg.grid, dim3(cg.cvb * cg.krows), 0, stream, 1,
-                                                  reinterpret_cast<const T*>(z), stats, rows, C, cg.cvb, cg.krows)));
+    SPNET_DISPATCH_DTYPE(dtype, (colstats_kernel<T><<<cg.grid, cg.cvb * cg.krows, 0, stream>>>(
+                                    reinterpret_cast<const T*>(z), stats, rows, C, cg.cvb, cg.krows)));
     return spnet_check_launch("colstats");
 }
 
 int spnet_bn_bwd_finalize(long long* stats, long long count, float* dgamma, float* dbeta, float* c1, float* c2,
                           int C, cudaStream_t stream) {
     SPNET_REQUIRE(stats && c1 && c2 && C > 0 && count >= 0, "bn_bwd_finalize: bad args");
-    cudaError_t e = spnet_launch_pdl(bn_bwd_finalize_kernel, dim3(ceil_div(C, 128)), dim3(128), 0, stream, 1, stats,
-                                     (double)count, dgamma, dbeta, c1, c2, C);
-    SPNET_REQUIRE(e == cudaSuccess, "bn_bwd_finalize: launch: %s", cudaGetErrorString(e));
+    bn_bwd_finalize_kernel<<<ceil_div(C, 128), 128, 0, stream>>>(stats, (double)count, dgamma, dbeta, c1, c2, C);
     return spnet_check_launch("bn_bwd_finalize");
 }
 
@@ -540,9 +523,9 @@ int spnet_bn_bwd_dz(const void* g, const void* z, const float* a, const float* s
     if (rc) return rc;
     SPNET_REQUIRE(g && z && a && save_mean && save_rstd && c1 && c2 && out, "bn_bwd_dz: null pointer");
     const ChanGrid cg = chan_grid(C / (dtype == SPNET_BF16 ? 8 : 4), rows, 3);
-    SPNET_DISPATCH_DTYPE(dtype, (spnet_launch_pdl(bn_bwd_dz_kernel<T>, cg.grid, dim3(cg.cvb * cg.krows), 0, stream, 1,
-                                                  reinterpret_cast<const T*>(g), reinterpret_cast<const T*>(z), a, save_mean,
-                                                  save_rstd, c1, c2, reinterpret_cast<T*>(out), rows, C, cg.cvb, cg.krows)));
+    SPNET_DISPATCH_DTYPE(dtype, (bn_bwd_dz_kernel<T><<<cg.grid, cg.cvb * cg.krows, 0, stream>>>(
+                                    reinterpret_cast<const T*>(g), reinterpret_cast<const T*>(z), a, save_mean, save_rstd,
+                                    c1, c2, reinterpret_cast<T*>(out), rows, C, cg.cvb, cg.krows)));
     return spnet_check_launch("bn_bwd_dz");
 }
 

@@ -120,53 +120,6 @@ __device__ __forceinline__ double stat_get(const long long* acc, long long i) {
 }
 __device__ __forceinline__ void stat_clear(long long* acc, long long i) { acc[2 * i] = 0; acc[2 * i + 1] = 0; }
 
-// ---- programmatic dependent launch (PDL) ------------------------------------------------------
-// The step is a chain of ~400 short kernels; with PDL (opt-in: SPNET_B200_PDL=1) a kernel's CTAs are
-// scheduled and run their prologue (barrier init, TMEM allocation, index math) while the previous
-// kernel drains, and block in pdl_wait() until that kernel has completed and flushed its memory.
-// Without the launch attribute both instructions are no-ops. Rules used throughout:
-// pdl_trigger() first thing, pdl_wait() before the FIRST global-memory access of any kind.
-// Measured on the captured step (round 2, 7.26 ms): attribute + early trigger 7.49 ms (the dependent's CTAs squat on
-// the SMs while the primary still runs), attribute without an explicit trigger 7.23 ms (noise) - so the trigger is
-// compiled out unless SPNET_PDL_EARLY_TRIGGER is defined, and the attribute stays opt-in.
-__device__ __forceinline__ void pdl_trigger() {
-#ifdef SPNET_PDL_EARLY_TRIGGER
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-#endif
-}
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-
-bool spnet_pdl_enabled();
-
-// Launch with the programmatic-stream-serialization attribute (and an optional cluster size).
-// Only for kernels that follow the rules above.
-template <typename... KArgs, typename... Args>
-static inline cudaError_t spnet_launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem,
-                                           cudaStream_t stream, int cluster, Args... args) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid;
-    cfg.blockDim = block;
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[2];
-    int na = 0;
-    if (cluster > 1) {
-        attr[na].id = cudaLaunchAttributeClusterDimension;
-        attr[na].val.clusterDim.x = cluster;
-        attr[na].val.clusterDim.y = 1;
-        attr[na].val.clusterDim.z = 1;
-        ++na;
-    }
-    if (spnet_pdl_enabled()) {
-        attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[na].val.programmaticStreamSerializationAllowed = 1;
-        ++na;
-    }
-    cfg.attrs = attr;
-    cfg.numAttrs = na;
-    return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
-}
-
 // cudaFuncSetAttribute (the dynamic shared-memory opt-in) is per DEVICE: one flag per device for a launcher's
 // "configured once" state. Returns true the first time it is called for the current device with these flags.
 static inline bool spnet_first_use_on_device(bool (&flags)[64]) {

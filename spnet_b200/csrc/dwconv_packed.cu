@@ -19,7 +19,6 @@
 // TMA map fills the halo with NaN, which the affine keeps and fmaxf(NaN, 0) turns into the exact
 // zero the padding needs — no per-element masking in the hot loop.
 #include "tma.cuh"
-#include <stdlib.h>
 
 namespace {
 
@@ -151,9 +150,7 @@ dw3x3_fwd_packed_kernel(const __grid_constant__ CUtensorMap tm_in, const float* 
         }
         mbar_fence_init();
     }
-    pdl_trigger();
     __syncthreads();
-    pdl_wait();  // everything below touches global memory
 
     // Producer duty: lane 0 of warp 0 keeps S-1 tiles in flight. Stage (it-1)%S is refilled at the
     // start of tile `it`, once every warp has released it (empty barrier).
@@ -304,9 +301,7 @@ dw3x3_bwd_packed_kernel(const __grid_constant__ CUtensorMap tm_g, const __grid_c
         }
         mbar_fence_init();
     }
-    pdl_trigger();
     __syncthreads();
-    pdl_wait();  // everything below touches global memory
 
     auto issue = [&](int tile, int s) {
         const TileCoord t = tile_coord(tile, tiles_w, tiles_h, TH, TW);
@@ -510,27 +505,16 @@ Tiling pick_tiling(int kind, int dtype, int B, int H, int W, int C) {
     const int ncons = t.TW / t.NC;
     t.threads = ncons * 32;
     // resident CTAs per SM this kernel is sized for (registers: <= 64K / threads per thread)
-    int ctas = kind == 0 ? (t.TW == 32 ? 2 : (t.TW == 16 ? 4 : 6)) : (t.TW == 32 ? 1 : (t.TW == 16 ? 2 : 3));
-    int force_th = 0, force_s = 0;
-    if (const char* e = getenv("SPNET_DW_TUNE")) {  // "ctas,TH,S" (0 = automatic): tuning sweeps only
-        int a = 0, b = 0, c = 0;
-        if (sscanf(e, "%d,%d,%d", &a, &b, &c) == 3) {
-            if (a > 0) ctas = a;
-            force_th = b;
-            force_s = c;
-        }
-    }
+    const int ctas = kind == 0 ? (t.TW == 32 ? 2 : (t.TW == 16 ? 4 : 6)) : (t.TW == 32 ? 1 : (t.TW == 16 ? 2 : 3));
     const size_t budget = (size_t)216 * 1024 / ctas - 1024;
     double best = 1e30;
     t.TH = 0;
     const int cands[] = {2, 3, 4, 6, 8, 12, 16};
     for (int th : cands) {
         if (th > H && th != 2) continue;
-        if (force_th && th != force_th) continue;
         const size_t stage = (size_t)(th + 2) * (t.TW + 2) * pix + (kind ? (size_t)th * t.TW * pix * (kind == 2 ? 2 : 1) : 0);
         int S = (int)(budget / stage);
         if (S > MAX_STAGES) S = MAX_STAGES;
-        if (force_s && S > force_s) S = force_s;
         if (S < 2) continue;
         const long long n = (long long)B * ceil_div(H, th) * t.tiles_w;
         long long gx = ((long long)spnet_num_sms() * ctas) / t.chunks;
@@ -562,9 +546,8 @@ int launch_fwd_inst(const CUtensorMap& tm, const float* k, const float* a, const
             return SPNET_ERR_CUDA;
         }
     }
-    cudaError_t e = spnet_launch_pdl(kern, dim3(t.grid_x, t.chunks), dim3(t.threads), t.smem, stream, 1, tm, k, a, b, y, B,
-                                     H, W, C, t.TH, t.TW, t.tiles_h, t.tiles_w, t.S);
-    SPNET_REQUIRE(e == cudaSuccess, "dwconv3x3_fwd: launch: %s", cudaGetErrorString(e));
+    kern<<<dim3(t.grid_x, t.chunks), t.threads, t.smem, stream>>>(tm, k, a, b, y, B, H, W, C, t.TH, t.TW, t.tiles_h,
+                                                                  t.tiles_w, t.S);
     return spnet_check_launch("dw3x3_fwd");
 }
 
@@ -598,10 +581,8 @@ int launch_bwd_inst(const CUtensorMap& tg, const CUtensorMap& tx, const CUtensor
             return SPNET_ERR_CUDA;
         }
     }
-    cudaError_t e = spnet_launch_pdl(kern, dim3(t.grid_x, t.chunks), dim3(t.threads), t.smem, stream, 1, tg, tx, ta, k, a,
-                                     b, mean, rstd, stats, sadd, gin, dk, dk_acc, B, H, W, C, t.TH, t.TW, t.tiles_h, t.tiles_w,
-                                     t.S);
-    SPNET_REQUIRE(e == cudaSuccess, "dwconv3x3_bwd_fused: launch: %s", cudaGetErrorString(e));
+    kern<<<dim3(t.grid_x, t.chunks), t.threads, t.smem, stream>>>(tg, tx, ta, k, a, b, mean, rstd, stats, sadd, gin, dk,
+                                                                  dk_acc, B, H, W, C, t.TH, t.TW, t.tiles_h, t.tiles_w, t.S);
     return spnet_check_launch("dw3x3_bwd_fused");
 }
 

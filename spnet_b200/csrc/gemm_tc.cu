@@ -19,7 +19,6 @@
 // Epilogue modes: store bf16, store fp32, atomic-add fp32 (split-K); optional fused
 // per-column sum / sum-of-squares (BatchNorm batch statistics) accumulated in fp64.
 #include "tma.cuh"
-#include <stdlib.h>
 
 #ifdef SPNET_GEMM_TRACE
 // diagnostic build only (tests/micro/gemm_trace.py): per-CTA cycle stamps of the kernel's phases
@@ -133,38 +132,6 @@ __device__ __forceinline__ void umma_commit_mc(uint32_t bar, uint16_t cta_mask, 
         "h"(cta_mask), "r"(leader)
         : "memory");
 }
-// ---- CTA-pair MMA (cta_group::2): one thread of the pair's EVEN CTA issues a 256-row MMA over both CTAs' shared memory
-// (A: 128 rows from each CTA; B: half of the N columns from each), each CTA's TMEM receives its 128 rows. Both CTAs'
-// TMA loads complete on the even CTA's "full" barrier: in the shared::cluster window bit 24 of a CTA-local address
-// selects the CTA of the pair, clearing it addresses the even CTA (cute::Sm100MmaPeerBitMask).
-constexpr uint32_t kPeerBitMask = 0xFEFFFFFFu;
-__device__ __forceinline__ void umma_bf16_2sm(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
-                                              uint32_t accumulate, uint32_t leader) {
-    asm volatile(
-        "{\n\t.reg .pred p, q;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "setp.ne.b32 q, %5, 0;\n\t"
-        "@q tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate), "r"(leader)
-        : "memory");
-}
-__device__ __forceinline__ void umma_commit_2sm(uint32_t bar, uint32_t leader) {  // arrives on `bar` in BOTH CTAs
-    asm volatile(
-        "{\n\t.reg .pred q;\n\t"
-        "setp.ne.b32 q, %1, 0;\n\t"
-        "@q tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %2;\n\t}" ::"r"(bar),
-        "r"(leader), "h"((uint16_t)3)
-        : "memory");
-}
-__device__ __forceinline__ void tma_load_2d_2sm(uint32_t dst, const CUtensorMap* map, uint32_t bar_even_cta, int c0, int c1) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-        ::"r"(dst), "l"(map), "r"(bar_even_cta), "r"(c0), "r"(c1)
-        : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t bar_cluster_addr) {
-    asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(bar_cluster_addr) : "memory");
-}
 __device__ __forceinline__ void cluster_sync_all() {
     asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
     asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
@@ -189,32 +156,28 @@ __device__ __forceinline__ void epi_bar_sync() {  // named barrier 1: the four e
 // CL = 2: CTA pairs (thread-block cluster of 2 along M). Both CTAs of a pair work on the same
 // n-tile and k-range with adjacent m-tiles; each loads its own A tile and HALF of the shared B tile,
 // multicast by TMA into both CTAs' shared memory, so the pair reads B from L2 once.
-// P2 (with CL = 2): the pair runs ONE cta_group::2 MMA per k-step instead of one cta_group::1 MMA per CTA over a
-// multicast copy of B: each CTA keeps only its half of the B tile (16 KB instead of 32 KB per stage: six ring stages
-// instead of four, a third less shared-memory traffic per k-block).
 // BRES (CONV 1, one n-tile, few k-blocks): the whole B operand (the convolution's weights, <= 72 KB) is loaded into
 // shared memory ONCE per CTA and stays there for all of its pixel tiles; the ring then carries A boxes only. Narrow
 // convolutions are bound by L2 -> SM delivery (a 128x64x64 k-block is 0.09 us of MMA), and re-fetching the weights for
 // every tile was a third of that traffic.
-template <int BN, bool A_MN, bool B_MN, int STAGES, int CL, int CONV, bool P2 = false, bool BRES = false>
+template <int BN, bool A_MN, bool B_MN, int STAGES, int CL, int CONV, bool BRES = false>
 __global__ void __launch_bounds__(kThreads, 1) gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA,
                                                               const __grid_constant__ CUtensorMap tmB,
                                                               const __grid_constant__ CUtensorMap tmD, GemmEpi epi,
                                                               int M, int N, int K, int kb_per_split, int tiles_m,
                                                               int tiles_n, int n_units, ConvGeom cg) {
     static_assert(CONV == 0 || CL == 1, "convolution modes run without CTA pairs");
-    static_assert(!P2 || CL == 2, "pair MMA needs the CTA pair");
     constexpr uint32_t A_BYTES = BM * BK * 2;
-    constexpr uint32_t B_BYTES = (P2 ? BN / 2 : BN) * BK * 2;  // P2: this CTA's half of the N columns
+    constexpr uint32_t B_BYTES = BN * BK * 2;
     static_assert(!BRES || (CONV == 1 && CL == 1), "resident B is a mode of the forward-type implicit convolution");
     constexpr uint32_t STAGE_BYTES = A_BYTES + (BRES ? 0u : B_BYTES);
     // TMA boxes per k-block issued by THIS CTA: A is one 128-row box (K-major) or BM/64 atoms (MN-major);
     // B one box (K-major) or BN/64 atoms (MN-major), of which a CTA of a pair issues 1/CL (multicast)
     constexpr int NA_BOX = (A_MN || CONV == 2) ? BM / 64 : 1;
-    constexpr int NB_BOX = (B_MN || CONV == 2) ? BN / 64 / CL : 1;  // (P2: BN / 2 columns = BN / 64 / 2 atoms)
+    constexpr int NB_BOX = (B_MN || CONV == 2) ? BN / 64 / CL : 1;
     constexpr int N_BOX = NA_BOX + NB_BOX;
     constexpr uint32_t A_BOX_BYTES = A_BYTES / NA_BOX;
-    constexpr uint32_t B_BOX_BYTES = P2 ? B_BYTES / NB_BOX : B_BYTES / (NB_BOX * CL);  // what one of this CTA's B boxes lands
+    constexpr uint32_t B_BOX_BYTES = B_BYTES / (NB_BOX * CL);  // what one of this CTA's B boxes lands
     extern __shared__ uint8_t smem_raw[];
     // SWIZZLE_128B tiles need 1024-byte alignment
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
@@ -251,46 +214,33 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_tc_kernel(const __grid_const
     if (threadIdx.x == 0) {
         for (int s = 0; s < STAGES; ++s) {
             mbar_init(full0 + 8 * s, 1);  // one arrive.expect_tx per k-block
-            mbar_init(empty0 + 8 * s, P2 ? 1 : CL);  // every CTA's MMAs (P2: the pair's MMAs) must have consumed the stage
+            mbar_init(empty0 + 8 * s, CL);  // every CTA's MMAs must have consumed the stage
         }
         mbar_init(bres_bar, 1);
         for (int a = 0; a < 2; ++a) {
             mbar_init(tfull0 + 8 * a, 1);
-            mbar_init(tempty0 + 8 * a, P2 ? 2 * kEpiWarps : kEpiWarps);  // one arrive per epilogue warp (P2: of both CTAs)
+            mbar_init(tempty0 + 8 * a, kEpiWarps);  // one arrive per epilogue warp
         }
         mbar_fence_init();
     }
     if (warp == 1) {
-        if (P2) {  // the same warp of both CTAs, same destination offset
-            asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(
-                             smem_u32(&tmem_base_holder)),
-                         "r"((uint32_t)(2 * BN))
-                         : "memory");
-            asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-        } else {
-            asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(
-                             smem_u32(&tmem_base_holder)),
-                         "r"((uint32_t)(2 * BN))
-                         : "memory");
-            asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-        }
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_holder)),
+                     "r"((uint32_t)(2 * BN))
+                     : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
     }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    pdl_trigger();
     if (CL > 1) cluster_sync_all(); else __syncthreads();  // barrier inits visible cluster-wide
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     const uint32_t tmem_base = tmem_base_holder;
     if (threadIdx.x == 0) TRACE(1);
-    pdl_wait();  // the set-up above overlapped the previous kernel's tail; global memory from here on
     // with CL = 2, tiles_m counts m-tile PAIRS; this CTA owns m-tile 2*pair + rank
 
     if (warp == 0) {
         // ---------------- TMA producer ----------------
         // every box of a k-block is issued by one elected thread, which announces the stage's bytes on its full
         // barrier (B boxes of a CTA pair land in both CTAs: each CTA expects CL x its own)
-        // (P2: the even CTA announces the bytes landing in BOTH CTAs on its barrier; the odd CTA only issues its loads)
-        constexpr uint32_t my_bytes = P2 ? 2 * (A_BYTES + B_BYTES)
-                                         : NA_BOX * A_BOX_BYTES + (BRES ? 0u : NB_BOX * B_BOX_BYTES * CL);
+        constexpr uint32_t my_bytes = NA_BOX * A_BOX_BYTES + (BRES ? 0u : NB_BOX * B_BOX_BYTES * CL);
         uint32_t g0 = 0;  // k-blocks of the units before this one
         const uint32_t issuer = elect_one();
         if (BRES && issuer && cluster_id < n_units) {  // the weights, once: k-block kb = (tap, channel block)
@@ -366,23 +316,9 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_tc_kernel(const __grid_const
                     const uint32_t sa = smem_u32(smem + (size_t)s * STAGE_BYTES);
                     const uint32_t sb = sa + A_BYTES;
                     const uint32_t bar = full0 + 8 * s;
-                    if (!P2 || crank == 0) mbar_expect_tx(bar, my_bytes);
-                    if (P2) {
-                        const uint32_t fbar = bar & kPeerBitMask;  // the even CTA's barrier
-                        const int nh = n0 + (int)crank * (BN / 2);
+                    mbar_expect_tx(bar, my_bytes);
 #pragma unroll
-                        for (int j = 0; j < NA_BOX; ++j) {
-                            if (A_MN) tma_load_2d_2sm(sa + j * (BK * 128), &tmA, fbar, m0 + 64 * j, k0);
-                            else tma_load_2d_2sm(sa, &tmA, fbar, k0, m0);
-                        }
-#pragma unroll
-                        for (int jb = 0; jb < NB_BOX; ++jb) {
-                            if (B_MN) tma_load_2d_2sm(sb + jb * (BK * 128), &tmB, fbar, nh + 64 * jb, k0);
-                            else tma_load_2d_2sm(sb, &tmB, fbar, k0, nh);
-                        }
-                    }
-#pragma unroll
-                    for (int j = 0; j < (P2 ? 0 : BRES ? NA_BOX : N_BOX); ++j) {
+                    for (int j = 0; j < (BRES ? NA_BOX : N_BOX); ++j) {
                         if (j < NA_BOX) {
                             if (CONV == 1) tma_load_4d(sa, &tmA, bar, kA, ax, ay, aimg);
                             else if (CONV == 2) tma_load_4d(sa + j * (BK * 128), &tmA, bar, m0 + 64 * j, ax, ay, aimg);
@@ -413,12 +349,11 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_tc_kernel(const __grid_const
             }
             g0 += (uint32_t)nkb;
         }
-    } else if (warp == 1 && (!P2 || crank == 0)) {
-        // ---------------- MMA issuer (P2: of the pair, in its even CTA) ----------------
-        // instruction descriptor: fp32 accumulate, bf16 x bf16, majors, N>>3, M>>4 (P2: 256 rows over the two CTAs)
+    } else if (warp == 1) {
+        // ---------------- MMA issuer ----------------
+        // instruction descriptor: fp32 accumulate, bf16 x bf16, majors, N>>3, M>>4
         const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((A_MN ? 1u : 0u) << 15) |
-                               ((B_MN ? 1u : 0u) << 16) | ((uint32_t)(BN >> 3) << 17) |
-                               ((uint32_t)((P2 ? 2 * BM : BM) >> 4) << 24);
+                               ((B_MN ? 1u : 0u) << 16) | ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
         // Shared-memory descriptors differ between stages / k-steps only in the 14-bit address field of
         // the low word: build the constant parts once so the per-MMA issue cost is a couple of adds.
         const uint32_t a_lbo = A_MN ? (uint32_t)(BK * 128) : 0u, b_lbo = B_MN ? (uint32_t)(BK * 128) : 0u;
@@ -451,16 +386,12 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_tc_kernel(const __grid_const
                     for (int k = 0; k < BK / UMMA_K; ++k) {
                         const uint64_t ad = ((uint64_t)desc_hi << 32) | (uint64_t)(a_lo + k * A_KSTEP);
                         const uint64_t bd = ((uint64_t)desc_hi << 32) | (uint64_t)(b_lo + k * B_KSTEP);
-                        if (P2) umma_bf16_2sm(tacc, ad, bd, idesc, (i > 0 || k > 0) ? 1u : 0u, 1u);
-                        else umma_bf16(tacc, ad, bd, idesc, (i > 0 || k > 0) ? 1u : 0u, 1u);
+                        umma_bf16(tacc, ad, bd, idesc, (i > 0 || k > 0) ? 1u : 0u, 1u);
                     }
                     // frees the smem stage (in every CTA of the cluster) when these MMAs retire
-                    if (P2) umma_commit_2sm(empty0 + 8 * s, 1u);
-                    else if (CL > 1) umma_commit_mc(empty0 + 8 * s, kMask, 1u);
+                    if (CL > 1) umma_commit_mc(empty0 + 8 * s, kMask, 1u);
                     else umma_commit(empty0 + 8 * s, 1u);
-                    if (i == nkb - 1) {  // accumulator complete (P2: in both CTAs' TMEM)
-                        if (P2) umma_commit_2sm(tfull0 + 8 * as, 1u); else umma_commit(tfull0 + 8 * as, 1u);
-                    }
+                    if (i == nkb - 1) umma_commit(tfull0 + 8 * as, 1u);  // accumulator complete
                     if (i == nkb - 1) { if (u == 0) TRACE(3); TRACE(4); }
                 }
                 __syncwarp();
@@ -643,10 +574,7 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_tc_kernel(const __grid_const
             // accumulator fully read: hand it back to the MMA warp
             asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
             __syncwarp();
-            if (e_leader) {
-                if (P2) mbar_arrive_cluster((tempty0 + 8 * as) & kPeerBitMask);  // the even CTA's MMA warp waits for both
-                else mbar_arrive(tempty0 + 8 * as);
-            }
+            if (e_leader) mbar_arrive(tempty0 + 8 * as);
             if (threadIdx.x == 64) { if (u == 0) TRACE(7); TRACE(9); }
             if (epi.colstats) {
                 // partial sums of this unit are visible after the barrier; the buffer alternates with the
@@ -669,20 +597,13 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_tc_kernel(const __grid_const
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     if (CL > 1) cluster_sync_all(); else __syncthreads();  // no CTA may exit while its peer still multicasts into it
     if (threadIdx.x == 0) { TRACE(11); TRACE_G(12); }
-    if (warp == 1) {
-        if (P2)
-            asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)(2 * BN))
-                         : "memory");
-        else
-            asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)(2 * BN))
-                         : "memory");
-    }
+    if (warp == 1)
+        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)(2 * BN)) : "memory");
 }
 
 // ---------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------
-int g_cta_cap = 0;  // 0 = every SM
 constexpr int kMaxResidentKb = 9;  // resident-B convolutions: at most 9 k-blocks of 64-wide weights (72 KB)
 // operand with `rows` along M/N and `kdim` along K; ld in elements
 int make_operand_map(CUtensorMap* map, const void* ptr, long long rows, long long kdim, long long ld, bool mn_major,
@@ -714,23 +635,18 @@ int make_operand_map(CUtensorMap* map, const void* ptr, long long rows, long lon
 }
 
 // CONV 0: tiles_m_conv / ntaps unused. CONV 1: tiles_m_conv = number of pixel tiles. CONV 2: ntaps = cg.ntaps.
-template <int BN, bool A_MN, bool B_MN, int CL, int CONV = 0, bool P2 = false, bool BRES = false>
+template <int BN, bool A_MN, bool B_MN, int CL, int CONV = 0, bool BRES = false>
 int launch_gemm(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& td, GemmEpi epi, int M, int N, int K,
                 int splits, cudaStream_t stream, ConvGeom cg = ConvGeom(), int tiles_m_conv = 0) {
     // BN = 128: one ring stage traded for the second staging box; BN = 64 (narrow convolutions): deep ring
-    // (pair MMA: a CTA holds half of the B tile - six stages in the space of four)
-    constexpr int STAGES = P2 ? 6 : BN <= 64 ? 7 : (BN <= 128) ? 5 : 4;
+    constexpr int STAGES = BN <= 64 ? 7 : (BN <= 128) ? 5 : 4;
     // (resident B: the ring carries A only; the weights take ceil(K/64) tiles of BN x 64 next to it)
-    const size_t smem = (size_t)STAGES * (BM * BK * 2 + (BRES ? 0 : (P2 ? BN / 2 : BN) * BK * 2)) +
+    const size_t smem = (size_t)STAGES * (BM * BK * 2 + (BRES ? 0 : BN * BK * 2)) +
                         (BRES ? (size_t)((K + BK - 1) / BK) * BN * BK * 2 : 0) + 1024 + kEpiWarps * 2048 * (BN <= 128 ? 2 : 1);
-    auto kern = gemm_tc_kernel<BN, A_MN, B_MN, STAGES, CL, CONV, P2, BRES>;
+    auto kern = gemm_tc_kernel<BN, A_MN, B_MN, STAGES, CL, CONV, BRES>;
     // per (instantiation, device): the dynamic shared-memory opt-in is a per-device function attribute
     static bool configured[64] = {};
-    static int num_sms_dev[64] = {};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    dev &= 63;
-    if (!configured[dev]) {
+    if (spnet_first_use_on_device(configured)) {
         // (resident B: the size depends on K; opt in to the largest this mode is dispatched with)
         const size_t smem_max = BRES ? (size_t)STAGES * BM * BK * 2 + (size_t)kMaxResidentKb * BN * BK * 2 + 1024 + kEpiWarps * 2048 * 2 : smem;
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_max);
@@ -738,14 +654,7 @@ int launch_gemm(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap&
             spnet_set_error("gemm_bf16: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
             return SPNET_ERR_CUDA;
         }
-        cudaDeviceGetAttribute(&num_sms_dev[dev], cudaDevAttrMultiProcessorCount, dev);
-        configured[dev] = true;
     }
-    // persistent grid: one CTA per SM, or fewer when the caller reserves SMs for a concurrent collective
-    // (spnet_gemm_set_cta_cap: NCCL's CTAs hold their SMs for the whole all-reduce, and a 148-CTA persistent GEMM
-    // would leave its last CTAs waiting for them)
-    int num_sms = num_sms_dev[dev];
-    if (g_cta_cap > 0 && g_cta_cap < num_sms) num_sms = g_cta_cap;
     const int total_kb = (K + BK - 1) / BK;
     if (splits < 1) splits = 1;
     if (splits > total_kb) splits = total_kb;
@@ -758,10 +667,22 @@ int launch_gemm(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap&
         spnet_set_error("gemm_bf16: too many tiles");
         return SPNET_ERR_ARG;
     }
-    const int max_clusters = num_sms / CL;
+    // persistent grid: one CTA per SM; CL > 1 launches the grid as clusters of CL CTAs (the CTA pairs)
+    const int max_clusters = spnet_num_sms() / CL;
     const int grid = (int)(units < max_clusters ? units : max_clusters) * CL;
-    cudaError_t e = spnet_launch_pdl(kern, dim3(grid), dim3(kThreads), smem, stream, CL, ta, tb, td, epi, M, N, K, kbps,
-                                     tiles_m, tiles_n, (int)units, cg);
+    cudaLaunchAttribute cluster = {};
+    cluster.id = cudaLaunchAttributeClusterDimension;
+    cluster.val.clusterDim.x = CL;
+    cluster.val.clusterDim.y = 1;
+    cluster.val.clusterDim.z = 1;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(grid);
+    cfg.blockDim = dim3(kThreads);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = stream;
+    cfg.attrs = &cluster;
+    cfg.numAttrs = CL > 1 ? 1 : 0;
+    cudaError_t e = cudaLaunchKernelEx(&cfg, kern, ta, tb, td, epi, M, N, K, kbps, tiles_m, tiles_n, (int)units, cg);
     if (e != cudaSuccess) {
         spnet_set_error("gemm_bf16: launch: %s", cudaGetErrorString(e));
         return SPNET_ERR_CUDA;
@@ -778,13 +699,6 @@ int spnet_gemm_trace_read(unsigned long long* host) {
     return cudaMemcpyFromSymbol(host, g_gemm_trace, sizeof(g_gemm_trace)) == cudaSuccess ? 0 : 1;
 }
 #endif
-
-// Upper bound on the CTAs of the persistent tensor-core GEMM (0 = one per SM). The data-parallel engine lowers it while
-// a gradient all-reduce is in flight so that NCCL's resident CTAs and the GEMM never queue behind each other.
-int spnet_gemm_set_cta_cap(int max_ctas) {
-    g_cta_cap = max_ctas > 0 ? max_ctas : 0;
-    return SPNET_OK;
-}
 
 // D[M,N] (op)= A[M,K] * B[K,N], bf16 operands, fp32 accumulation in TMEM.
 //   a_mn / b_mn : 0 = K-major (ptr[r*ld + k]), 1 = MN-major (ptr[k*ld + r])
@@ -810,19 +724,19 @@ int spnet_gemm_bf16(const void* A, long long lda, int a_mn, const void* B, long 
     SPNET_REQUIRE(out_mode >= 0 && out_mode <= 3, "gemm_bf16: bad out_mode %d", out_mode);
     SPNET_REQUIRE(out_mode != OUT_BF16 || (N % 8 == 0 && ldd % 8 == 0), "gemm_bf16: bf16 output needs N, ldd %% 8 == 0");
     SPNET_REQUIRE(out_mode == OUT_BF16 || ldd % 4 == 0, "gemm_bf16: fp32 output needs ldd %% 4 == 0");
-    static const bool force_narrow = getenv("SPNET_GEMM_FORCE_NARROW") != nullptr, no_cluster = getenv("SPNET_B200_NO_CLUSTER") != nullptr;
-    const bool wide_ = N >= 512 && !force_narrow, pair_ = wide_ && M > BM && !no_cluster;
+    // 128x256 tiles when N is wide: one A tile then feeds 256 output columns, which cuts the
+    // L2->SM operand traffic per FLOP by a third (the 128x128 kernel is L2-bandwidth bound).
+    const bool wide = N >= 512;
+    // CTA pairs (B tile multicast) when there are at least two m-tiles to pair up
+    const bool pair = wide && M > BM;
     if (splits <= 0) {
         // auto split-K (atomic output only): fill the SMs (or SM pairs) once without spilling into a
         // second, nearly empty round; keep at least 4 k-blocks per split
         splits = 1;
         if (out_mode == OUT_ATOMIC_F32) {
-            const int bn = wide_ ? 256 : 128, cl = pair_ ? 2 : 1;
+            const int bn = wide ? 256 : 128, cl = pair ? 2 : 1;
             const long long tiles = (long long)(((M + BM - 1) / BM + cl - 1) / cl) * ((N + bn - 1) / bn);
-            int nsm = 148;
-            { int d_ = 0; cudaGetDevice(&d_); cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, d_); }
-            if (g_cta_cap > 0 && g_cta_cap < nsm) nsm = g_cta_cap;
-            const long long slots = nsm / cl;
+            const long long slots = spnet_num_sms() / cl;
             long long sp = tiles >= slots ? 1 : slots / tiles;
             const long long kb = (K + BK - 1) / BK;
             if (sp > kb / 4) sp = kb / 4;
@@ -839,11 +753,6 @@ int spnet_gemm_bf16(const void* A, long long lda, int a_mn, const void* B, long 
         n_slabs = (kb + kbps - 1) / kbps;
     }
     SPNET_REQUIRE(!(colstats && splits > 1), "gemm_bf16: column statistics are not defined for split-K partials");
-    // 128x256 tiles when N is wide: one A tile then feeds 256 output columns, which cuts the
-    // L2->SM operand traffic per FLOP by a third (the 128x128 kernel is L2-bandwidth bound).
-    const bool wide = wide_;
-    // CTA pairs (B tile multicast) when there are at least two m-tiles to pair up
-    const bool pair = pair_;
     CUtensorMap ta, tb;
     int rc = make_operand_map(&ta, A, M, K, lda, a_mn != 0, BM);
     if (rc) return rc;
@@ -863,30 +772,23 @@ int spnet_gemm_bf16(const void* A, long long lda, int a_mn, const void* B, long 
         SPNET_REQUIRE(r == CUDA_SUCCESS, "gemm_bf16: cuTensorMapEncodeTiled (output) failed (%d) M=%d N=%d ldd=%lld", (int)r, M, N, ldd);
     }
     GemmEpi epi = {D, ldd, out_mode, 0, colstats};
-#define SPNET_GEMM_DISPATCH(BN_, CL_, P2_)                                                                                  \
+#define SPNET_GEMM_DISPATCH(BN_, CL_)                                                                                       \
     do {                                                                                                                    \
         if (a_mn) {                                                                                                         \
-            if (b_mn) return launch_gemm<BN_, true, true, CL_, 0, P2_>(ta, tb, td, epi, M, N, K, splits, stream);          \
-            return launch_gemm<BN_, true, false, CL_, 0, P2_>(ta, tb, td, epi, M, N, K, splits, stream);                   \
+            if (b_mn) return launch_gemm<BN_, true, true, CL_>(ta, tb, td, epi, M, N, K, splits, stream);                   \
+            return launch_gemm<BN_, true, false, CL_>(ta, tb, td, epi, M, N, K, splits, stream);                            \
         }                                                                                                                   \
-        if (b_mn) return launch_gemm<BN_, false, true, CL_, 0, P2_>(ta, tb, td, epi, M, N, K, splits, stream);             \
-        return launch_gemm<BN_, false, false, CL_, 0, P2_>(ta, tb, td, epi, M, N, K, splits, stream);                      \
+        if (b_mn) return launch_gemm<BN_, false, true, CL_>(ta, tb, td, epi, M, N, K, splits, stream);                      \
+        return launch_gemm<BN_, false, false, CL_>(ta, tb, td, epi, M, N, K, splits, stream);                               \
     } while (0)
-    // CTA pairs: by default one cta_group::1 MMA per CTA over a multicast copy of B. SPNET_B200_PAIR_MMA=1 selects the
-    // cta_group::2 form (one 256-row MMA per k-step over both CTAs' shared memory, half of B per CTA, six ring stages).
-    // Measured on B200 (round 2): the cta_group::2 form is SLOWER on every shape of this network - 12288x728x728
-    // 18.4-20.1 us against 17.5-18.2 us, the K-stacked weight gradient 333 against 294 us (938 / 1062 TFLOP/s),
-    // 49152x728x728 66-73 against 62-64 us, step 7.32 against 7.16 ms: the M = 128, N = 256 single-CTA MMA already runs
-    // at the cuBLAS-peak rate, shared-memory bandwidth was not the limiter, and the pair now advances in lock step
-    // (one "full" barrier for both CTAs' loads, +1.5 us of set-up).
-    static const bool pair_mma = getenv("SPNET_B200_PAIR_MMA") != nullptr;
-    if (pair && pair_mma) SPNET_GEMM_DISPATCH(256, 2, true);
-    if (pair) SPNET_GEMM_DISPATCH(256, 2, false);
-    if (wide) SPNET_GEMM_DISPATCH(256, 1, false);
+    // CTA pairs run one cta_group::1 MMA per CTA over a multicast copy of B; a cta_group::2 pair MMA (one 256-row MMA
+    // over both CTAs' shared memory) measured slower on every shape of this network on B200 (step 7.32 against 7.16 ms).
+    if (pair) SPNET_GEMM_DISPATCH(256, 2);
+    if (wide) SPNET_GEMM_DISPATCH(256, 1);
     // N <= 64 (the data gradients into Xception's 64-channel block 1 output): 64-wide tiles - a 128-wide tile would
     // spend half of its B traffic, MMA columns and epilogue on columns that do not exist
-    if (N <= 64) SPNET_GEMM_DISPATCH(64, 1, false);
-    SPNET_GEMM_DISPATCH(128, 1, false);
+    if (N <= 64) SPNET_GEMM_DISPATCH(64, 1);
+    SPNET_GEMM_DISPATCH(128, 1);
 #undef SPNET_GEMM_DISPATCH
 }
 
@@ -974,14 +876,13 @@ int conv_tc_fwd_like(bool dgrad, const void* in, long long ld_in, int NB, int IH
     GemmEpi epi = {out, ld_out, OUT_BF16, 0, colstats};
     const int M = (int)(tiles_m * BM);
     // one 64-wide n-tile and at most kMaxResidentKb k-blocks: the weights stay in shared memory (BRES)
-    static const bool no_bres = getenv("SPNET_B200_NO_RESIDENT_B") != nullptr;
-    const bool bres = bn == 64 && K / BK <= kMaxResidentKb && !no_bres;
+    const bool bres = bn == 64 && K / BK <= kMaxResidentKb;
     if (!dgrad) {
-        if (bres) return launch_gemm<64, false, true, 1, 1, false, true>(ta, tb, td, epi, M, N, K, 1, stream, cg, (int)tiles_m);
+        if (bres) return launch_gemm<64, false, true, 1, 1, true>(ta, tb, td, epi, M, N, K, 1, stream, cg, (int)tiles_m);
         if (bn == 64) return launch_gemm<64, false, true, 1, 1>(ta, tb, td, epi, M, N, K, 1, stream, cg, (int)tiles_m);
         return launch_gemm<128, false, true, 1, 1>(ta, tb, td, epi, M, N, K, 1, stream, cg, (int)tiles_m);
     }
-    if (bres) return launch_gemm<64, false, false, 1, 1, false, true>(ta, tb, td, epi, M, N, K, 1, stream, cg, (int)tiles_m);
+    if (bres) return launch_gemm<64, false, false, 1, 1, true>(ta, tb, td, epi, M, N, K, 1, stream, cg, (int)tiles_m);
     if (bn == 64) return launch_gemm<64, false, false, 1, 1>(ta, tb, td, epi, M, N, K, 1, stream, cg, (int)tiles_m);
     return launch_gemm<128, false, false, 1, 1>(ta, tb, td, epi, M, N, K, 1, stream, cg, (int)tiles_m);
 }

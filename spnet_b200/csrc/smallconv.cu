@@ -13,7 +13,6 @@
 // through shared memory so that global stores are contiguous too. BatchNorm statistics and weight
 // gradients are accumulated in registers across all tiles of a CTA and reduced once at the end.
 #include "common.cuh"
-#include <stdlib.h>
 
 namespace {
 
@@ -992,9 +991,6 @@ template <typename K> void strip_smem_optin(K kern, size_t bytes) {
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
 }
 
-// SPNET_B200_NO_STRIP=1: the pixel-per-thread kernels for every width (comparison runs)
-const bool g_no_strip = getenv("SPNET_B200_NO_STRIP") != nullptr;
-
 }  // namespace
 
 extern "C" {
@@ -1020,7 +1016,7 @@ int spnet_conv_small_fwd(int which, const void* in, const float* w, const float*
                                         reinterpret_cast<const float*>(in), w, in_a, in_b, act, reinterpret_cast<T*>(out),
                                         reinterpret_cast<T*>(skip), stats, nullptr, nullptr, nullptr, B, H, W, OH, OW, 1,
                                         1, th, tw)));
-    } else if (which == 1 && W % 8 == 0 && !g_no_strip) {
+    } else if (which == 1 && W % 8 == 0) {
         const int th = ceil_div(H, SK_TH), tw = ceil_div(W, SK_TW);
         const int grid = persist_grid_tiles((long long)B * th * tw, 2);
         SPNET_DISPATCH_DTYPE(dtype, (strip_smem_optin(conv3c3_strip_kernel<T, 0>, StripWindow<T>::smem_bytes()),
@@ -1064,7 +1060,7 @@ int spnet_conv_small_wgrad(int which, const void* in, const float* in_a, const f
         SPNET_DISPATCH_DTYPE(dtype, (conv3out_wgrad_kernel<float, T, 1, 4, 2><<<grid, kThreads, 0, stream>>>(
                                         reinterpret_cast<const float*>(in), in_a, in_b, act, reinterpret_cast<const T*>(g),
                                         dw, dw_acc, B, H, W, OH, OW, 1, 1, th, tw)));
-    } else if (which == 1 && W % 8 == 0 && !g_no_strip) {
+    } else if (which == 1 && W % 8 == 0) {
         const int th = ceil_div(H, SK_TH), tw = ceil_div(W, SK_TW);
         const int grid = persist_grid_tiles((long long)B * th * tw, 1);
         SPNET_DISPATCH_DTYPE(dtype, (strip_smem_optin(conv3c3_wgrad_strip_kernel<T>, StripWindow<T>::smem_bytes()),
@@ -1099,7 +1095,7 @@ int spnet_conv_small_dgrad(int which, const void* g, const float* w, const void*
                            cudaStream_t stream) {
     SPNET_REQUIRE(g && w && gin && B > 0 && H > 2 && W > 2, "conv_small_dgrad: bad args");
     SPNET_REQUIRE(!mask_z || (mask_a && mask_b), "conv_small_dgrad: mask needs its affine");
-    if (which == 1 && W % 8 == 0 && !g_no_strip) {
+    if (which == 1 && W % 8 == 0) {
         const int th = ceil_div(H, SK_TH), tw = ceil_div(W, SK_TW);
         const int grid = persist_grid_tiles((long long)B * th * tw, 2);
         SPNET_DISPATCH_DTYPE(dtype, (strip_smem_optin(conv3c3_strip_kernel<T, 2>, StripWindow<T>::smem_bytes()),

@@ -51,7 +51,6 @@ class SPNetEngineBase:
         self._slabs = None
         self._affine_fixed = False
         self._gacc = None  # accumulator scratch of the deterministic weight-gradient paths (allocated with the activations)
-        rc = lib().check_device  # noqa: F841  (resolved lazily below, after the device is selected)
         self.device = torch.device(device)
         torch.cuda.set_device(self.device)
         lib().check_device()
@@ -483,31 +482,14 @@ class SPNetEngineBase:
         self.loss(with_grad=True)
         self.backward_head()
 
-    def _reserve_sms(self, on):
-        """Data parallelism: while a gradient all-reduce is in flight the persistent GEMMs leave the SMs NCCL holds alone
-        (grid = dp_gemm_cap CTAs instead of one per SM; the grid is baked into the captured graph)."""
-        cap = getattr(self, "dp_gemm_cap", 0)
-        if cap:
-            lib().gemm_set_cta_cap(cap if on else 0)
-
-    def _step_part2a(self):
-        self._reserve_sms(True)
-        self.backward_body_a()
-        self._reserve_sms(False)
-
-    def _step_part2b(self):
-        self._reserve_sms(True)
-        self.backward_body_b()
-        self._reserve_sms(False)
-        if self.grad_hook is None:
-            self.optimizer_step()
-
     def _step_body(self):
         self._step_part1()
         self._bucket_ready("head")
-        self._step_part2a()
+        self.backward_body_a()
         self._bucket_ready("tail")
-        self._step_part2b()
+        self.backward_body_b()
+        if self.grad_hook is None:
+            self.optimizer_step()
 
     def _bucket_ready(self, which):
         fn = getattr(self.grad_hook, "bucket_ready", None)
@@ -536,9 +518,9 @@ class SPNetEngineBase:
             with torch.cuda.graph(g1):
                 self._step_part1()
             with torch.cuda.graph(g2, pool=g1.pool()):
-                self._step_part2a()
+                self.backward_body_a()
             with torch.cuda.graph(g3, pool=g1.pool()):
-                self._step_part2b()
+                self.backward_body_b()
             self.graph = (g1, g2, g3)
 
     def train_step(self, lr):
@@ -692,7 +674,7 @@ class XceptionSPNetEngine(SPNetEngineBase):
         h2, w2 = sh["b1c2"]
         # block1_conv2 (3x3 'valid', 32 -> 64): bf16 runs it as an implicit GEMM on the materialised activation a11
         # (csrc/gemm_tc.cu kw-fold entry points); fp32 and the deterministic mode keep the im2col + GEMM route
-        self.b1_fold = self.lowp and not self.deterministic and os.environ.get("SPNET_B200_B1_IM2COL") is None
+        self.b1_fold = self.lowp and not self.deterministic
         if self.b1_fold:
             self.a11 = A(B, h1, w1, 32)
         else:
@@ -740,7 +722,7 @@ class XceptionSPNetEngine(SPNetEngineBase):
             names = ["block%d_sepconv%d/pointwise_kernel" % (b, j) for b in arch.MIDDLE_BLOCKS for j in (1, 2, 3)]
             even = all(self.offsets[n][0] == o0 + i * stride for i, n in enumerate(names))
             rows = B * mh * mw
-            self.mid_batched = even and rows % (64 if self.lowp else 16) == 0 and os.environ.get("SPNET_B200_NO_BATCHED_WGRAD") is None
+            self.mid_batched = even and rows % (64 if self.lowp else 16) == 0
             self.mid_gw_off, self.mid_gw_stride = o0, stride
 
     def _backbone_fwd(self, training):

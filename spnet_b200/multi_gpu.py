@@ -73,15 +73,6 @@ class GradAllReduce:
             self.ready = {k: torch.cuda.Event() for k in ("head", "tail")}
             self.done = {k: torch.cuda.Event() for k in ("head", "tail")}
         self.in_flight = set()
-        # diagnostic knobs (profiles/r2/dp_timeline.md): skip the collectives / run every Adam after backward
-        self.no_comm = os.environ.get("SPNET_B200_DP_NOCOMM") is not None
-        self.adam_late = os.environ.get("SPNET_B200_DP_ADAM_LATE") is not None
-        # when the head bucket's all-reduce starts: "early" = as soon as it is final (it then overlaps the GEMM-heavy
-        # exit / middle-flow backward), "late" = together with the tail bucket (it overlaps the bandwidth-bound entry flow)
-        self.head_late = os.environ.get("SPNET_B200_DP_HEAD", "early") == "late"
-        self._deferred = None
-        cap = os.environ.get("SPNET_B200_DP_GEMM_CTAS")
-        engine.dp_gemm_cap = int(cap) if cap else 0
         self.trace = bool(int(os.environ.get("SPNET_B200_DP_TRACE", "0"))) if trace is None else trace
         self.trace_log, self._ev = [], None
 
@@ -117,13 +108,11 @@ class GradAllReduce:
             from . import ops
             if not (which == "head" and engine.head_grad_lp is not None):
                 ops.cast_f32_to_bf16(engine.grads[lo:hi], self.glp[lo:hi])
-            if not self.no_comm:
-                self.dist.all_reduce(self.glp[lo:hi], group=self.group)
-        elif not self.no_comm:
+            self.dist.all_reduce(self.glp[lo:hi], group=self.group)
+        else:
             self.dist.all_reduce(engine.grads[lo:hi], group=self.group)
         self._mark(which + "_ar_end", stream)
-        if not self.adam_late:
-            engine.optimizer_step(grad_scale=1.0 / self.world, lo=lo, hi=hi, g_bf16=self.glp)
+        engine.optimizer_step(grad_scale=1.0 / self.world, lo=lo, hi=hi, g_bf16=self.glp)
         self._mark(which + "_adam_end", stream)
 
     def bucket_ready(self, engine, which):
@@ -132,17 +121,9 @@ class GradAllReduce:
         if not self.on_cuda or hi <= lo:
             return
         self._mark(which + "_ready")
-        if which == "head" and self.head_late and self.ranges["tail"][1] > self.ranges["tail"][0]:
-            self._deferred = "head"      # launched when the tail bucket is ready
-            return
         self.ready[which].record()
         with torch.cuda.stream(self.side):
             self.side.wait_event(self.ready[which])
-            if self._deferred:
-                self._reduce_and_step(engine, self._deferred, self.side)
-                self.done[self._deferred].record(self.side)
-                self.in_flight.add(self._deferred)
-                self._deferred = None
             self._reduce_and_step(engine, which, self.side)
             self.done[which].record(self.side)
         self.in_flight.add(which)
@@ -156,8 +137,6 @@ class GradAllReduce:
         for which in self.in_flight:
             torch.cuda.current_stream().wait_event(self.done[which])
         self.in_flight.clear()
-        if self.adam_late:
-            engine.optimizer_step(grad_scale=1.0 / self.world, g_bf16=self.glp)
         self._mark("step_end")
         if self._ev is not None:
             self.trace_log.append(self._ev)

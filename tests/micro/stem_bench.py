@@ -1,5 +1,5 @@
 """Times the stem / block-1 small-channel convolutions at the bench shape (B=64, 192x256x3 after the folded
-average pool). SPNET_B200_NO_STRIP=1 selects the pixel-per-thread kernels for which == 1."""
+average pool)."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
 import torch
