@@ -91,7 +91,7 @@ int spnet_dwconv3x3_bwd_fused(const void* gout, const void* in, const float* k, 
  *      summation order (spnet_slab_reduce), or a batch of GEMMs stacked along K in ONE launch (the weight gradients
  *      of Xception's 24 identical middle-flow layers, written straight into the flat gradient buffer). ---- */
 int spnet_gemm_bf16(const void* A, long long lda, int a_mn, const void* B, long long ldb, int b_mn, void* D, long long ldd, long long slab_stride, int out_mode, int M, int N, int K, int splits, long long* colstats, cudaStream_t stream);
-int spnet_gemm_simt(const void* A, long long sa_r, long long sa_k, const void* B, long long sb_r, long long sb_k, void* D, long long ldd, long long slab_stride, int dtype, int out_mode, int M, int N, int K, int splits, long long* colstats, cudaStream_t stream);
+int spnet_gemm_simt(const float* A, long long sa_r, long long sa_k, const float* B, long long sb_r, long long sb_k, float* D, long long ldd, long long slab_stride, int out_mode, int M, int N, int K, int splits, long long* colstats, cudaStream_t stream);
 
 /* ---- Conv2D k x k, stride 1, as implicit GEMM on tcgen05 (gemm_tc.cu, no im2col buffer): Xception
  *      block1_conv2 (keras.applications.Xception; spnet/models.py:359) and the InceptionResNetV2 branch
@@ -124,7 +124,7 @@ int spnet_maxpool3s2_bwd(const void* gout, const unsigned char* argmax, void* gi
 int spnet_gather_s2(const void* in, void* out, int dtype, int B, int H, int W, int C, int off_h, int off_w, cudaStream_t stream);
 int spnet_scatter_s2(const void* in, void* out, int dtype, int B, int H, int W, int C, int off_h, int off_w, cudaStream_t stream);
 
-/* ---- SPNet stem (spnet/models.py:319-340), block1_conv1, block1_conv2 im2col ---- */
+/* ---- SPNet stem (spnet/models.py:319-340), block1_conv1 ---- */
 int spnet_conv_small_fwd(int which, const void* in, const float* w, const float* in_a, const float* in_b, int act, void* out, void* skip, long long* stats, int dtype, int B, int H, int W, cudaStream_t stream);
 int spnet_conv_small_wgrad(int which, const void* in, const float* in_a, const float* in_b, int act, const void* g, float* dw, long long* dw_acc, int dtype, int B, int H, int W, cudaStream_t stream);
 int spnet_conv_small_dgrad(int which, const void* g, const float* w, const void* mask_z, const float* mask_a, const float* mask_b, int act, void* gin, int dtype, int B, int H, int W, cudaStream_t stream);
@@ -134,12 +134,11 @@ int spnet_stem_out_fwd(const void* c3, const float* a, const float* b, const voi
 int spnet_stem_out_bwd(const void* g, void* gout, int dtype, long long pixels, float rate, const unsigned long long* seed, cudaStream_t stream);
 int spnet_bn3_bwd_reduce(const void* g, const void* z, const float* save_mean, const float* save_rstd, long long* stats, int dtype, long long pixels, cudaStream_t stream);
 int spnet_bn3_bwd_dz(const void* g, const void* z, const float* a, const float* save_mean, const float* save_rstd, const float* c1, const float* c2, void* out, int dtype, long long pixels, cudaStream_t stream);
-int spnet_im2col3x3(const void* in, const float* a, const float* b, int relu, void* col, int dtype, int B, int H, int W, int C, cudaStream_t stream);
-int spnet_col2im3x3(const void* gcol, const void* z, const float* a, const float* b, int relu, void* gin, int dtype, int B, int H, int W, int C, cudaStream_t stream);
 
 /* ---- dense-convolution backbone pieces (keras.applications.InceptionResNetV2 via spnet/models.py:18,357-359):
- *      generic im2col / col2im around the GEMMs, 'valid' max-pool, AveragePooling2D(3,1,'same'), channel-slice
- *      copies (Concatenate), the scaled residual of the Inception-ResNet blocks, bias gradient ---- */
+ *      generic im2col / col2im around the GEMMs (also Xception's block1_conv2 in the fp32 and deterministic modes),
+ *      'valid' max-pool, AveragePooling2D(3,1,'same'), channel-slice copies (Concatenate), the scaled residual of the
+ *      Inception-ResNet blocks, bias gradient ---- */
 int spnet_im2col(const void* in, void* col, int dtype, int B, int H, int W, int C, int KH, int KW, int sh, int sw, int pt, int pl, int OH, int OW, cudaStream_t stream);
 int spnet_col2im(const void* gcol, void* gin, int accumulate, int dtype, int B, int H, int W, int C, int KH, int KW, int sh, int sw, int pt, int pl, int OH, int OW, cudaStream_t stream);
 int spnet_maxpool3s2_valid_fwd(const void* z, void* out, unsigned char* argmax, int dtype, int B, int H, int W, int C, cudaStream_t stream);
@@ -161,8 +160,6 @@ int spnet_sumsq(const float* p, long long n, float scale, long long* out, cudaSt
 int spnet_acc_to_f32(long long* acc, float* out, long long n, int accumulate, int clear, cudaStream_t stream);
 int spnet_slab_reduce(const float* slabs, int nslabs, long long slab_stride, long long lds, const float* bias, float* out, long long ldo, int rows, int cols, int accumulate, cudaStream_t stream);
 int spnet_cast_f32_to_bf16(const float* src, void* dst, long long n, cudaStream_t stream);
-int spnet_cast_bf16_to_f32(const void* src, float* dst, long long n, cudaStream_t stream);
-int spnet_bias_fill(const float* bias, float* out, int rows, int cols, cudaStream_t stream);
 int spnet_colsum(const float* g, float* out, int rows, int cols, cudaStream_t stream);
 
 #ifdef __cplusplus

@@ -1,6 +1,7 @@
 // Generic pieces for the dense-convolution backbone (keras.applications.InceptionResNetV2 behind
 // spnet/models.py:18,357-359 — BASELINE configs[3]): im2col / col2im for an arbitrary kh x kw, stride
-// and TF padding (the GEMM itself is gemm_tc.cu / gemm_simt.cu), 'valid' max-pooling entry points,
+// and TF padding (the GEMM itself is gemm_tc.cu / gemm_simt.cu; Xception's block1_conv2 uses the pair
+// too in the fp32 and deterministic modes), 'valid' max-pooling entry points,
 // AveragePooling2D(3, 1, 'same'), channel-slice copies for Concatenate, the scaled residual
 // `x + scale * (up + bias)` (+ReLU) of the Inception-ResNet blocks, accumulation and column sums.
 // All HBM-bound element-wise work on 16-byte channel vectors (C % 8 == 0 for bf16, % 4 for fp32).

@@ -1,8 +1,7 @@
 // Exact-fp32 GEMM on the CUDA cores (FFMA, fp32 accumulate) with arbitrary operand
 // strides. It is the fp32-mode engine behind the same layers gemm_tc.cu serves in bf16
 // mode (the reference network runs fp32: spnet/config.py:4), so that "fp32 within 1e-4"
-// parity can be checked without tensor-core rounding, and it also takes bf16 inputs for
-// shapes the tcgen05 kernel does not cover.
+// parity can be checked without tensor-core rounding.
 //
 //   D[M,N] (op)= sum_k A(r,k) * B(n,k),  A(r,k) = A[r*sa_r + k*sa_k],  B(n,k) = B[n*sb_r + k*sb_k]
 #include "common.cuh"
@@ -13,10 +12,9 @@ constexpr int TM = 64, TN = 64, TK = 16, PAD = 4;
 
 enum { OUT_T = 0, OUT_F32 = 1, OUT_ATOMIC_F32 = 2, OUT_SLAB_F32 = 3 };
 
-template <typename T>
-__global__ void __launch_bounds__(256) gemm_simt_kernel(const T* __restrict__ A, long long sa_r, long long sa_k,
-                                                        const T* __restrict__ B, long long sb_r, long long sb_k,
-                                                        void* __restrict__ D, long long ldd, long long slab_stride,
+__global__ void __launch_bounds__(256) gemm_simt_kernel(const float* __restrict__ A, long long sa_r, long long sa_k,
+                                                        const float* __restrict__ B, long long sb_r, long long sb_k,
+                                                        float* __restrict__ D, long long ldd, long long slab_stride,
                                                         int out_mode, int M, int N, int K, int k_per_split,
                                                         long long* __restrict__ colstats) {
     __shared__ float As[TK][TM + PAD];
@@ -41,11 +39,11 @@ __global__ void __launch_bounds__(256) gemm_simt_kernel(const T* __restrict__ A,
             int r, k;
             if (a_kfast) { k = e & (TK - 1); r = e >> 4; } else { r = e & (TM - 1); k = e >> 6; }
             float v = 0.f;
-            if (m0 + r < M && k0 + k < kend) v = to_f32(A[(long long)(m0 + r) * sa_r + (long long)(k0 + k) * sa_k]);
+            if (m0 + r < M && k0 + k < kend) v = A[(long long)(m0 + r) * sa_r + (long long)(k0 + k) * sa_k];
             As[k][r] = v;
             if (b_kfast) { k = e & (TK - 1); r = e >> 4; } else { r = e & (TN - 1); k = e >> 6; }
             v = 0.f;
-            if (n0 + r < N && k0 + k < kend) v = to_f32(B[(long long)(n0 + r) * sb_r + (long long)(k0 + k) * sb_k]);
+            if (n0 + r < N && k0 + k < kend) v = B[(long long)(n0 + r) * sb_r + (long long)(k0 + k) * sb_k];
             Bs[k][r] = v;
         }
         __syncthreads();
@@ -73,16 +71,14 @@ __global__ void __launch_bounds__(256) gemm_simt_kernel(const T* __restrict__ A,
             const int c = n0 + tx * 4 + j;
             if (c >= N) continue;
             float v = acc[i][j];
-            if (out_mode == OUT_T) {
-                T* o = reinterpret_cast<T*>(D) + (long long)r * ldd + c;
-                *o = from_f32<T>(v);
-                v = round_to<T>(v);
+            if (out_mode == OUT_T) {  // D in the operands' type: fp32, the same store as OUT_F32
+                D[(long long)r * ldd + c] = v;
             } else if (out_mode == OUT_F32) {
-                reinterpret_cast<float*>(D)[(long long)r * ldd + c] = v;
+                D[(long long)r * ldd + c] = v;
             } else if (out_mode == OUT_SLAB_F32) {  // split z keeps its partial in its own slab (fixed-order split-K)
-                reinterpret_cast<float*>(D)[(long long)blockIdx.z * slab_stride + (long long)r * ldd + c] = v;
+                D[(long long)blockIdx.z * slab_stride + (long long)r * ldd + c] = v;
             } else {
-                atomicAdd(reinterpret_cast<float*>(D) + (long long)r * ldd + c, v);
+                atomicAdd(D + (long long)r * ldd + c, v);
             }
             csum[j] += v;
             csq[j] = fmaf(v, v, csq[j]);
@@ -108,9 +104,9 @@ __global__ void __launch_bounds__(256) gemm_simt_kernel(const T* __restrict__ A,
 
 extern "C" {
 
-// dtype: element type of A and B (0 fp32, 1 bf16). out_mode 0 stores D in that same type.
-int spnet_gemm_simt(const void* A, long long sa_r, long long sa_k, const void* B, long long sb_r, long long sb_k,
-                    void* D, long long ldd, long long slab_stride, int dtype, int out_mode, int M, int N, int K, int splits,
+// A, B and D are fp32 in every out_mode.
+int spnet_gemm_simt(const float* A, long long sa_r, long long sa_k, const float* B, long long sb_r, long long sb_k,
+                    float* D, long long ldd, long long slab_stride, int out_mode, int M, int N, int K, int splits,
                     long long* colstats, cudaStream_t stream) {
     SPNET_REQUIRE(A && B && D, "gemm_simt: null pointer");
     SPNET_REQUIRE(M > 0 && N > 0 && K > 0, "gemm_simt: bad shape %d %d %d", M, N, K);
@@ -123,9 +119,8 @@ int spnet_gemm_simt(const void* A, long long sa_r, long long sa_k, const void* B
     splits = ceil_div(K, kps);
     dim3 grid(ceil_div(N, TN), ceil_div(M, TM), splits);
     SPNET_REQUIRE(grid.y <= 65535 && grid.z <= 65535, "gemm_simt: grid too large");
-    SPNET_DISPATCH_DTYPE(dtype, (gemm_simt_kernel<T><<<grid, 256, 0, stream>>>(
-                                    reinterpret_cast<const T*>(A), sa_r, sa_k, reinterpret_cast<const T*>(B), sb_r,
-                                    sb_k, D, ldd, slab_stride, out_mode, M, N, K, kps, colstats)));
+    gemm_simt_kernel<<<grid, 256, 0, stream>>>(A, sa_r, sa_k, B, sb_r, sb_k, D, ldd, slab_stride, out_mode, M, N, K, kps,
+                                               colstats);
     return spnet_check_launch("gemm_simt");
 }
 

@@ -141,17 +141,7 @@ __global__ void cast_f32_bf16_kernel(const float* __restrict__ src, bf16* __rest
          i += (long long)gridDim.x * blockDim.x)
         dst[i] = __float2bfloat16_rn(src[i]);
 }
-__global__ void cast_bf16_f32_kernel(const bf16* __restrict__ src, float* __restrict__ dst, long long n) {
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n;
-         i += (long long)gridDim.x * blockDim.x)
-        dst[i] = __bfloat162float(src[i]);
-}
 
-// out[r, c] = bias[c]
-__global__ void bias_fill_kernel(const float* __restrict__ bias, float* __restrict__ out, int rows, int cols) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < rows * cols) out[i] = bias[i % cols];
-}
 // out[c] = sum_r g[r, c]   (rows small: the Dense bias gradient)
 __global__ void colsum_kernel(const float* __restrict__ g, float* __restrict__ out, int rows, int cols) {
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
@@ -196,17 +186,7 @@ int spnet_cast_f32_to_bf16(const float* src, void* dst, long long n, cudaStream_
     cast_f32_bf16_kernel<<<grid_for(n), 256, 0, stream>>>(src, reinterpret_cast<bf16*>(dst), n);
     return spnet_check_launch("cast_f32_to_bf16");
 }
-int spnet_cast_bf16_to_f32(const void* src, float* dst, long long n, cudaStream_t stream) {
-    SPNET_REQUIRE(src && dst && n > 0, "cast_bf16_to_f32: bad args");
-    cast_bf16_f32_kernel<<<grid_for(n), 256, 0, stream>>>(reinterpret_cast<const bf16*>(src), dst, n);
-    return spnet_check_launch("cast_bf16_to_f32");
-}
 
-int spnet_bias_fill(const float* bias, float* out, int rows, int cols, cudaStream_t stream) {
-    SPNET_REQUIRE(bias && out && rows > 0 && cols > 0, "bias_fill: bad args");
-    bias_fill_kernel<<<ceil_div((long long)rows * cols, 256), 256, 0, stream>>>(bias, out, rows, cols);
-    return spnet_check_launch("bias_fill");
-}
 int spnet_colsum(const float* g, float* out, int rows, int cols, cudaStream_t stream) {
     SPNET_REQUIRE(g && out && rows > 0 && cols > 0, "colsum: bad args");
     colsum_kernel<<<ceil_div(cols, 128), 128, 0, stream>>>(g, out, rows, cols);

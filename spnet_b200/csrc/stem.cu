@@ -1,5 +1,4 @@
-// Stem glue kernels and the im2col pair for block1_conv2 (the small-channel convolutions
-// themselves are in smallconv.cu).
+// Stem glue kernels (the small-channel convolutions themselves are in smallconv.cu).
 //
 //  * SPNet stem (spnet/models.py:319-340): Conv2D(3,3x3,same,no bias) -> AveragePooling2D(2)
 //    -> BN -> LeakyReLU(0.1) -> Conv2D(3) -> BN -> LeakyReLU(0.1) -> Conv2D(3) -> BN
@@ -7,7 +6,6 @@
 //    conv+avgpool is evaluated as the equivalent 4x4 stride-2 convolution (pad 1) whose
 //    kernel is the 2x2 box average of the shifted 3x3 kernel, at a quarter of the work.
 //  * keras.applications.Xception block1_conv1 (3x3, stride 2, valid, 3->32).
-//  * block1_conv2 (3x3, valid, 32->64) as im2col + GEMM (gemm_tc.cu / gemm_simt.cu).
 //
 // All kernels are HBM/latency-bound (<1 % of the model's FLOPs); one thread per pixel,
 // weights in shared memory, BatchNorm statistics reduced in the epilogue.
@@ -252,94 +250,6 @@ __global__ void __launch_bounds__(256) bn3_bwd_dz_kernel(const T* g, const T* __
     }
 }
 
-// ---- im2col / col2im for a 3x3 'valid' stride-1 convolution ----
-// col[(b,oh,ow), (kh*3+kw)*C + c] = act(a*in+b)[b, oh+kh, ow+kw, c]
-// One CTA per output row (b, oh). A thread keeps ONE (tap, channel vector) of the 9*C-wide column row for the
-// whole launch - its coefficients sit in registers, its source offset is a constant - and steps through the
-// pixels of the row, blockDim / (9*CV) at a time; the threads of one pixel write 16-byte chunks of one
-// contiguous 2*9*C-byte row. (The one-thread-per-chunk version paid four divisions and 2*V scalar coefficient
-// loads per 16 bytes: 174 us for the 428 MB of block1_conv2.)
-template <typename T>
-__global__ void __launch_bounds__(256) im2col3x3_kernel(const T* __restrict__ in, const float* __restrict__ a,
-                                                        const float* __restrict__ b, int relu, T* __restrict__ col,
-                                                        int B, int H, int W, int C) {
-    constexpr int V = VecN<T>::N;
-    const int CV = C / V, OH = H - 2, OW = W - 2;
-    const int per_px = 9 * CV;                 // 16-byte chunks of one column row
-    const int px_step = blockDim.x / per_px;   // pixels handled per pass (host: >= 1)
-    const int sub = threadIdx.x % per_px, pxl = threadIdx.x / per_px;
-    if (pxl >= px_step) return;                // threads beyond a whole number of pixels
-    const int tap = sub / CV, cv = sub - tap * CV, c0 = cv * V;
-    const int kh = tap / 3, kw = tap - kh * 3;
-    const int row = blockIdx.x;                // bi * OH + oh
-    const int bi = row / OH, oh = row - bi * OH;
-    float av[V], bv[V];
-#pragma unroll
-    for (int i = 0; i < V; ++i) {
-        av[i] = a ? a[c0 + i] : 1.f;
-        bv[i] = a ? b[c0 + i] : 0.f;
-    }
-    const T* src = in + (((size_t)bi * H + oh + kh) * W + kw) * C + c0;
-    T* dst = col + (size_t)row * OW * 9 * C + (size_t)sub * V;
-    for (int ow = blockIdx.y * px_step + pxl; ow < OW; ow += px_step * gridDim.y) {
-        float v[V];
-        load_vec(src + (size_t)ow * C, v);
-#pragma unroll
-        for (int i = 0; i < V; ++i) {
-            float y = fmaf(v[i], av[i], bv[i]);
-            if (relu) y = fmaxf(y, 0.f);
-            v[i] = y;
-        }
-        store_vec(dst + (size_t)ow * 9 * C, v);
-    }
-}
-// gin[b,ih,iw,c] = relu'(a*z+b) * sum_{kh,kw} gcol[(b,ih-kh,iw-kw), (kh*3+kw)*C + c]
-template <typename T>
-__global__ void __launch_bounds__(256) col2im3x3_kernel(const T* __restrict__ gcol, const T* __restrict__ z,
-                                                        const float* __restrict__ a, const float* __restrict__ b,
-                                                        int relu, T* __restrict__ gin, int B, int H, int W, int C) {
-    constexpr int V = VecN<T>::N;
-    const int CV = C / V, OH = H - 2, OW = W - 2;
-    const long long n = (long long)B * H * W * CV;
-    const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (idx >= n) return;
-    const unsigned uidx = (unsigned)idx;
-    const int cv = (int)(uidx % CV);
-    unsigned r = uidx / CV;
-    const int iw = (int)(r % W);
-    r /= W;
-    const int ih = (int)(r % H);
-    const int bi = (int)(r / H);
-    const int c0 = cv * V;
-    float acc[V];
-#pragma unroll
-    for (int i = 0; i < V; ++i) acc[i] = 0.f;
-#pragma unroll
-    for (int kh = 0; kh < 3; ++kh) {
-        const int oh = ih - kh;
-        if (oh < 0 || oh >= OH) continue;
-#pragma unroll
-        for (int kw = 0; kw < 3; ++kw) {
-            const int ow = iw - kw;
-            if (ow < 0 || ow >= OW) continue;
-            float v[V];
-            load_vec(gcol + ((((size_t)bi * OH + oh) * OW + ow) * 9 + kh * 3 + kw) * C + c0, v);
-#pragma unroll
-            for (int i = 0; i < V; ++i) acc[i] += v[i];
-        }
-    }
-    if (relu) {
-        float zv[V];
-        load_vec(z + idx * V, zv);
-#pragma unroll
-        for (int i = 0; i < V; ++i) {
-            const float pre = a ? fmaf(zv[i], a[c0 + i], b[c0 + i]) : zv[i];
-            if (!(pre > 0.f)) acc[i] = 0.f;
-        }
-    }
-    store_vec(gin + idx * V, acc);
-}
-
 int persist_grid(long long n) {
     long long g = (n + 255) / 256;
     const long long cap = (long long)spnet_num_sms() * 4;
@@ -401,33 +311,6 @@ int spnet_bn3_bwd_dz(const void* g, const void* z, const float* a, const float* 
                                     reinterpret_cast<const T*>(g), reinterpret_cast<const T*>(z), a, save_mean, save_rstd,
                                     c1, c2, reinterpret_cast<T*>(out), pixels)));
     return spnet_check_launch("bn3_bwd_dz");
-}
-
-int spnet_im2col3x3(const void* in, const float* a, const float* b, int relu, void* col, int dtype, int B, int H,
-                    int W, int C, cudaStream_t stream) {
-    SPNET_REQUIRE(in && col && B > 0 && H > 2 && W > 2, "im2col3x3: bad args");
-    const int V = dtype == SPNET_BF16 ? 8 : 4;
-    SPNET_REQUIRE(C % V == 0 && (a == nullptr) == (b == nullptr), "im2col3x3: bad channel count or affine");
-    const int per_px = 9 * (C / V);
-    SPNET_REQUIRE(per_px <= 256, "im2col3x3: at most %d channels", 256 / 9 * V);
-    const int threads = 256 / per_px * per_px;       // a whole number of pixels per pass
-    const int px_step = threads / per_px;
-    int gy = ((W - 2) + 4 * px_step - 1) / (4 * px_step);  // ~4 pixels per thread
-    if (gy < 1) gy = 1;
-    SPNET_DISPATCH_DTYPE(dtype, (im2col3x3_kernel<T><<<dim3((unsigned)(B * (H - 2)), (unsigned)gy), threads, 0, stream>>>(
-                                    reinterpret_cast<const T*>(in), a, b, relu, reinterpret_cast<T*>(col), B, H, W, C)));
-    return spnet_check_launch("im2col3x3");
-}
-int spnet_col2im3x3(const void* gcol, const void* z, const float* a, const float* b, int relu, void* gin, int dtype,
-                    int B, int H, int W, int C, cudaStream_t stream) {
-    SPNET_REQUIRE(gcol && gin && B > 0 && H > 2 && W > 2, "col2im3x3: bad args");
-    const int V = dtype == SPNET_BF16 ? 8 : 4;
-    SPNET_REQUIRE(C % V == 0 && (a == nullptr) == (b == nullptr) && (!relu || z), "col2im3x3: bad args");
-    const long long n = (long long)B * H * W * (C / V);
-    SPNET_DISPATCH_DTYPE(dtype, (col2im3x3_kernel<T><<<ceil_div(n, 256), 256, 0, stream>>>(
-                                    reinterpret_cast<const T*>(gcol), reinterpret_cast<const T*>(z), a, b, relu,
-                                    reinterpret_cast<T*>(gin), B, H, W, C)));
-    return spnet_check_launch("col2im3x3");
 }
 
 }  // extern "C"

@@ -672,12 +672,11 @@ class XceptionSPNetEngine(SPNetEngineBase):
         h1, w1 = sh["b1c1"]
         self.z11 = A(B, h1, w1, 32)
         h2, w2 = sh["b1c2"]
-        # block1_conv2 (3x3 'valid', 32 -> 64): bf16 runs it as an implicit GEMM on the materialised activation a11
-        # (csrc/gemm_tc.cu kw-fold entry points); fp32 and the deterministic mode keep the im2col + GEMM route
+        # block1_conv2 (3x3 'valid', 32 -> 64) reads the materialised activation a11 = relu(BN(z11)): bf16 runs it as
+        # an implicit GEMM (csrc/gemm_tc.cu kw-fold entry points); fp32 and the deterministic mode as im2col + GEMM
         self.b1_fold = self.lowp and not self.deterministic
-        if self.b1_fold:
-            self.a11 = A(B, h1, w1, 32)
-        else:
+        self.a11 = A(B, h1, w1, 32)
+        if not self.b1_fold:
             self.col = A(B * h2 * w2, 288)
         self.z12 = A(B, h2, w2, 64)
         self.x2 = A(B, h2, w2, 64)
@@ -733,12 +732,12 @@ class XceptionSPNetEngine(SPNetEngineBase):
         ops.conv_small_fwd(2, self.d, w["block1_conv1/kernel"], self.z11, stats=st(self.b1_bn1))
         self._bn_ready(self.b1_bn1, B * h1 * w1, training)
         h2, w2 = sh["b1c2"]
+        ops.bn_apply(self.z11, self.b1_bn1.a, self.b1_bn1.b, act=1, out=self.a11)
         if self.b1_fold:
-            ops.bn_apply(self.z11, self.b1_bn1.a, self.b1_bn1.b, act=1, out=self.a11)
             ops.conv_tc_fwd_kwfold(self.a11, self.wl["block1_conv2/kernel"], self.z12, colstats=st(self.b1_bn2))
             self._bn_ready(self.b1_bn2, B * h2 * w2, training)
         else:
-            ops.im2col3x3(self.z11, self.col, self.b1_bn1.a, self.b1_bn1.b, True)
+            ops.im2col(self.a11, self.col, 3, 3, 1, 0, 0, h2, w2)
             self._pw_fwd(self.col, self.wl["block1_conv2/kernel"].view(288, 64), self.z12.view(-1, 64), B * h2 * w2, 288,
                          64, self.b1_bn2, training)
         ops.bn_apply(self.z12, self.b1_bn2.a, self.b1_bn2.b, act=1, out=self.x2)
@@ -829,20 +828,18 @@ class XceptionSPNetEngine(SPNetEngineBase):
         g_z12 = self._bn_bwd(g_x, self.z12, self.b1_bn2, M2, relu_mask=True)
         W2l = self.wl["block1_conv2/kernel"].view(288, 64)
         g_y11 = self._view(G1, B, h1, w1, 32)
-        if self.lowp:
-            # weight gradient from the forward's im2col buffer; data gradient as implicit GEMM (csrc/gemm_tc.cu
-            # CONV mode: 95 us instead of a 120 us GEMM into a 428 MB column-gradient buffer + 97 us col2im),
-            # the ReLU mask of block1_conv1_act is applied by the BatchNorm-backward reduction that follows
-            if self.b1_fold:
-                ops.conv_tc_wgrad_kwfold(self.a11, g_z12.view(B, h2, w2, 64), g["block1_conv2/kernel"].view(3, 3, 32, 64))
-            else:
-                self._pw_bwd(self.col, W2l, g["block1_conv2/kernel"].view(288, 64), g_z12.view(M2, 64), None, M2, 288, 64)
-            ops.conv_tc_dgrad(g_z12.view(B, h2, w2, 64), self.wl["block1_conv2/kernel"], g_y11, 0, 0)
-            g_z11 = self._bn_bwd(g_y11, self.z11, self.b1_bn1, B * h1 * w1, relu_mask=True)
-        else:
+        if self.b1_fold:
+            ops.conv_tc_wgrad_kwfold(self.a11, g_z12.view(B, h2, w2, 64), g["block1_conv2/kernel"].view(3, 3, 32, 64))
+        else:  # weight gradient from the forward's im2col buffer; fp32 also forms the column gradient (gcol)
             self._pw_bwd(self.col, W2l, g["block1_conv2/kernel"].view(288, 64), g_z12.view(M2, 64), self.gcol, M2, 288, 64)
-            ops.col2im3x3(self.gcol, g_y11, z=self.z11, a=self.b1_bn1.a, b=self.b1_bn1.b, relu=True)
-            g_z11 = self._bn_bwd(g_y11, self.z11, self.b1_bn1, B * h1 * w1)
+        if self.lowp:
+            # data gradient as implicit GEMM (csrc/gemm_tc.cu CONV mode: 95 us instead of a 120 us GEMM into a 428 MB
+            # column-gradient buffer + 97 us col2im)
+            ops.conv_tc_dgrad(g_z12.view(B, h2, w2, 64), self.wl["block1_conv2/kernel"], g_y11, 0, 0)
+        else:
+            ops.col2im(self.gcol, g_y11, 3, 3, 1, 0, 0, h2, w2)
+        # the ReLU mask of block1_conv1_act is applied by the BatchNorm-backward reduction
+        g_z11 = self._bn_bwd(g_y11, self.z11, self.b1_bn1, B * h1 * w1, relu_mask=True)
         ops.conv_small_wgrad(2, self.d, g_z11, g["block1_conv1/kernel"], acc=self._gacc)
         ops.conv_small_dgrad(2, g_z11, w["block1_conv1/kernel"], ga)
 

@@ -133,21 +133,8 @@ def gemm(A, a_mn, B, b_mn, D, M, N, K, out_mode=OUT_T, splits=1, colstats=None, 
         assert A.dtype == torch.float32 and B.dtype == torch.float32
         sa = (1, lda) if a_mn else (lda, 1)
         sb = (1, ldb) if b_mn else (ldb, 1)
-        lib().gemm_simt(_p(A), sa[0], sa[1], _p(B), sb[0], sb[1], _p(D), ldd, ss, F32, out_mode, M, N, K, splits,
-                        _p(colstats), _s())
-    return D
-
-
-def gemm_simt(A, a_mn, B, b_mn, D, M, N, K, out_mode=OUT_T, splits=1, colstats=None, lda=None, ldb=None, ldd=None):
-    """Same contract as gemm() but always on the CUDA-core kernel (any supported dtype)."""
-    _chk(A, B, D, colstats)
-    lda = lda if lda is not None else (M if a_mn else K)
-    ldb = ldb if ldb is not None else (N if b_mn else K)
-    ldd = ldd if ldd is not None else N
-    sa = (1, lda) if a_mn else (lda, 1)
-    sb = (1, ldb) if b_mn else (ldb, 1)
-    lib().gemm_simt(_p(A), sa[0], sa[1], _p(B), sb[0], sb[1], _p(D), ldd, M * ldd if out_mode == OUT_SLAB else 0,
-                    dtype_code(A), out_mode, M, N, K, splits, _p(colstats), _s())
+        lib().gemm_simt(_p(A), sa[0], sa[1], _p(B), sb[0], sb[1], _p(D), ldd, ss, out_mode, M, N, K, splits, _p(colstats),
+                        _s())
     return D
 
 
@@ -389,20 +376,6 @@ def bn3_bwd_dz(g, z, a, save_mean, save_rstd, c1, c2, out):
     return out
 
 
-def im2col3x3(x, col, a=None, b=None, relu=False):
-    _chk(x, col)
-    B, H, W, C = x.shape
-    lib().im2col3x3(_p(x), _p(a), _p(b), int(relu), _p(col), dtype_code(x), B, H, W, C, _s())
-    return col
-
-
-def col2im3x3(gcol, gin, z=None, a=None, b=None, relu=False):
-    _chk(gcol, gin, z)
-    B, H, W, C = gin.shape
-    lib().col2im3x3(_p(gcol), _p(z), _p(a), _p(b), int(relu), _p(gin), dtype_code(gin), B, H, W, C, _s())
-    return gin
-
-
 # ----------------------------------------------------------------------------- optimiser
 def adam_keras_step(p, g, m, v, lr_t_dev, n_l2=0, l2=1e-4, beta1=0.9, beta2=0.999, eps=1e-7, grad_scale=1.0,
                     p_bf16=None, frozen8=None, g_bf16=None):
@@ -494,15 +467,6 @@ def normalize_u8(x_u8, out=None):
 
 def cast_f32_to_bf16(src, dst):
     lib().cast_f32_to_bf16(_p(src), _p(dst), src.numel(), _s())
-
-
-def cast_bf16_to_f32(src, dst):
-    lib().cast_bf16_to_f32(_p(src), _p(dst), src.numel(), _s())
-
-
-def bias_fill(bias, out):
-    rows, cols = out.shape
-    lib().bias_fill(_p(bias), _p(out), rows, cols, _s())
 
 
 def colsum(g, out):

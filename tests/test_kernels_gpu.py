@@ -498,29 +498,39 @@ def test_stem_and_block1_convs(dtype, hw):
 
 
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16])
-def test_im2col_col2im(dtype):
+@pytest.mark.parametrize("stride,pad,accumulate", [(1, 0, False), (2, 1, False), (1, 0, True)],
+                         ids=["valid", "stride2_pad1", "accumulate"])
+def test_im2col_col2im(stride, pad, accumulate, dtype):
+    """block1_conv2's column route (fp32 and deterministic modes, 'valid'): im2col of relu(a*x+b) from bn_apply; col2im
+    of the column gradient, masked by the ReLU inside bn_bwd_reduce. Also the same pair with stride 2 and a leading pad
+    of 1, and a col2im that adds into the gradient already there."""
     ops = _ops()
     torch.manual_seed(13)
     B, H, W, C = 2, 11, 13, 32
     x = torch.randn(B, H, W, C, device=dev()).to(dtype)
     a = torch.rand(C, device=dev()) + 0.5
     b = torch.randn(C, device=dev()) * 0.2
-    col = torch.empty(B * (H - 2) * (W - 2), 9 * C, device=dev(), dtype=dtype)
-    ops.im2col3x3(x, col, a, b, True)
-    v = torch.relu(x.float() * a + b)
-    ref = F.unfold(nchw(v), 3)  # [B, C*9, L] with channel-major rows
-    ref = ref.reshape(B, C, 9, -1).permute(0, 3, 2, 1).reshape(B * (H - 2) * (W - 2), 9 * C)
+    pre = x.float() * a + b
+    act = ops.bn_apply(x, a, b, act=1)
+    OH, OW = (H + 2 * pad - 3) // stride + 1, (W + 2 * pad - 3) // stride + 1
+    col = torch.empty(B * OH * OW, 9 * C, device=dev(), dtype=dtype)
+    ops.im2col(act, col, 3, 3, stride, pad, pad, OH, OW)
+    ref = F.unfold(nchw(torch.relu(pre)), 3, padding=pad, stride=stride)  # [B, C*9, L] with channel-major rows
+    ref = ref.reshape(B, C, 9, -1).permute(0, 3, 2, 1).reshape(B * OH * OW, 9 * C)
     torch.testing.assert_close(col.float(), ref, **tol(dtype))
     gcol = torch.randn_like(col.float()).to(dtype)
-    gin = torch.empty_like(x)
-    ops.col2im3x3(gcol, gin, z=x, a=a, b=b, relu=True)
+    gin0 = torch.randn_like(x.float()).to(dtype)
+    gin = gin0.clone() if accumulate else torch.full_like(x, float("nan"))  # without accumulate col2im overwrites
+    ops.col2im(gcol, gin, 3, 3, stride, pad, pad, OH, OW, accumulate=accumulate)
+    mean, rstd = torch.zeros(C, device=dev()), torch.ones(C, device=dev())
+    ops.bn_bwd_reduce(gin, x, mean, rstd, ops.stats_alloc(2 * C, dev()), relu_a=a, relu_b=b, act=1)
     gref = gcol.float().reshape(B, -1, 9, C).permute(0, 3, 2, 1).reshape(B, C * 9, -1)
-    gref = nhwc(F.fold(gref, (H, W), 3)) * ((x.float() * a + b) > 0)
-    torch.testing.assert_close(gin.float(), gref, **tol(dtype))
+    gref = nhwc(F.fold(gref, (H, W), 3, padding=pad, stride=stride)) + (gin0.float() if accumulate else 0)
+    torch.testing.assert_close(gin.float(), gref * (pre > 0), **tol(dtype))
 
 
 # ------------------------------------------------------------------ optimiser
-def test_adam_keras_and_helpers():
+def test_adam_keras_sumsq_and_colsum():
     ops = _ops()
     torch.manual_seed(17)
     n, n_l2 = 10000, 3000
@@ -563,10 +573,6 @@ def test_adam_keras_and_helpers():
     vr2 = 0.999 * v.double() + 0.001 * gg2 * gg2
     pr2 = p.double() - lr_t * mr2 / (vr2.sqrt() + 1e-7)
     torch.testing.assert_close(p2.double()[~fr], pr2[~fr], rtol=1e-5, atol=1e-7)
-    bias = torch.randn(576, device=dev())
-    y = torch.empty(5, 576, device=dev())
-    ops.bias_fill(bias, y)
-    torch.testing.assert_close(y, bias.expand(5, 576))
     cs = torch.empty(576, device=dev())
     gy = torch.randn(5, 576, device=dev())
     ops.colsum(gy, cs)
@@ -577,8 +583,9 @@ def test_adam_keras_and_helpers():
 # (BASELINE.json configs[1] shapes: batch 64, 384x512 -> layer shapes below; no CPU oracle at these sizes)
 @pytest.mark.parametrize("M,N,K,a_mn,b_mn", [(12288, 728, 728, False, True), (744000, 128, 64, False, True),
                                               (728, 728, 12288, True, True), (49152, 728, 256, False, False)])
-def test_fullsize_gemm_two_implementations_agree(M, N, K, a_mn, b_mn):
-    """tcgen05 GEMM vs the independent fp32 FFMA GEMM on the same bf16-rounded operands."""
+def test_fullsize_gemm_tcgen05_matches_fp32_ffma(M, N, K, a_mn, b_mn):
+    """tcgen05 GEMM (bf16 operands) vs the independent fp32 FFMA GEMM (the same operands as fp32), both through
+    ops.gemm, which picks the kernel from the operand dtype."""
     ops = _ops()
     torch.manual_seed(M % 1000 + N + K)
     A = (torch.randn((K, M) if a_mn else (M, K), device=dev()) * 0.5).to(torch.bfloat16)
@@ -587,7 +594,7 @@ def test_fullsize_gemm_two_implementations_agree(M, N, K, a_mn, b_mn):
     D1 = torch.zeros(M, N, device=dev())
     ops.gemm(A, a_mn, B, b_mn, D1, M, N, K, out_mode=mode, splits=0 if a_mn else 1)
     D2 = torch.zeros(M, N, device=dev())
-    ops.gemm_simt(A.float(), a_mn, B.float(), b_mn, D2, M, N, K, out_mode=ops.OUT_F32)
+    ops.gemm(A.float(), a_mn, B.float(), b_mn, D2, M, N, K, out_mode=ops.OUT_F32)
     scale = float(D2.abs().max())
     torch.testing.assert_close(D1, D2, rtol=1e-3, atol=2e-4 * scale)
 

@@ -335,7 +335,7 @@ def test_bf16_kernels_layer_by_layer_teacher_forced():
         pooled = xt.maxpool3s2_same(y2.permute(0, 3, 1, 2)).permute(0, 2, 3, 1)   # TF 'same' padding with -inf
         res = e["zr"].double() * e["res_bn"].a.double() + e["res_bn"].b.double()
         check(tag + "_out", e["out"], pooled + res, pooled.abs() + res.abs() + e["res_bn"].b.double().abs() + e["sep2"].bn.b.double().abs())
-    # block 1 conv2 (im2col GEMM) and the Dense head
+    # block 1 conv2 (3x3 'valid' over the bf16 activation a11 = relu(BN(z11))) and the Dense head
     z11 = eng.z11.double() * eng.b1_bn1.a.double() + eng.b1_bn1.b.double()
     col = torch.relu(z11).to(torch.bfloat16).double().permute(0, 3, 1, 2)
     k2 = eng.wl["block1_conv2/kernel"].double().permute(3, 2, 0, 1)
