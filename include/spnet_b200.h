@@ -83,7 +83,7 @@ int spnet_augment_on_the_fly(const float* x_orig, float* x, int n, int H, int W,
 
 /* ---- SeparableConv2D depthwise half (keras.applications.Xception; spnet/models.py:359) ---- */
 int spnet_dwconv3x3_fwd(const void* in, const float* k, const float* in_a, const float* in_b, int relu, void* out, int dtype, int B, int H, int W, int C, cudaStream_t stream);
-int spnet_dwconv3x3_bwd_fused(const void* gout, const void* in, const float* k, const float* in_a, const float* in_b, int relu, const float* bn_mean, const float* bn_rstd, long long* stats, const void* add_src, const void* add_strided, void* gin, float* dk, long long* dk_acc, int dtype, int B, int H, int W, int C, cudaStream_t stream);
+int spnet_dwconv3x3_bwd_fused(const void* gout, const void* in, const float* k, const float* in_a, const float* in_b, int relu, const float* bn_mean, const float* bn_rstd, long long* stats, const void* add_src, const void* add_strided, void* gin, float* dk, long long* dk_acc, int dtype, int B, int H, int W, int C, const void* zo, const float* zo_mean, const float* zo_rstd, long long* zo_stats, const float* mask_a, const float* mask_b, cudaStream_t stream);
 
 /* ---- GEMMs: pointwise 1x1, strided 1x1 residual convs, block1_conv2 (im2col), Dense head
  *      (spnet/models.py:359,388). See gemm_tc.cu / gemm_simt.cu for operand conventions. out_mode 3 (slabs): split s
@@ -120,7 +120,7 @@ int spnet_bn_bwd_dz(const void* g, const void* z, const float* a, const float* s
 
 /* ---- MaxPooling2D(3,2,'same') + BN-apply + residual Add (Xception blocks 2-4, 13) ---- */
 int spnet_maxpool3s2_add_fwd(const void* z, const float* a, const float* b, const void* res, const float* ra, const float* rb, void* out, unsigned char* argmax, int dtype, int B, int H, int W, int C, cudaStream_t stream);
-int spnet_maxpool3s2_bwd(const void* gout, const unsigned char* argmax, void* gin, int dtype, int B, int H, int W, int C, cudaStream_t stream);
+int spnet_maxpool3s2_bwd(const void* gout, const unsigned char* argmax, void* gin, int dtype, int B, int H, int W, int C, const void* z, const float* mean, const float* rstd, long long* stats, cudaStream_t stream);
 int spnet_gather_s2(const void* in, void* out, int dtype, int B, int H, int W, int C, int off_h, int off_w, cudaStream_t stream);
 int spnet_scatter_s2(const void* in, void* out, int dtype, int B, int H, int W, int C, int off_h, int off_w, cudaStream_t stream);
 

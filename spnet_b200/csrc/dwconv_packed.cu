@@ -260,16 +260,24 @@ dw3x3_fwd_packed_kernel(const __grid_constant__ CUtensorMap tm_in, const float* 
 //   dk   += sum act(in)[h+kh-1, w+kw-1] * gout[h, w]                      (weight gradient)
 //   stats += (sum gin, sum gin * xhat),  xhat = (in - mean)*rstd          (BatchNorm-backward sums of
 //            the BN that produced `in`; only when stats != nullptr)
+// or, with ZO, the BatchNorm-backward sums of the BN whose output gradient gin IS (zo = that BN's raw input,
+// same shape as gin), taken on the final gin after the epilogue add and the optional ReLU mask
+//   gin   = 0 where !(mask_a*zo + mask_b > 0)                              (mask_a != nullptr)
+//   stats += (sum gin, sum gin * xhat),  xhat = zo*rstd - mean*rstd        (mean/rstd/stats: zo's BN)
+// so that no separate bn_bwd_reduce pass has to read gin and zo again. The mask and xhat use the same FMAs as
+// bn_bwd_reduce_kernel: the stored gin is bit-identical to what the masked reduce writes back. ZO uses the stats
+// slots of the input BN, and no caller needs both.
 // Both gradients use the SAME 3x3 neighbourhood G of gout around a pixel p:
 //   gin[p] = sum_n G_n * kflip_n,   dkflip_n += act(in)[p] * G_n
 // so a thread keeps a 3-row window of the gradient in registers and runs both from it.
-// Stage = gout tile with halo (zero-filled) + in tile (+ add_src tile), one mbarrier.
+// Stage = gout tile with halo (zero-filled) + in tile (+ add_src tile) (+ zo tile), one mbarrier.
 // EPI: 0 none, 1 add_src (TMA-staged), 2 add_strided (global loads at even rows/columns).
 // =================================================================================================
-template <typename T, bool AFFINE, int RELU, int EPI>
+template <typename T, bool AFFINE, int RELU, int EPI, bool ZO>
 __global__ void __launch_bounds__(512, 1)
 dw3x3_bwd_packed_kernel(const __grid_constant__ CUtensorMap tm_g, const __grid_constant__ CUtensorMap tm_x,
-                        const __grid_constant__ CUtensorMap tm_add, const float* __restrict__ k,
+                        const __grid_constant__ CUtensorMap tm_add, const __grid_constant__ CUtensorMap tm_zo,
+                        const float* __restrict__ mask_a, const float* __restrict__ mask_b, const float* __restrict__ k,
                         const float* __restrict__ in_a, const float* __restrict__ in_b,
                         const float* __restrict__ bn_mean, const float* __restrict__ bn_rstd, long long* __restrict__ stats,
                         const T* __restrict__ add_strided, T* __restrict__ gin, float* __restrict__ dk,
@@ -291,7 +299,8 @@ dw3x3_bwd_packed_kernel(const __grid_constant__ CUtensorMap tm_g, const __grid_c
     const uint32_t g_bytes = (uint32_t)(TH + 2) * grow_bytes;
     const uint32_t xrow_bytes = (uint32_t)TW * PIX;            // input / add tile row
     const uint32_t x_bytes = (uint32_t)TH * xrow_bytes;
-    const uint32_t stage_bytes = g_bytes + x_bytes * (EPI == 1 ? 2u : 1u);
+    const uint32_t zo_off = g_bytes + x_bytes * (EPI == 1 ? 2u : 1u);  // zo tile (ZO), after in (+ add_src)
+    const uint32_t stage_bytes = zo_off + (ZO ? x_bytes : 0u);
     const int n_tiles = B * tiles_h * tiles_w;
 
     if (threadIdx.x == 0) {
@@ -310,6 +319,7 @@ dw3x3_bwd_packed_kernel(const __grid_constant__ CUtensorMap tm_g, const __grid_c
         tma_load_4d(dst, &tm_g, bar, cbase, t.w0 - 1, t.h0 - 1, t.b);
         tma_load_4d(dst + g_bytes, &tm_x, bar, cbase, t.w0, t.h0, t.b);
         if (EPI == 1) tma_load_4d(dst + g_bytes + x_bytes, &tm_add, bar, cbase, t.w0, t.h0, t.b);
+        if (ZO) tma_load_4d(dst + zo_off, &tm_zo, bar, cbase, t.w0, t.h0, t.b);
     };
     if (threadIdx.x == 0)
         for (int i = 0; i < S - 1; ++i)
@@ -327,6 +337,15 @@ dw3x3_bwd_packed_kernel(const __grid_constant__ CUtensorMap tm_g, const __grid_c
     av = (AFFINE && c_ok) ? make_float2(in_a[c0], in_a[c0 + 1]) : make_float2(1.f, 1.f);
     bv = (AFFINE && c_ok) ? make_float2(in_b[c0], in_b[c0 + 1]) : make_float2(0.f, 0.f);
     s1 = s2 = make_float2(0.f, 0.f);
+    // ZO: xhat = zo*rs + nm, nm = -mean*rs (as bn_bwd_reduce_kernel); mask open where ma*zo + mb > 0
+    float2 rs, nm, ma, mb;
+    const bool masked = ZO && mask_a != nullptr;
+    if (ZO) {
+        rs = c_ok ? make_float2(bn_rstd[c0], bn_rstd[c0 + 1]) : make_float2(0.f, 0.f);
+        nm = c_ok ? make_float2(-bn_mean[c0] * rs.x, -bn_mean[c0 + 1] * rs.y) : make_float2(0.f, 0.f);
+        ma = (masked && c_ok) ? make_float2(mask_a[c0], mask_a[c0 + 1]) : make_float2(0.f, 0.f);
+        mb = (masked && c_ok) ? make_float2(mask_b[c0], mask_b[c0 + 1]) : make_float2(0.f, 0.f);
+    }
     const int col0 = warp * NC;
     const size_t rowC = (size_t)W * C;
     const int H2 = (H + 1) >> 1, W2 = (W + 1) >> 1;
@@ -379,11 +398,12 @@ dw3x3_bwd_packed_kernel(const __grid_constant__ CUtensorMap tm_g, const __grid_c
                 }
                 if (r >= 2) {
                     const int oh = h0 + r - 2;
-                    raw_t xr[NC], ar[NC], sr;
+                    raw_t xr[NC], ar[NC], zr[NC], sr;
 #pragma unroll
                     for (int oc = 0; oc < NC; ++oc) {
                         xr[oc] = lds_raw(s_x + oc * PIX, (const T*)nullptr);
                         if (EPI == 1) ar[oc] = lds_raw(s_x + x_bytes + oc * PIX, (const T*)nullptr);
+                        if (ZO) zr[oc] = lds_raw(s_x + (zo_off - g_bytes) + oc * PIX, (const T*)nullptr);
                     }
                     const bool sa_row = sa_ok && (oh & 1) == 0;
                     if (EPI == 2 && sa_row) sr = ldg_raw(sa_ptr + (size_t)(oh >> 1) * W2 * C);
@@ -411,13 +431,24 @@ dw3x3_bwd_packed_kernel(const __grid_constant__ CUtensorMap tm_g, const __grid_c
                             if (!act_open<RELU>(pre.x)) d.x = 0.f;
                             if (!act_open<RELU>(pre.y)) d.y = 0.f;
                         }
-                        if (stats) {
+                        if (!ZO && stats) {
                             const float2 rr = round_pair(d, (const T*)nullptr);
                             s1 = fadd2(s1, rr);
                             s2 = ffma2(rr, u, s2);
                         }
                         if (EPI == 1) d = fadd2(d, widen(ar[oc]));
                         if (EPI == 2 && sa_row && oc == oc_even) d = fadd2(d, widen(sr));
+                        if (ZO) {
+                            const float2 zu = widen(zr[oc]);
+                            if (masked) {
+                                const float2 y = ffma2(zu, ma, mb);
+                                if (!(y.x > 0.f)) d.x = 0.f;
+                                if (!(y.y > 0.f)) d.y = 0.f;
+                            }
+                            const float2 rr = round_pair(d, (const T*)nullptr);
+                            s1 = fadd2(s1, rr);
+                            s2 = ffma2(rr, ffma2(zu, rs, nm), s2);
+                        }
                         if (c_ok) stg_pair(o_ptr + (size_t)oc * C, d);
                     }
                     o_ptr += rowC;
@@ -456,6 +487,8 @@ dw3x3_bwd_packed_kernel(const __grid_constant__ CUtensorMap tm_g, const __grid_c
         } else if (stats) {
             if (q == 9) {
                 stat_add(stats, c, (double)sum);  // sum g
+            } else if (ZO) {
+                stat_add(stats, (long long)C + c, (double)sum);  // sum g*xhat
             } else {
                 // sum g*xhat = rstd * (sum g*in - mean * sum g)
                 float sg = 0.f;
@@ -494,7 +527,8 @@ int make_map(CUtensorMap* map, const void* ptr, int dtype, int B, int H, int W, 
 
 struct Tiling { int TH, TW, NC, S, tiles_h, tiles_w, threads, chunks, grid_x; size_t smem; };
 
-// kind 0: forward (stage = haloed input tile); 1: backward (haloed gradient + input); 2: backward + add_src tile
+// kind 0: forward (stage = haloed input tile); kind >= 1: backward, haloed gradient tile + `kind` unhaloed tiles
+// (input, then add_src and zo where present)
 Tiling pick_tiling(int kind, int dtype, int B, int H, int W, int C) {
     Tiling t;
     const size_t pix = (size_t)CB * (dtype == SPNET_BF16 ? 2 : 4);
@@ -512,7 +546,7 @@ Tiling pick_tiling(int kind, int dtype, int B, int H, int W, int C) {
     const int cands[] = {2, 3, 4, 6, 8, 12, 16};
     for (int th : cands) {
         if (th > H && th != 2) continue;
-        const size_t stage = (size_t)(th + 2) * (t.TW + 2) * pix + (kind ? (size_t)th * t.TW * pix * (kind == 2 ? 2 : 1) : 0);
+        const size_t stage = (size_t)(th + 2) * (t.TW + 2) * pix + (size_t)th * t.TW * pix * kind;
         int S = (int)(budget / stage);
         if (S > MAX_STAGES) S = MAX_STAGES;
         if (S < 2) continue;
@@ -568,11 +602,12 @@ int launch_fwd(const void* in, const float* k, const float* a, const float* b, i
     return launch_fwd_inst<T, 4, false, 0>(tm, k, a, b, y, B, H, W, C, t, stream);
 }
 
-template <typename T, bool AF, int RL, int EPI>
-int launch_bwd_inst(const CUtensorMap& tg, const CUtensorMap& tx, const CUtensorMap& ta, const float* k, const float* a,
-                    const float* b, const float* mean, const float* rstd, long long* stats, const T* sadd, T* gin,
-                    float* dk, long long* dk_acc, int B, int H, int W, int C, const Tiling& t, cudaStream_t stream) {
-    auto kern = dw3x3_bwd_packed_kernel<T, AF, RL, EPI>;
+template <typename T, bool AF, int RL, int EPI, bool ZO>
+int launch_bwd_inst(const CUtensorMap& tg, const CUtensorMap& tx, const CUtensorMap& ta, const CUtensorMap& tz,
+                    const float* ma, const float* mb, const float* k, const float* a, const float* b, const float* mean,
+                    const float* rstd, long long* stats, const T* sadd, T* gin, float* dk, long long* dk_acc, int B,
+                    int H, int W, int C, const Tiling& t, cudaStream_t stream) {
+    auto kern = dw3x3_bwd_packed_kernel<T, AF, RL, EPI, ZO>;
     static bool configured[64] = {};
     if (spnet_first_use_on_device(configured)) {
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024);
@@ -581,21 +616,24 @@ int launch_bwd_inst(const CUtensorMap& tg, const CUtensorMap& tx, const CUtensor
             return SPNET_ERR_CUDA;
         }
     }
-    kern<<<dim3(t.grid_x, t.chunks), t.threads, t.smem, stream>>>(tg, tx, ta, k, a, b, mean, rstd, stats, sadd, gin, dk,
-                                                                  dk_acc, B, H, W, C, t.TH, t.TW, t.tiles_h, t.tiles_w, t.S);
+    kern<<<dim3(t.grid_x, t.chunks), t.threads, t.smem, stream>>>(tg, tx, ta, tz, ma, mb, k, a, b, mean, rstd, stats,
+                                                                  sadd, gin, dk, dk_acc, B, H, W, C, t.TH, t.TW,
+                                                                  t.tiles_h, t.tiles_w, t.S);
     return spnet_check_launch("dw3x3_bwd_fused");
 }
 
 template <typename T>
 int launch_bwd(const void* gout, const void* in, const float* k, const float* a, const float* b, int relu,
                const float* mean, const float* rstd, long long* stats, const void* add_src, const void* add_strided,
-               void* gin, float* dk, long long* dk_acc, int dtype, int B, int H, int W, int C, cudaStream_t stream) {
+               void* gin, float* dk, long long* dk_acc, const void* zo, const float* zo_mean, const float* zo_rstd,
+               long long* zo_stats, const float* mask_a, const float* mask_b, int dtype, int B, int H, int W, int C,
+               cudaStream_t stream) {
     const int epi = add_src ? 1 : (add_strided ? 2 : 0);
-    Tiling t = pick_tiling(epi == 1 ? 2 : 1, dtype, B, H, W, C);
+    Tiling t = pick_tiling(1 + (epi == 1) + (zo != nullptr), dtype, B, H, W, C);
     SPNET_REQUIRE(t.TH > 0, "dwconv3x3_bwd: no tile fits shared memory");
     const size_t red_bytes = (size_t)(t.TW / 2) * 11 * CB * 4 + 128;
     if (t.smem < red_bytes) t.smem = red_bytes;
-    CUtensorMap tg, tx, ta;
+    CUtensorMap tg, tx, ta, tz;
     int rc = make_map(&tg, gout, dtype, B, H, W, C, t.TW + 2, t.TH + 2, false);
     if (rc) return rc;
     rc = make_map(&tx, in, dtype, B, H, W, C, t.TW, t.TH, false);
@@ -604,11 +642,26 @@ int launch_bwd(const void* gout, const void* in, const float* k, const float* a,
     if (rc) return rc;
     const T* sadd = reinterpret_cast<const T*>(add_strided);
     T* y = reinterpret_cast<T*>(gin);
+    if (zo) {
+        // the combinations XceptionSPNetEngine runs: the first sepconv of a block (input not BN'd), after the
+        // residual add of a middle block (EPI 1) or of a stride-2 block (EPI 2), or without one (block 14)
+        rc = make_map(&tz, zo, dtype, B, H, W, C, t.TW, t.TH, false);
+        if (rc) return rc;
+        SPNET_REQUIRE(!a && (epi == 1 ? relu == 1 : (epi == 2 ? relu <= 1 : relu == 0)),
+                      "dwconv3x3_bwd_fused: zo is not instantiated for in_a=%s relu=%d epilogue=%d", a ? "set" : "null",
+                      relu, epi);
+#define DWZ(RL, EPI) launch_bwd_inst<T, false, RL, EPI, true>(tg, tx, ta, tz, mask_a, mask_b, k, a, b, zo_mean, zo_rstd, \
+                                                              zo_stats, sadd, y, dk, dk_acc, B, H, W, C, t, stream)
+        if (epi == 1) return DWZ(1, 1);
+        if (epi == 2) return relu ? DWZ(1, 2) : DWZ(0, 2);
+        return DWZ(0, 0);
+#undef DWZ
+    }
 #define DWB(AF, RL)                                                                                                    \
     do {                                                                                                               \
-        if (epi == 1) return launch_bwd_inst<T, AF, RL, 1>(tg, tx, ta, k, a, b, mean, rstd, stats, sadd, y, dk, dk_acc, B, H, W, C, t, stream); \
-        if (epi == 2) return launch_bwd_inst<T, AF, RL, 2>(tg, tx, ta, k, a, b, mean, rstd, stats, sadd, y, dk, dk_acc, B, H, W, C, t, stream); \
-        return launch_bwd_inst<T, AF, RL, 0>(tg, tx, ta, k, a, b, mean, rstd, stats, sadd, y, dk, dk_acc, B, H, W, C, t, stream);   \
+        if (epi == 1) return launch_bwd_inst<T, AF, RL, 1, false>(tg, tx, ta, tx, nullptr, nullptr, k, a, b, mean, rstd, stats, sadd, y, dk, dk_acc, B, H, W, C, t, stream); \
+        if (epi == 2) return launch_bwd_inst<T, AF, RL, 2, false>(tg, tx, ta, tx, nullptr, nullptr, k, a, b, mean, rstd, stats, sadd, y, dk, dk_acc, B, H, W, C, t, stream); \
+        return launch_bwd_inst<T, AF, RL, 0, false>(tg, tx, ta, tx, nullptr, nullptr, k, a, b, mean, rstd, stats, sadd, y, dk, dk_acc, B, H, W, C, t, stream);   \
     } while (0)
     if (a && relu == 2) DWB(true, 2);
     if (a && relu) DWB(true, 1);
@@ -648,17 +701,25 @@ int spnet_dwconv3x3_fwd(const void* in, const float* k, const float* in_a, const
 //   dk_acc      : nullable accumulators, 9*C entries: the kernel-gradient partial sums of the CTAs go there (order-
 //                 independent, spnet_acc_to_f32 adds them into dk) instead of fp32 atomics on dk
 //   add_src / add_strided : optional residual-path gradients added to gin (at most one of them)
+//   zo          : nullable, same shape as gin: the raw input of the BatchNorm whose output gradient gin is. Then
+//                 zo_stats (2*C entries) += (sum gin, sum gin*xhat), xhat = (zo-zo_mean)*zo_rstd, over the final gin;
+//                 with mask_a/mask_b (nullable pair) gin is first zeroed where !(mask_a*zo+mask_b > 0), the ReLU that
+//                 followed that BatchNorm. Exclusive with stats; implemented for in_a = null, relu 0 or 1.
 int spnet_dwconv3x3_bwd_fused(const void* gout, const void* in, const float* k, const float* in_a, const float* in_b,
                               int relu, const float* bn_mean, const float* bn_rstd, long long* stats, const void* add_src,
                               const void* add_strided, void* gin, float* dk, long long* dk_acc, int dtype, int B, int H,
-                              int W, int C, cudaStream_t stream) {
+                              int W, int C, const void* zo, const float* zo_mean, const float* zo_rstd,
+                              long long* zo_stats, const float* mask_a, const float* mask_b, cudaStream_t stream) {
     int rc = check_args("dwconv3x3_bwd_fused", gout, gin, dtype, B, H, W, C);
     if (rc) return rc;
     SPNET_REQUIRE(in && k && dk && ((in_a == nullptr) == (in_b == nullptr)) && relu >= 0 && relu <= 2, "dwconv3x3_bwd_fused: bad pointers or relu code");
     SPNET_REQUIRE(!stats || (bn_mean && bn_rstd), "dwconv3x3_bwd_fused: stats need bn_mean / bn_rstd");
     SPNET_REQUIRE(!(add_src && add_strided), "dwconv3x3_bwd_fused: add_src and add_strided are exclusive");
+    SPNET_REQUIRE(!zo || (zo_mean && zo_rstd && zo_stats && !stats), "dwconv3x3_bwd_fused: zo needs zo_mean / zo_rstd / zo_stats and excludes stats");
+    SPNET_REQUIRE((mask_a == nullptr) == (mask_b == nullptr) && (!mask_a || zo), "dwconv3x3_bwd_fused: mask_a / mask_b come in pairs, with zo");
     SPNET_DISPATCH_DTYPE(dtype, return launch_bwd<T>(gout, in, k, in_a, in_b, relu, bn_mean, bn_rstd, stats, add_src,
-                                                     add_strided, gin, dk, dk_acc, dtype, B, H, W, C, stream));
+                                                     add_strided, gin, dk, dk_acc, zo, zo_mean, zo_rstd, zo_stats, mask_a,
+                                                     mask_b, dtype, B, H, W, C, stream));
 }
 
 }  // extern "C"

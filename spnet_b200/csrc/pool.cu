@@ -232,7 +232,53 @@ __global__ void __launch_bounds__(256) maxpool_add_fwd_bf16_kernel(const bf16* _
 // the block lies inside window (j, i) - taps (0..1, 0..1) - and its first row / column are taps 2 of windows
 // j-1 / i-1, so FOUR (gout, argmax) loads serve four outputs (one item per input position needed four loads
 // each, 7 of every 16 of them for windows that cannot contain the position). The sums run in the order
-// (j,i), (j,i-1), (j-1,i), (j-1,i-1).
+// (j,i), (j,i-1), (j-1,i), (j-1,i-1). a[k] = gradient of block position k = 2*(row - r0) + (column - q0).
+template <typename T, int V>
+__device__ __forceinline__ void maxpool_bwd_item(const T* __restrict__ gout, const unsigned char* __restrict__ argmax,
+                                                 int bi, int j, int i, int c0, int C, int OH, int OW, float (&a)[4][V]) {
+    const bool okj0 = j < OH, okj1 = j >= 1 && j - 1 < OH;  // windows j and j-1 exist
+    const bool oki0 = i < OW, oki1 = i >= 1 && i - 1 < OW;
+    // windows in summation order: (j,i) (j,i-1) (j-1,i) (j-1,i-1)
+    const bool okw[4] = {okj0 && oki0, okj0 && oki1, okj1 && oki0, okj1 && oki1};
+    float g[4][V];
+    uint32_t am[4][2];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        const int oh = (k < 2) ? (okj0 ? j : 0) : (okj1 ? j - 1 : 0);
+        const int ow = (k & 1) ? (oki1 ? i - 1 : 0) : (oki0 ? i : 0);
+        const size_t o = (((size_t)bi * OH + oh) * OW + ow) * C + c0;
+        load_vec(gout + o, g[k]);
+        if (V == 8) {
+            const uint2 q = *reinterpret_cast<const uint2*>(argmax + o);
+            am[k][0] = q.x; am[k][1] = q.y;
+        } else {
+            am[k][0] = *reinterpret_cast<const uint32_t*>(argmax + o); am[k][1] = 0;
+        }
+        if (!okw[k]) { am[k][0] = 0xffffffffu; am[k][1] = 0xffffffffu; }  // code 255: matches no tap
+    }
+#pragma unroll
+    for (int e = 0; e < V; ++e) {
+        const int sh = 8 * (e & 3), wd = e >> 2;
+        const uint32_t k0 = (am[0][wd] >> sh) & 0xffu, k1 = (am[1][wd] >> sh) & 0xffu;
+        const uint32_t k2 = (am[2][wd] >> sh) & 0xffu, k3 = (am[3][wd] >> sh) & 0xffu;
+        float s = 0.f;
+        if (k0 == 0u) s += g[0][e];
+        if (k1 == 2u) s += g[1][e];
+        if (k2 == 6u) s += g[2][e];
+        if (k3 == 8u) s += g[3][e];
+        a[0][e] = s;
+        s = 0.f;
+        if (k0 == 1u) s += g[0][e];
+        if (k2 == 7u) s += g[2][e];
+        a[1][e] = s;
+        s = 0.f;
+        if (k0 == 3u) s += g[0][e];
+        if (k1 == 5u) s += g[1][e];
+        a[2][e] = s;
+        a[3][e] = (k0 == 4u) ? g[0][e] : 0.f;
+    }
+}
+
 template <typename T>
 __global__ void __launch_bounds__(256) maxpool_bwd_kernel(const T* __restrict__ gout,
                                                           const unsigned char* __restrict__ argmax,
@@ -245,58 +291,101 @@ __global__ void __launch_bounds__(256) maxpool_bwd_kernel(const T* __restrict__ 
     const int items = WP * CV;
     const int r0 = 2 * j - pt, r1 = r0 + 1;
     const bool okr0 = r0 >= 0, okr1 = r1 < H;             // r0 < H and r1 >= 0 by construction of HP
-    const bool okj0 = j < OH, okj1 = j >= 1 && j - 1 < OH;  // windows j and j-1 exist
     for (int it = blockIdx.y * blockDim.x + threadIdx.x; it < items; it += blockDim.x * gridDim.y) {
         const int i = it / CV, cv = it - i * CV;
         const int c0 = cv * V;
         const int q0 = 2 * i - pl, q1 = q0 + 1;
         const bool okq0 = q0 >= 0, okq1 = q1 < W;
-        const bool oki0 = i < OW, oki1 = i >= 1 && i - 1 < OW;
-        // windows in summation order: (j,i) (j,i-1) (j-1,i) (j-1,i-1)
-        const bool okw[4] = {okj0 && oki0, okj0 && oki1, okj1 && oki0, okj1 && oki1};
-        float g[4][V];
-        uint32_t am[4][2];
+        float a[4][V];
+        maxpool_bwd_item<T, V>(gout, argmax, bi, j, i, c0, C, OH, OW, a);
+        T* base = gin + (((size_t)bi * H + r0) * W + q0) * C + c0;
+        if (okr0 && okq0) store_vec(base, a[0]);
+        if (okr0 && okq1) store_vec(base + C, a[1]);
+        if (okr1 && okq0) store_vec(base + (size_t)W * C, a[2]);
+        if (okr1 && okq1) store_vec(base + (size_t)W * C + C, a[3]);
+    }
+}
+
+// The same gin, plus the BatchNorm-backward sums of the BN that produced the pooled tensor (z = its raw input):
+//   stats[c] += sum gin,  stats[C+c] += sum gin * xhat,  xhat = z*rstd - mean*rstd  (as bn_bwd_reduce_kernel),
+// over gin as stored. Channel-stationary: a thread keeps one channel vector and walks the items of its CTA's
+// contiguous range, its partial sums in registers; one CTA per SM and ONE flush per CTA, so that the per-address
+// fp64-atomic chains stay ~148 deep (a flush per tensor row would build chains thousands deep).
+template <typename T>
+__global__ void __launch_bounds__(512, 1) maxpool_bwd_stats_kernel(const T* __restrict__ gout,
+                                                                   const unsigned char* __restrict__ argmax,
+                                                                   T* __restrict__ gin, const T* __restrict__ z,
+                                                                   const float* __restrict__ mean,
+                                                                   const float* __restrict__ rstd,
+                                                                   long long* __restrict__ stats, int B, int H, int W,
+                                                                   int C, int OH, int OW, int pt, int pl, int HP, int WP,
+                                                                   int cvb, int krows) {
+    constexpr int V = VecN<T>::N;
+    const int CV = C / V;
+    const int cvl = threadIdx.x % cvb, rl = threadIdx.x / cvb;
+    const int cv = blockIdx.y * cvb + cvl;
+    const bool active = cv < CV;
+    const int c0 = cv * V;
+    float s1[V], s2[V];
 #pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            const int oh = (k < 2) ? (okj0 ? j : 0) : (okj1 ? j - 1 : 0);
-            const int ow = (k & 1) ? (oki1 ? i - 1 : 0) : (oki0 ? i : 0);
-            const size_t o = (((size_t)bi * OH + oh) * OW + ow) * C + c0;
-            load_vec(gout + o, g[k]);
-            if (V == 8) {
-                const uint2 q = *reinterpret_cast<const uint2*>(argmax + o);
-                am[k][0] = q.x; am[k][1] = q.y;
-            } else {
-                am[k][0] = *reinterpret_cast<const uint32_t*>(argmax + o); am[k][1] = 0;
+    for (int e = 0; e < V; ++e) s1[e] = s2[e] = 0.f;
+    if (active) {
+        float rs[V], nm[V];
+        load_coef<V>(rstd, c0, rs);
+        load_coef<V>(mean, c0, nm);
+#pragma unroll
+        for (int e = 0; e < V; ++e) nm[e] = -nm[e] * rs[e];
+        const int items = B * HP * WP;  // < 2^31: check_pool bounds B*H*W*C
+        const int per_cta = (items + gridDim.x - 1) / gridDim.x;
+        const int begin = blockIdx.x * per_cta, end = min(begin + per_cta, items);
+        for (int p = begin + rl; p < end; p += krows) {
+            const int bj = p / WP, i = p - bj * WP;
+            const int bi = bj / HP, j = bj - bi * HP;
+            const int r0 = 2 * j - pt, q0 = 2 * i - pl;
+            const bool ok[4] = {r0 >= 0 && q0 >= 0, r0 >= 0 && q0 + 1 < W, r0 + 1 < H && q0 >= 0, r0 + 1 < H && q0 + 1 < W};
+            // z of the four positions (clamped addresses, flagged by ok) is in flight with the gradient loads
+            const int rc0 = max(r0, 0), rc1 = min(r0 + 1, H - 1), qc0 = max(q0, 0), qc1 = min(q0 + 1, W - 1);
+            const T* zb = z + ((size_t)bi * H) * W * C + c0;
+            float zv[4][V];
+            load_vec(zb + ((size_t)rc0 * W + qc0) * C, zv[0]);
+            load_vec(zb + ((size_t)rc0 * W + qc1) * C, zv[1]);
+            load_vec(zb + ((size_t)rc1 * W + qc0) * C, zv[2]);
+            load_vec(zb + ((size_t)rc1 * W + qc1) * C, zv[3]);
+            float a[4][V];
+            maxpool_bwd_item<T, V>(gout, argmax, bi, j, i, c0, C, OH, OW, a);
+            T* base = gin + (((size_t)bi * H + r0) * W + q0) * C + c0;
+            const size_t off[4] = {0, (size_t)C, (size_t)W * C, (size_t)W * C + C};
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                if (!ok[k]) continue;
+                store_vec(base + off[k], a[k]);
+#pragma unroll
+                for (int e = 0; e < V; ++e) {
+                    const float v = round_to<T>(a[k][e]);
+                    s1[e] += v;
+                    s2[e] = fmaf(v, fmaf(zv[k][e], rs[e], nm[e]), s2[e]);
+                }
             }
-            if (!okw[k]) { am[k][0] = 0xffffffffu; am[k][1] = 0xffffffffu; }  // code 255: matches no tap
         }
-        float a00[V], a01[V], a10[V], a11[V];
+    }
+    __shared__ float red[2][512 * 8];
+#pragma unroll
+    for (int e = 0; e < V; ++e) {
+        red[0][threadIdx.x * V + e] = s1[e];
+        red[1][threadIdx.x * V + e] = s2[e];
+    }
+    __syncthreads();
+    if (rl == 0 && active) {
 #pragma unroll
         for (int e = 0; e < V; ++e) {
-            const int sh = 8 * (e & 3), wd = e >> 2;
-            const uint32_t k0 = (am[0][wd] >> sh) & 0xffu, k1 = (am[1][wd] >> sh) & 0xffu;
-            const uint32_t k2 = (am[2][wd] >> sh) & 0xffu, k3 = (am[3][wd] >> sh) & 0xffu;
-            float s = 0.f;
-            if (k0 == 0u) s += g[0][e];
-            if (k1 == 2u) s += g[1][e];
-            if (k2 == 6u) s += g[2][e];
-            if (k3 == 8u) s += g[3][e];
-            a00[e] = s;
-            s = 0.f;
-            if (k0 == 1u) s += g[0][e];
-            if (k2 == 7u) s += g[2][e];
-            a01[e] = s;
-            s = 0.f;
-            if (k0 == 3u) s += g[0][e];
-            if (k1 == 5u) s += g[1][e];
-            a10[e] = s;
-            a11[e] = (k0 == 4u) ? g[0][e] : 0.f;
+            float t1 = 0.f, t2 = 0.f;
+            for (int r = 0; r < krows; ++r) {
+                t1 += red[0][(r * cvb + cvl) * V + e];
+                t2 += red[1][(r * cvb + cvl) * V + e];
+            }
+            stat_add(stats, c0 + e, (double)t1);
+            stat_add(stats, C + c0 + e, (double)t2);
         }
-        T* base = gin + (((size_t)bi * H + r0) * W + q0) * C + c0;
-        if (okr0 && okq0) store_vec(base, a00);
-        if (okr0 && okq1) store_vec(base + C, a01);
-        if (okr1 && okq0) store_vec(base + (size_t)W * C, a10);
-        if (okr1 && okq1) store_vec(base + (size_t)W * C + C, a11);
     }
 }
 
@@ -389,15 +478,33 @@ int spnet_maxpool3s2_add_fwd(const void* z, const float* a, const float* b, cons
     return spnet_check_launch("maxpool3s2_add_fwd");
 }
 
+// z, mean, rstd, stats (all or none): also stats[2*C] += (sum gin, sum gin*xhat), xhat = (z-mean)*rstd, over gin as
+// stored, the BatchNorm-backward sums of the BN whose output was pooled (z = its raw input, [B,H,W,C] like gin)
 int spnet_maxpool3s2_bwd(const void* gout, const unsigned char* argmax, void* gin, int dtype, int B, int H, int W,
-                         int C, cudaStream_t stream) {
+                         int C, const void* z, const float* mean, const float* rstd, long long* stats,
+                         cudaStream_t stream) {
     int rc = check_pool("maxpool3s2_bwd", dtype, B, H, W, C);
     if (rc) return rc;
     SPNET_REQUIRE(gout && argmax && gin, "maxpool3s2_bwd: null pointer");
+    SPNET_REQUIRE((z == nullptr) == (stats == nullptr) && (z == nullptr) == (mean == nullptr) &&
+                      (z == nullptr) == (rstd == nullptr), "maxpool3s2_bwd: z, mean, rstd and stats come together");
     const int OH = (H + 1) / 2, OW = (W + 1) / 2;
     const int V = dtype == SPNET_BF16 ? 8 : 4;
     const int pt = same_pad_before(H), pl = same_pad_before(W);
     const int HP = (H - 1 + pt) / 2 + 1, WP = (W - 1 + pl) / 2 + 1;  // 2 x 2 blocks of input positions
+    if (z) {
+        // up to 128 channel vectors per CTA, the rest of 512 threads on items; one CTA per SM
+        const int CV = C / V, nchunks = ceil_div(CV, 128);
+        const int cvb = ceil_div(CV, nchunks), krows = 512 / cvb > 0 ? 512 / cvb : 1;
+        long long gx = ceil_div((long long)B * HP * WP, krows);
+        const long long cap = spnet_num_sms() / nchunks > 0 ? spnet_num_sms() / nchunks : 1;
+        if (gx > cap) gx = cap;
+        SPNET_DISPATCH_DTYPE(dtype, (maxpool_bwd_stats_kernel<T><<<dim3((unsigned)gx, nchunks), cvb * krows, 0, stream>>>(
+                                        reinterpret_cast<const T*>(gout), argmax, reinterpret_cast<T*>(gin),
+                                        reinterpret_cast<const T*>(z), mean, rstd, stats, B, H, W, C, OH, OW, pt, pl, HP,
+                                        WP, cvb, krows)));
+        return spnet_check_launch("maxpool3s2_bwd_stats");
+    }
     SPNET_DISPATCH_DTYPE(dtype, (maxpool_bwd_kernel<T><<<row_grid(B * HP, WP * (C / V)), 256, 0, stream>>>(
                                     reinterpret_cast<const T*>(gout), argmax, reinterpret_cast<T*>(gin), B, H, W, C,
                                     OH, OW, pt, pl, HP, WP)));

@@ -344,21 +344,29 @@ class SPNetEngineBase:
             ops.acc_to_f32(self.l2_acc, self.l2_out)
 
     # ------------------------------------------------------------------ backward
-    def _sep_bwd(self, s, gz, x, in_bn, relu, g_t, g_in, add_src=None, add_strided=None, wgrad=True):
+    def _sep_bwd(self, s, gz, x, in_bn, relu, g_t, g_in, add_src=None, add_strided=None, wgrad=True, out_bn=None):
         """gz: grad wrt s.z [B,H,W,cout]. Produces the gradient wrt the sepconv's input tensor x
         (before its on-load BN/ReLU transform) in g_in; for a BN'd input this is still the grad wrt
-        the BN OUTPUT (masked by relu'), to be pushed through _bn_bwd by the caller."""
+        the BN OUTPUT (masked by relu'), to be pushed through _bn_bwd by the caller.
+        out_bn = (z, bn, relu_mask): x = [relu](bn(z)) [+ ...], the BN that produced the UNtransformed input x. The
+        depthwise backward then accumulates that BN's backward sums on the final g_in (masked by the ReLU when
+        relu_mask), so the caller's _bn_bwd on g_in runs with reduced=True."""
         B = self.B
         M = B * s.H * s.W
         self._pw_bwd(s.t, s.pwl, s.gpw if wgrad else None, gz, g_t, M, s.cin, s.cout)
         gt4 = g_t.view(B, s.H, s.W, s.cin)
+        zo, zbn, zmask = out_bn if out_bn else (None, None, False)
         ops.dwconv3x3_bwd_fused(gt4, x, s.dwk, s.gdwk, in_a=in_bn.a if in_bn else None, in_b=in_bn.b if in_bn else None,
                                 relu=relu, bn_mean=in_bn.mean if in_bn else None, bn_rstd=in_bn.rstd if in_bn else None,
                                 stats=in_bn.stats if in_bn else None, add_src=add_src, add_strided=add_strided,
-                                out=g_in.view(B, s.H, s.W, s.cin), acc=self._gacc)
+                                out=g_in.view(B, s.H, s.W, s.cin), acc=self._gacc,
+                                zo=zo, zo_mean=zbn.mean if zbn else None, zo_rstd=zbn.rstd if zbn else None,
+                                zo_stats=zbn.stats if zbn else None, mask_a=zbn.a if zmask else None,
+                                mask_b=zbn.b if zmask else None)
 
-    def _entry_bwd(self, e, x, g_out, bufs):
-        """g_out: grad wrt block output [B,oh,ow,c]. Returns grad wrt block input x."""
+    def _entry_bwd(self, e, x, g_out, bufs, x_bn):
+        """g_out: grad wrt block output [B,oh,ow,c], its residual BN's backward sums already accumulated (by the
+        producer of g_out). Returns grad wrt block input x, with the sums of x's BN x_bn = (z, bn, relu_mask)."""
         B = self.B
         (H, W), (oh, ow) = e["hw"], e["ohw"]
         cin, c = e["cin"], e["c"]
@@ -367,19 +375,20 @@ class SPNetEngineBase:
         M = B * H * W
         s1, s2 = e["sep1"], e["sep2"]
         # residual branch
-        g_zr = self._bn_bwd(g_out, e["zr"], e["res_bn"], Mo, out=self._view(G1, B, oh, ow, c))
+        g_zr = self._bn_bwd(g_out, e["zr"], e["res_bn"], Mo, out=self._view(G1, B, oh, ow, c), reduced=True)
         g_xs = self._view(S, Mo, cin)
         self._pw_bwd(e["xs"].view(Mo, cin), self.wl[e["res"] + "/kernel"].view(cin, c),
                      self.g[e["res"] + "/kernel"].view(cin, c), g_zr.view(Mo, c), g_xs, Mo, cin, c)
         # main branch
-        g_y2 = ops.maxpool3s2_bwd(g_out, e["argmax"], H, W, out=self._view(G1, B, H, W, c))
-        g_z2 = self._bn_bwd(g_y2, s2.z, s2.bn, M)
+        g_y2 = ops.maxpool3s2_bwd(g_out, e["argmax"], H, W, out=self._view(G1, B, H, W, c), z=s2.z, mean=s2.bn.mean,
+                                  rstd=s2.bn.rstd, stats=s2.bn.stats)
+        g_z2 = self._bn_bwd(g_y2, s2.z, s2.bn, M, reduced=True)
         g_y1 = self._view(G3, B, H, W, s2.cin)
         self._sep_bwd(s2, g_z2.view(M, c), s1.z, s1.bn, True, self._view(G2, M, s2.cin), g_y1)
         g_z1 = self._bn_bwd(g_y1, s1.z, s1.bn, M, reduced=True)
         g_x = self._view(R, B, H, W, cin)
         self._sep_bwd(s1, g_z1.view(M, s1.cout), x, None, e["relu_in"], self._view(G1, M, cin), g_x,
-                      add_strided=g_xs.view(B, oh, ow, cin))
+                      add_strided=g_xs.view(B, oh, ow, cin), out_bn=x_bn)
         return g_x
 
     def backward_head(self):
@@ -774,11 +783,13 @@ class XceptionSPNetEngine(SPNetEngineBase):
         self._sep_bwd(s2, g_z.view(M, 2048), s1.z, s1.bn, True, self._view(G2, M, 1536), g_y)
         g_z = self._bn_bwd(g_y, s1.z, s1.bn, M, reduced=True)
         g_x = self._view(R0, B, fh, fw, 1024)
-        self._sep_bwd(s1, g_z.view(M, 1536), x13, None, False, self._view(G1, M, 1024), g_x)
+        self._sep_bwd(s1, g_z.view(M, 1536), x13, None, False, self._view(G1, M, 1024), g_x,
+                      out_bn=(self.exit13["zr"], self.exit13["res_bn"], False))
         # ---- exit block 13
         R_cur, R_nxt = R0, R1
         x_in13 = self.mid_out[-1]
-        g_x = self._entry_bwd(self.exit13, x_in13, g_x, (G1, G2, G3, S, R_nxt))
+        g_x = self._entry_bwd(self.exit13, x_in13, g_x, (G1, G2, G3, S, R_nxt),
+                              (self.middle[-1][2].z, self.middle[-1][2].bn, False))
         R_cur, R_nxt = R_nxt, R_cur
         # ---- middle blocks 12..5
         mh, mw = sh["middle"]
@@ -787,9 +798,12 @@ class XceptionSPNetEngine(SPNetEngineBase):
         for i in range(len(self.middle) - 1, -1, -1):
             blk = self.middle[i]
             x_in = self.mid_out[i - 1] if i > 0 else self.entry[-1]["out"]
+            # the BN on x_in's residual path: the previous middle block's sepconv3 BN or entry block 4's residual BN
+            x_bn = (self.middle[i - 1][2].z, self.middle[i - 1][2].bn, False) if i > 0 else \
+                (self.entry[-1]["zr"], self.entry[-1]["res_bn"], False)
             # with the batched weight gradient every dz is kept (mid_dz) until the end of the middle flow
             dz3, dz2, dz1 = (self.mid_dz[3 * i + 2], self.mid_dz[3 * i + 1], self.mid_dz[3 * i]) if bat else (None, None, None)
-            g3 = self._bn_bwd(g_x, blk[2].z, blk[2].bn, M, out=dz3 if bat else self._view(G1, B, mh, mw, 728))
+            g3 = self._bn_bwd(g_x, blk[2].z, blk[2].bn, M, out=dz3 if bat else self._view(G1, B, mh, mw, 728), reduced=True)
             gy2 = self._view(G3, B, mh, mw, 728)
             self._sep_bwd(blk[2], g3.view(M, 728), blk[1].z, blk[1].bn, True, self._view(G2, M, 728), gy2, wgrad=not bat)
             g2 = self._bn_bwd(gy2, blk[1].z, blk[1].bn, M, reduced=True, out=dz2)
@@ -797,7 +811,8 @@ class XceptionSPNetEngine(SPNetEngineBase):
             self._sep_bwd(blk[1], g2.view(M, 728), blk[0].z, blk[0].bn, True, self._view(G2, M, 728), gy1, wgrad=not bat)
             g1 = self._bn_bwd(gy1, blk[0].z, blk[0].bn, M, reduced=True, out=dz1)
             g_new = self._view(R_nxt, B, mh, mw, 728)
-            self._sep_bwd(blk[0], g1.view(M, 728), x_in, None, True, self._view(G2, M, 728), g_new, add_src=g_x, wgrad=not bat)
+            self._sep_bwd(blk[0], g1.view(M, 728), x_in, None, True, self._view(G2, M, 728), g_new, add_src=g_x, wgrad=not bat,
+                          out_bn=x_bn)
             g_x = g_new
             R_cur, R_nxt = R_nxt, R_cur
         if bat:
@@ -819,13 +834,16 @@ class XceptionSPNetEngine(SPNetEngineBase):
         for i in range(len(self.entry) - 1, -1, -1):
             e = self.entry[i]
             x_in = self.entry[i - 1]["out"] if i > 0 else self.x2
-            g_x = self._entry_bwd(e, x_in, g_x, (G1, G2, G3, S, R_nxt))
+            x_bn = (self.entry[i - 1]["zr"], self.entry[i - 1]["res_bn"], False) if i > 0 else \
+                (self.z12, self.b1_bn2, True)  # x2 = relu(BN(z12))
+            g_x = self._entry_bwd(e, x_in, g_x, (G1, G2, G3, S, R_nxt), x_bn)
             R_cur, R_nxt = R_nxt, R_cur
         # ---- block 1
         h2, w2 = sh["b1c2"]
         h1, w1 = sh["b1c1"]
         M2 = B * h2 * w2
-        g_z12 = self._bn_bwd(g_x, self.z12, self.b1_bn2, M2, relu_mask=True)
+        # masked by the block-1 ReLU, with its sums, by block2_sepconv1's depthwise backward
+        g_z12 = self._bn_bwd(g_x, self.z12, self.b1_bn2, M2, reduced=True)
         W2l = self.wl["block1_conv2/kernel"].view(288, 64)
         g_y11 = self._view(G1, B, h1, w1, 32)
         if self.b1_fold:

@@ -84,15 +84,18 @@ def dwconv3x3_fwd(x, k, in_a=None, in_b=None, relu=False, out=None):
 
 
 def dwconv3x3_bwd_fused(gout, x, k, dk, in_a=None, in_b=None, relu=False, bn_mean=None, bn_rstd=None, stats=None,
-                        add_src=None, add_strided=None, out=None, acc=None):
-    """gin, dk (+=) and optional BatchNorm-backward sums in one pass (see dwconv_packed.cu)."""
-    _chk(gout, x, k, dk, in_a, in_b, stats, add_src, add_strided, out)
+                        add_src=None, add_strided=None, out=None, acc=None, zo=None, zo_mean=None, zo_rstd=None,
+                        zo_stats=None, mask_a=None, mask_b=None):
+    """gin, dk (+=) and optional BatchNorm-backward sums in one pass (see dwconv_packed.cu).
+    zo: raw input of the BatchNorm whose output gradient gin is; its sums go to zo_stats, taken on the final gin,
+    which is first masked by (mask_a*zo + mask_b > 0) when mask_a/mask_b are given."""
+    _chk(gout, x, k, dk, in_a, in_b, stats, add_src, add_strided, out, zo, zo_mean, zo_rstd, zo_stats, mask_a, mask_b)
     B, H, W, C = gout.shape
     if out is None:
         out = torch.empty_like(gout)
     lib().dwconv3x3_bwd_fused(_p(gout), _p(x), _p(k), _p(in_a), _p(in_b), int(relu), _p(bn_mean), _p(bn_rstd),
                               _p(stats), _p(add_src), _p(add_strided), _p(out), _p(dk), _p(acc), dtype_code(gout), B, H, W, C,
-                              _s())
+                              _p(zo), _p(zo_mean), _p(zo_rstd), _p(zo_stats), _p(mask_a), _p(mask_b), _s())
     if acc is not None:  # order-independent kernel gradient: accumulators -> dk (+=), accumulators cleared
         lib().acc_to_f32(_p(acc), _p(dk), dk.numel(), 1, 1, _s())
     return out
@@ -281,12 +284,15 @@ def maxpool3s2_add_fwd(z, a=None, b=None, res=None, ra=None, rb=None, out=None, 
     return out
 
 
-def maxpool3s2_bwd(gout, argmax, H, W, out=None):
-    _chk(gout, argmax, out)
+def maxpool3s2_bwd(gout, argmax, H, W, out=None, z=None, mean=None, rstd=None, stats=None):
+    """gin; with z (the raw input of the BatchNorm whose output was pooled) also that BatchNorm's backward sums
+    (sum gin, sum gin*xhat) into stats, over gin as stored."""
+    _chk(gout, argmax, out, z, mean, rstd, stats)
     B, OH, OW, C = gout.shape
     if out is None:
         out = torch.empty(B, H, W, C, device=gout.device, dtype=gout.dtype)
-    lib().maxpool3s2_bwd(_p(gout), _p(argmax), _p(out), dtype_code(gout), B, H, W, C, _s())
+    lib().maxpool3s2_bwd(_p(gout), _p(argmax), _p(out), dtype_code(gout), B, H, W, C, _p(z), _p(mean), _p(rstd),
+                         _p(stats), _s())
     return out
 
 
