@@ -92,6 +92,14 @@ int spnet_dwconv3x3_bwd_fused(const void* gout, const void* in, const float* k, 
  *      of Xception's 24 identical middle-flow layers, written straight into the flat gradient buffer). ---- */
 int spnet_gemm_bf16(const void* A, long long lda, int a_mn, const void* B, long long ldb, int b_mn, void* D, long long ldd, long long slab_stride, int out_mode, int M, int N, int K, int splits, long long* colstats, cudaStream_t stream);
 int spnet_gemm_simt(const float* A, long long sa_r, long long sa_k, const float* B, long long sb_r, long long sb_k, float* D, long long ldd, long long slab_stride, int out_mode, int M, int N, int K, int splits, long long* colstats, cudaStream_t stream);
+/* Backward of a pointwise conv whose output z [M, cout] feeds a BatchNorm, in one pass (pw_bwd.cu; bf16, cout = 128,
+ * cin = 64 or 128: Xception's block-2 pointwise and residual convs). g = gradient wrt the BN output, with
+ * spnet_bn_bwd_finalize already run (c1, c2); t [M, cin] = the conv input; W [cin, cout] its bf16 kernel.
+ * dz = the value spnet_bn_bwd_dz would store, kept in shared memory; gA [M, cin] = dz W^T (bf16, the value
+ * spnet_gemm_bf16 stores for that product); gW [cin, cout] fp32 += t^T dz by reduce-add, or, with slabs, CTA s stores
+ * its partial sum at slabs + s * cin * cout for s < nslabs (1 <= nslabs <= ceil(M/128); the caller adds them in
+ * order with spnet_slab_reduce). gA must not alias g, z or t. */
+int spnet_pw_bwd_bn(const void* g, const void* z, const void* t, const void* W, const float* a, const float* save_mean, const float* save_rstd, const float* c1, const float* c2, void* gA, float* gW, float* slabs, int nslabs, int M, int cin, int cout, cudaStream_t stream);
 
 /* ---- Conv2D k x k, stride 1, as implicit GEMM on tcgen05 (gemm_tc.cu, no im2col buffer): Xception
  *      block1_conv2 (keras.applications.Xception; spnet/models.py:359) and the InceptionResNetV2 branch

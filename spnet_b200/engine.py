@@ -274,6 +274,17 @@ class SPNetEngineBase:
         if gA is not None:
             ops.gemm(gz, False, Wl, False, gA, M, K, N, out_mode=ops.OUT_T, ldb=N)
 
+    def _pw_bwd_fusable(self, K, N):
+        """The BatchNorm backward and both pointwise GEMMs of a K -> N layer run as one kernel (csrc/pw_bwd.cu)."""
+        return self.lowp and N == 128 and K in (64, 128)
+
+    def _bn_pw_bwd(self, g, z, bn, A, Wl, gW, gA, M, K, N):
+        """g = grad wrt the output of the BatchNorm of z = A W -> gA [M,K] = dz W^T, gW [K,N] += A^T dz, with
+        dz = _bn_bwd(g, z, bn, M, reduced=True) never leaving the chip (g is left as it is)."""
+        ops.bn_bwd_finalize(bn.stats, self._bwd_count(bn, M), bn.ggamma, bn.gbeta, bn.c1, bn.c2)
+        slabs = self._slab_buf(ops.pw_bwd_bn_slabs(M, self.device), K, N) if self.deterministic else None
+        ops.pw_bwd_bn(g, z, A, Wl, bn.a, bn.mean, bn.rstd, bn.c1, bn.c2, gA, gW, M, K, N, slabs=slabs)
+
     def _sep_fwd(self, s, x, in_bn, relu, training):
         B = self.B
         ops.dwconv3x3_fwd(x, s.dwk, in_bn.a if in_bn else None, in_bn.b if in_bn else None, relu, out=s.t)
@@ -344,8 +355,10 @@ class SPNetEngineBase:
             ops.acc_to_f32(self.l2_acc, self.l2_out)
 
     # ------------------------------------------------------------------ backward
-    def _sep_bwd(self, s, gz, x, in_bn, relu, g_t, g_in, add_src=None, add_strided=None, wgrad=True, out_bn=None):
-        """gz: grad wrt s.z [B,H,W,cout]. Produces the gradient wrt the sepconv's input tensor x
+    def _sep_bwd(self, s, gz, x, in_bn, relu, g_t, g_in, add_src=None, add_strided=None, wgrad=True, out_bn=None,
+                 gz_bn=False):
+        """gz: grad wrt s.z [B,H,W,cout] (gz_bn: grad wrt the output of s.bn, its sums already accumulated; the
+        BatchNorm backward then runs inside the pointwise backward). Produces the gradient wrt the sepconv's input tensor x
         (before its on-load BN/ReLU transform) in g_in; for a BN'd input this is still the grad wrt
         the BN OUTPUT (masked by relu'), to be pushed through _bn_bwd by the caller.
         out_bn = (z, bn, relu_mask): x = [relu](bn(z)) [+ ...], the BN that produced the UNtransformed input x. The
@@ -353,7 +366,10 @@ class SPNetEngineBase:
         relu_mask), so the caller's _bn_bwd on g_in runs with reduced=True."""
         B = self.B
         M = B * s.H * s.W
-        self._pw_bwd(s.t, s.pwl, s.gpw if wgrad else None, gz, g_t, M, s.cin, s.cout)
+        if gz_bn:
+            self._bn_pw_bwd(gz, s.z, s.bn, s.t, s.pwl, s.gpw, g_t, M, s.cin, s.cout)
+        else:
+            self._pw_bwd(s.t, s.pwl, s.gpw if wgrad else None, gz, g_t, M, s.cin, s.cout)
         gt4 = g_t.view(B, s.H, s.W, s.cin)
         zo, zbn, zmask = out_bn if out_bn else (None, None, False)
         ops.dwconv3x3_bwd_fused(gt4, x, s.dwk, s.gdwk, in_a=in_bn.a if in_bn else None, in_b=in_bn.b if in_bn else None,
@@ -374,21 +390,26 @@ class SPNetEngineBase:
         Mo = B * oh * ow
         M = B * H * W
         s1, s2 = e["sep1"], e["sep2"]
-        # residual branch
-        g_zr = self._bn_bwd(g_out, e["zr"], e["res_bn"], Mo, out=self._view(G1, B, oh, ow, c), reduced=True)
+        # residual branch (g_out is read again by the max-pool backward: the unfused route writes dz to G1)
         g_xs = self._view(S, Mo, cin)
-        self._pw_bwd(e["xs"].view(Mo, cin), self.wl[e["res"] + "/kernel"].view(cin, c),
-                     self.g[e["res"] + "/kernel"].view(cin, c), g_zr.view(Mo, c), g_xs, Mo, cin, c)
+        xs, Wr, gWr = e["xs"].view(Mo, cin), self.wl[e["res"] + "/kernel"].view(cin, c), self.g[e["res"] + "/kernel"].view(cin, c)
+        if self._pw_bwd_fusable(cin, c):
+            self._bn_pw_bwd(g_out, e["zr"], e["res_bn"], xs, Wr, gWr, g_xs, Mo, cin, c)
+        else:
+            g_zr = self._bn_bwd(g_out, e["zr"], e["res_bn"], Mo, out=self._view(G1, B, oh, ow, c), reduced=True)
+            self._pw_bwd(xs, Wr, gWr, g_zr.view(Mo, c), g_xs, Mo, cin, c)
         # main branch
         g_y2 = ops.maxpool3s2_bwd(g_out, e["argmax"], H, W, out=self._view(G1, B, H, W, c), z=s2.z, mean=s2.bn.mean,
                                   rstd=s2.bn.rstd, stats=s2.bn.stats)
-        g_z2 = self._bn_bwd(g_y2, s2.z, s2.bn, M, reduced=True)
         g_y1 = self._view(G3, B, H, W, s2.cin)
-        self._sep_bwd(s2, g_z2.view(M, c), s1.z, s1.bn, True, self._view(G2, M, s2.cin), g_y1)
-        g_z1 = self._bn_bwd(g_y1, s1.z, s1.bn, M, reduced=True)
+        fuse2 = self._pw_bwd_fusable(s2.cin, c)
+        g_z2 = g_y2 if fuse2 else self._bn_bwd(g_y2, s2.z, s2.bn, M, reduced=True)
+        self._sep_bwd(s2, g_z2.view(M, c), s1.z, s1.bn, True, self._view(G2, M, s2.cin), g_y1, gz_bn=fuse2)
+        fuse1 = self._pw_bwd_fusable(cin, s1.cout)
+        g_z1 = g_y1 if fuse1 else self._bn_bwd(g_y1, s1.z, s1.bn, M, reduced=True)
         g_x = self._view(R, B, H, W, cin)
         self._sep_bwd(s1, g_z1.view(M, s1.cout), x, None, e["relu_in"], self._view(G1, M, cin), g_x,
-                      add_strided=g_xs.view(B, oh, ow, cin), out_bn=x_bn)
+                      add_strided=g_xs.view(B, oh, ow, cin), out_bn=x_bn, gz_bn=fuse1)
         return g_x
 
     def backward_head(self):

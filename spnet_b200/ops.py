@@ -242,6 +242,25 @@ def bn_bwd_dz(g, z, a, save_mean, save_rstd, c1, c2, out=None):
     return out
 
 
+def pw_bwd_bn_slabs(M, device=None):
+    """Slabs spnet_pw_bwd_bn writes in deterministic mode: one per CTA of its persistent grid."""
+    n_sms = torch.cuda.get_device_properties(device if device is not None else torch.cuda.current_device()).multi_processor_count
+    return min(-(-M // 128), n_sms)
+
+
+def pw_bwd_bn(g, z, t, W, a, save_mean, save_rstd, c1, c2, gA, gW, M, cin, cout, slabs=None):
+    """Backward of a pointwise conv z = t W followed by a BatchNorm, in one kernel: dz = bn_bwd_dz(g, z, ...) stays on
+    chip, gA [M, cin] = dz W^T, gW [cin, cout] += t^T dz. bn_bwd_finalize must have run. slabs (fp32, at least
+    pw_bwd_bn_slabs(M) * cin * cout): the weight gradient goes through per-CTA slabs added in a fixed order."""
+    _chk(g, z, t, W, gA, gW, slabs)
+    n = pw_bwd_bn_slabs(M, g.device) if slabs is not None else 0
+    lib().pw_bwd_bn(_p(g), _p(z), _p(t), _p(W), _p(a), _p(save_mean), _p(save_rstd), _p(c1), _p(c2), _p(gA), _p(gW),
+                    _p(slabs), n, M, cin, cout, _s())
+    if slabs is not None:
+        slab_reduce(slabs, n, cin, cout, gW, accumulate=True)
+    return gA
+
+
 def augment_on_the_fly(x_orig, x, seed, max_regions=6, minsize=11, maxsize=75, sp_prob=0.5, sp_amount=0.004,
                        salt_vs_pepper=0.2):
     """x[n,H,W,C] = cutout + salt-and-pepper copy of the pristine frames x_orig (fp32, on the device)."""
