@@ -60,27 +60,6 @@ __global__ void bn_inference_affine_kernel(const float* __restrict__ gamma, cons
 // wave would pay the prologue latency again.
 constexpr int UNROLL = 4;
 
-__device__ __forceinline__ uint64_t pk2(float2 v) {
-    uint64_t r;
-    asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(v.x), "f"(v.y));
-    return r;
-}
-__device__ __forceinline__ float2 upk2(uint64_t r) {
-    float2 v;
-    asm("mov.b64 {%0, %1}, %2;" : "=f"(v.x), "=f"(v.y) : "l"(r));
-    return v;
-}
-__device__ __forceinline__ float2 ffma2(float2 a, float2 b, float2 c) {
-    uint64_t d;
-    asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(pk2(a)), "l"(pk2(b)), "l"(pk2(c)));
-    return upk2(d);
-}
-__device__ __forceinline__ float2 fadd2(float2 a, float2 b) {
-    uint64_t d;
-    asm("add.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(pk2(a)), "l"(pk2(b)));
-    return upk2(d);
-}
-
 // A 16-byte vector of activations as NP fp32 pairs (bf16: 4 pairs, fp32: 2 pairs).
 template <typename T> struct RawVec;
 template <> struct RawVec<bf16> {

@@ -74,6 +74,33 @@ template <> __device__ __forceinline__ bf16 from_f32<bf16>(float x) { return __f
 // value as it will read back after being stored as T
 template <typename T> __device__ __forceinline__ float round_to(float x) { return to_f32(from_f32<T>(x)); }
 
+// ---- packed fp32 pair arithmetic (FFMA2 / FMUL2 / FADD2): one issue slot per two fp32 operations ---------------
+__device__ __forceinline__ uint64_t pk2(float2 v) {
+    uint64_t r;
+    asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(v.x), "f"(v.y));
+    return r;
+}
+__device__ __forceinline__ float2 upk2(uint64_t r) {
+    float2 v;
+    asm("mov.b64 {%0, %1}, %2;" : "=f"(v.x), "=f"(v.y) : "l"(r));
+    return v;
+}
+__device__ __forceinline__ float2 ffma2(float2 a, float2 b, float2 c) {
+    uint64_t d;
+    asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(pk2(a)), "l"(pk2(b)), "l"(pk2(c)));
+    return upk2(d);
+}
+__device__ __forceinline__ float2 fmul2(float2 a, float2 b) {
+    uint64_t d;
+    asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(pk2(a)), "l"(pk2(b)));
+    return upk2(d);
+}
+__device__ __forceinline__ float2 fadd2(float2 a, float2 b) {
+    uint64_t d;
+    asm("add.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(pk2(a)), "l"(pk2(b)));
+    return upk2(d);
+}
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
@@ -120,15 +147,22 @@ __device__ __forceinline__ double stat_get(const long long* acc, long long i) {
 }
 __device__ __forceinline__ void stat_clear(long long* acc, long long i) { acc[2 * i] = 0; acc[2 * i + 1] = 0; }
 
-// cudaFuncSetAttribute (the dynamic shared-memory opt-in) is per DEVICE: one flag per device for a launcher's
-// "configured once" state. Returns true the first time it is called for the current device with these flags.
-static inline bool spnet_first_use_on_device(bool (&flags)[64]) {
+// Dynamic shared memory above 48 KB is an opt-in of each kernel, and cudaFuncSetAttribute sets it for the current
+// DEVICE only. `configured` is the caller's per-device flag array for this kernel: the attribute is set once per
+// device, to `bytes`, the most any launch of the kernel asks for. `who` names the caller in the error message.
+template <typename Kernel>
+static inline int spnet_smem_optin(bool (&configured)[64], Kernel kern, size_t bytes, const char* who) {
     int dev = 0;
     cudaGetDevice(&dev);
     dev &= 63;
-    if (flags[dev]) return false;
-    flags[dev] = true;
-    return true;
+    if (configured[dev]) return SPNET_OK;
+    const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    if (e != cudaSuccess) {
+        spnet_set_error("%s: cudaFuncSetAttribute: %s", who, cudaGetErrorString(e));
+        return SPNET_ERR_CUDA;
+    }
+    configured[dev] = true;
+    return SPNET_OK;
 }
 
 // SM count of the current device (148 on B200), cached per device: persistent grids are sized from it.

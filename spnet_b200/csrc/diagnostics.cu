@@ -521,14 +521,8 @@ int spnet_ellipse_iou(const float* yp, const float* yt, int n, int ncols, int nx
         // exact: the reference's own raster (cv2's anti-aliased filled polygon), pixel for pixel; 512 x 384 canvas only
         SPNET_REQUIRE(nx == RX && ny == RY, "ellipse_iou: the exact raster is built for the reference's 512 x 384 canvas");
         static bool configured[64] = {};
-        if (spnet_first_use_on_device(configured)) {
-            cudaError_t e = cudaFuncSetAttribute(ellipse_iou_exact_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                 (int)sizeof(RasterSmem));
-            if (e != cudaSuccess) {
-                spnet_set_error("ellipse_iou: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-                return SPNET_ERR_CUDA;
-            }
-        }
+        const int rc = spnet_smem_optin(configured, ellipse_iou_exact_kernel, sizeof(RasterSmem), "ellipse_iou");
+        if (rc) return rc;
         ellipse_iou_exact_kernel<<<n * (ncols / VARS), 256, sizeof(RasterSmem), stream>>>(yp, yt, ncols, iou, counts);
         return spnet_check_launch("ellipse_iou");
     }

@@ -25,32 +25,6 @@ namespace {
 constexpr int CB = 64;        // channels per CTA: 32 lanes x one channel pair
 constexpr int MAX_STAGES = 6;
 
-// ---- packed fp32 pair arithmetic (FFMA2 / FMUL2 / FADD2) ---------------------------------------
-__device__ __forceinline__ uint64_t pk(float2 v) {
-    uint64_t r;
-    asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(v.x), "f"(v.y));
-    return r;
-}
-__device__ __forceinline__ float2 upk(uint64_t r) {
-    float2 v;
-    asm("mov.b64 {%0, %1}, %2;" : "=f"(v.x), "=f"(v.y) : "l"(r));
-    return v;
-}
-__device__ __forceinline__ float2 ffma2(float2 a, float2 b, float2 c) {
-    uint64_t d;
-    asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(pk(a)), "l"(pk(b)), "l"(pk(c)));
-    return upk(d);
-}
-__device__ __forceinline__ float2 fmul2(float2 a, float2 b) {
-    uint64_t d;
-    asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(pk(a)), "l"(pk(b)));
-    return upk(d);
-}
-__device__ __forceinline__ float2 fadd2(float2 a, float2 b) {
-    uint64_t d;
-    asm("add.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(pk(a)), "l"(pk(b)));
-    return upk(d);
-}
 __device__ __forceinline__ float2 relu2(float2 v) { return make_float2(fmaxf(v.x, 0.f), fmaxf(v.y, 0.f)); }
 // activation applied on load: RELU = 0 none, 1 ReLU (Xception), 2 ReLU6 (MobileNet). NaN (the padding fill) maps to 0.
 template <int RELU> __device__ __forceinline__ float2 act2(float2 v) {
@@ -91,9 +65,6 @@ __device__ __forceinline__ void stg_pair(float* p, float2 v) { *reinterpret_cast
 __device__ __forceinline__ float2 round_pair(float2 v, const bf16*) { return widen(pack_bf16x2(v.x, v.y)); }
 __device__ __forceinline__ float2 round_pair(float2 v, const float*) { return v; }
 
-__device__ __forceinline__ void mbar_arrive_cta(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
 __device__ __forceinline__ void consumer_bar_sync(int nthreads) {
     asm volatile("bar.sync 1, %0;" ::"r"(nthreads) : "memory");
 }
@@ -114,13 +85,6 @@ __device__ __forceinline__ TileCoord tile_coord(int tile, int tiles_w, int tiles
 // CTA = TW/NC warps; blockIdx.y = 64-channel chunk, blockIdx.x walks
 // (image, row-tile, col-tile) tiles round-robin.
 // =================================================================================================
-// one lane of a converged warp, always the same one, in a form the compiler treats as a single thread
-__device__ __forceinline__ uint32_t elect_one_lane() {
-    uint32_t leader;
-    asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(leader));
-    return leader;
-}
-
 template <typename T, int NC, bool AFFINE, int RELU>
 __global__ void __launch_bounds__(256, 2)
 dw3x3_fwd_packed_kernel(const __grid_constant__ CUtensorMap tm_in, const float* __restrict__ k,
@@ -180,7 +144,7 @@ dw3x3_fwd_packed_kernel(const __grid_constant__ CUtensorMap tm_in, const float* 
     // Producer duty rotates over the warps (tile i of this CTA is refilled by warp i % ncons): the refill has to
     // wait until EVERY warp has released the stage and then costs a few hundred cycles of coordinate decode + TMA
     // issue; pinned to warp 0 that made warp 0 the last one through every tile and the pace of the whole CTA.
-    const uint32_t issuer_lane = elect_one_lane();
+    const uint32_t issuer_lane = elect_one();
     int s = 0, n = 0, duty = 0;
     for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
         if (warp == duty) {  // warp-uniform
@@ -249,7 +213,7 @@ dw3x3_fwd_packed_kernel(const __grid_constant__ CUtensorMap tm_in, const float* 
             if (r < rows) { step(A_, B_, C_); if (r < rows) step(B_, C_, A_); }
         }
         __syncwarp();
-        if (lane == 0) mbar_arrive_cta(empty0 + 8 * s);
+        if (lane == 0) mbar_arrive(empty0 + 8 * s);
         if (++s == S) { s = 0; ++n; }
     }
 }
@@ -354,7 +318,7 @@ dw3x3_bwd_packed_kernel(const __grid_constant__ CUtensorMap tm_g, const __grid_c
     // Producer duty rotates over the warps (tile i of this CTA is refilled by warp i % ncons): the refill has to
     // wait until EVERY warp has released the stage and then costs a few hundred cycles of coordinate decode + TMA
     // issue; pinned to warp 0 that made warp 0 the last one through every tile and the pace of the whole CTA.
-    const uint32_t issuer_lane = elect_one_lane();
+    const uint32_t issuer_lane = elect_one();
     int s = 0, n = 0, duty = 0;
     for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
         if (warp == duty) {  // warp-uniform
@@ -460,7 +424,7 @@ dw3x3_bwd_packed_kernel(const __grid_constant__ CUtensorMap tm_g, const __grid_c
             if (r < rows) { step(G0, G1, G2); if (r < rows) step(G1, G2, G0); }
         }
         __syncwarp();
-        if (lane == 0) mbar_arrive_cta(empty0 + 8 * s);
+        if (lane == 0) mbar_arrive(empty0 + 8 * s);
         if (++s == S) { s = 0; ++n; }
     }
 
@@ -504,25 +468,14 @@ dw3x3_bwd_packed_kernel(const __grid_constant__ CUtensorMap tm_g, const __grid_c
 // =================================================================================================
 int make_map(CUtensorMap* map, const void* ptr, int dtype, int B, int H, int W, int C, int box_w, int box_h,
              bool nan_fill) {
-    PFN_cuTensorMapEncodeTiled enc = spnet_get_tensormap_encoder();
-    if (!enc) {
-        spnet_set_error("dwconv3x3: cuTensorMapEncodeTiled entry point not available");
-        return SPNET_ERR_CUDA;
-    }
     const cuuint64_t es = dtype == SPNET_BF16 ? 2 : 4;
-    cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)B};
-    cuuint64_t strides[3] = {(cuuint64_t)C * es, (cuuint64_t)W * C * es, (cuuint64_t)H * W * C * es};
-    cuuint32_t box[4] = {(cuuint32_t)CB, (cuuint32_t)box_w, (cuuint32_t)box_h, 1};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = enc(map, dtype == SPNET_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4,
-                     const_cast<void*>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                     CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                     nan_fill ? CU_TENSOR_MAP_FLOAT_OOB_FILL_NAN_REQUEST_ZERO_FMA : CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-        spnet_set_error("dwconv3x3: cuTensorMapEncodeTiled failed (%d) for [%d,%d,%d,%d]", (int)r, B, H, W, C);
-        return SPNET_ERR_CUDA;
-    }
-    return SPNET_OK;
+    const cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)B};
+    const cuuint64_t strides[3] = {(cuuint64_t)C * es, (cuuint64_t)W * C * es, (cuuint64_t)H * W * C * es};
+    const cuuint32_t box[4] = {(cuuint32_t)CB, (cuuint32_t)box_w, (cuuint32_t)box_h, 1};
+    return spnet_encode_tiled(map, "dwconv3x3",
+                              dtype == SPNET_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4,
+                              ptr, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                              nan_fill ? CU_TENSOR_MAP_FLOAT_OOB_FILL_NAN_REQUEST_ZERO_FMA : CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
 }
 
 struct Tiling { int TH, TW, NC, S, tiles_h, tiles_w, threads, chunks, grid_x; size_t smem; };
@@ -573,13 +526,8 @@ int launch_fwd_inst(const CUtensorMap& tm, const float* k, const float* a, const
                     int C, const Tiling& t, cudaStream_t stream) {
     auto kern = dw3x3_fwd_packed_kernel<T, NC, AF, RL>;
     static bool configured[64] = {};
-    if (spnet_first_use_on_device(configured)) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024);
-        if (e != cudaSuccess) {
-            spnet_set_error("dwconv3x3_fwd: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-            return SPNET_ERR_CUDA;
-        }
-    }
+    const int rc = spnet_smem_optin(configured, kern, 220 * 1024, "dwconv3x3_fwd");
+    if (rc) return rc;
     kern<<<dim3(t.grid_x, t.chunks), t.threads, t.smem, stream>>>(tm, k, a, b, y, B, H, W, C, t.TH, t.TW, t.tiles_h,
                                                                   t.tiles_w, t.S);
     return spnet_check_launch("dw3x3_fwd");
@@ -609,13 +557,8 @@ int launch_bwd_inst(const CUtensorMap& tg, const CUtensorMap& tx, const CUtensor
                     int H, int W, int C, const Tiling& t, cudaStream_t stream) {
     auto kern = dw3x3_bwd_packed_kernel<T, AF, RL, EPI, ZO>;
     static bool configured[64] = {};
-    if (spnet_first_use_on_device(configured)) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024);
-        if (e != cudaSuccess) {
-            spnet_set_error("dwconv3x3_bwd: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-            return SPNET_ERR_CUDA;
-        }
-    }
+    const int rc = spnet_smem_optin(configured, kern, 220 * 1024, "dwconv3x3_bwd");
+    if (rc) return rc;
     kern<<<dim3(t.grid_x, t.chunks), t.threads, t.smem, stream>>>(tg, tx, ta, tz, ma, mb, k, a, b, mean, rstd, stats,
                                                                   sadd, gin, dk, dk_acc, B, H, W, C, t.TH, t.TW,
                                                                   t.tiles_h, t.tiles_w, t.S);

@@ -179,12 +179,7 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_tc_kernel(const __grid_const
         }
         mbar_fence_init();
     }
-    if (warp == 1) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_holder)),
-                     "r"((uint32_t)(2 * BN))
-                     : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    if (warp == 1) tmem_alloc(smem_u32(&tmem_base_holder), 2 * BN);
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     if (CL > 1) cluster_sync_all(); else __syncthreads();  // barrier inits visible cluster-wide
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
@@ -421,27 +416,15 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_tc_kernel(const __grid_const
                     // rows >= M and columns >= N are clipped by the TMA unit
                     if (col0 < N && rows_live) {  // warp-uniform
                         const uint32_t stg = stage_out0 + ((uint32_t)(warp - 2) * SD + sbox) * 2048u;
-                        if (e_leader) asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(SD - 1) : "memory");  // this box was read out
+                        if (e_leader) tma_store_wait_read<SD - 1>();  // this box was read out
                         __syncwarp();
-                        const uint32_t rowaddr = stg + (uint32_t)lane * 64u, sw = ((uint32_t)lane >> 1) & 3u;
-#pragma unroll
-                        for (int g = 0; g < 4; ++g)
-                            asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(rowaddr + (((uint32_t)g ^ sw) << 4)),
-                                         "r"(packed[4 * g]), "r"(packed[4 * g + 1]), "r"(packed[4 * g + 2]),
-                                         "r"(packed[4 * g + 3])
-                                         : "memory");
-                        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+                        stage_box_row_sw64(stg, (uint32_t)lane, packed);
+                        fence_proxy_async_smem();
                         __syncwarp();
                         if (e_leader) {
-                            if (CONV == 1)
-                                asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];" ::"l"(&tmD),
-                                             "r"(stg), "r"(col0), "r"(dx), "r"(dy), "r"(dimg)
-                                             : "memory");
-                            else
-                                asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(&tmD),
-                                             "r"(stg), "r"(col0), "r"(drow)
-                                             : "memory");
-                            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+                            if (CONV == 1) tma_store_4d(&tmD, stg, col0, dx, dy, dimg);
+                            else tma_store_2d(&tmD, stg, col0, drow);
+                            tma_store_commit();
                         }
                         last_box = stg;
                         if (SD > 1) sbox ^= 1u;
@@ -452,37 +435,24 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_tc_kernel(const __grid_const
                     // fp32 store / split-K accumulation through the same 2 KB staging box, 16 columns (64-byte
                     // rows) at a time: TMA store, or TMA reduce-add into the fp32 gradient for OUT_ATOMIC_F32
                     if (CONV != 1 && rows_live) {  // warp-uniform (the convolution forward / data gradient store bf16 only)
-                        const uint32_t sw = ((uint32_t)lane >> 1) & 3u;
 #pragma unroll
                         for (int h = 0; h < 2; ++h) {
                             if (col0 + 16 * h >= N) break;  // warp-uniform
                             const uint32_t stg = stage_out0 + ((uint32_t)(warp - 2) * SD + sbox) * 2048u;
-                            const uint32_t rowaddr = stg + (uint32_t)lane * 64u;
                             if (SD > 1) sbox ^= 1u;
-                            if (e_leader) asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(SD - 1) : "memory");
+                            if (e_leader) tma_store_wait_read<SD - 1>();
                             __syncwarp();
-#pragma unroll
-                            for (int g = 0; g < 4; ++g)
-                                asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(rowaddr + (((uint32_t)g ^ sw) << 4)),
-                                             "r"(v[16 * h + 4 * g]), "r"(v[16 * h + 4 * g + 1]), "r"(v[16 * h + 4 * g + 2]),
-                                             "r"(v[16 * h + 4 * g + 3])
-                                             : "memory");
-                            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+                            stage_box_row_sw64(stg, (uint32_t)lane, v + 16 * h);
+                            fence_proxy_async_smem();
                             __syncwarp();
                             if (e_leader) {
                                 if (epi.mode == OUT_SLAB_F32)  // rows >= M of the slab are clipped: slabs may sit inside other data
-                                    asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];" ::"l"(&tmD),
-                                                 "r"(stg), "r"(col0 + 16 * h), "r"(drow), "r"(dslab)
-                                                 : "memory");
+                                    tma_store_3d(&tmD, stg, col0 + 16 * h, drow, dslab);
                                 else if (epi.mode != OUT_ATOMIC_F32)
-                                    asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(&tmD),
-                                                 "r"(stg), "r"(col0 + 16 * h), "r"(drow)
-                                                 : "memory");
+                                    tma_store_2d(&tmD, stg, col0 + 16 * h, drow);
                                 else
-                                    asm volatile("cp.reduce.async.bulk.tensor.2d.global.shared::cta.add.bulk_group [%0, {%2, %3}], [%1];" ::"l"(&tmD),
-                                                 "r"(stg), "r"(col0 + 16 * h), "r"(drow)
-                                                 : "memory");
-                                asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+                                    tma_reduce_add_2d(&tmD, stg, col0 + 16 * h, drow);
+                                tma_store_commit();
                             }
                         }
                     }
@@ -547,14 +517,13 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_tc_kernel(const __grid_const
             }
         }
         if (epi.colstats) flush_stats();
-        if (e_leader) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");  // staging may not die under a store
+        if (e_leader) tma_store_wait_read<0>();  // staging may not die under a store
         if (threadIdx.x == 64) TRACE(10);
     }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     if (CL > 1) cluster_sync_all(); else __syncthreads();  // no CTA may exit while its peer still multicasts into it
     if (threadIdx.x == 0) { TRACE(11); TRACE_G(12); }
-    if (warp == 1)
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)(2 * BN)) : "memory");
+    if (warp == 1) tmem_dealloc(tmem_base, 2 * BN);
 }
 
 // ---------------------------------------------------------------------------------
@@ -564,13 +533,8 @@ constexpr int kMaxResidentKb = 9;  // resident-B convolutions: at most 9 k-block
 // operand with `rows` along M/N and `kdim` along K; ld in elements
 int make_operand_map(CUtensorMap* map, const void* ptr, long long rows, long long kdim, long long ld, bool mn_major,
                      int tile_rows) {
-    PFN_cuTensorMapEncodeTiled enc = spnet_get_tensormap_encoder();
-    if (!enc) {
-        spnet_set_error("gemm_bf16: cuTensorMapEncodeTiled entry point not available");
-        return SPNET_ERR_CUDA;
-    }
-    cuuint64_t dims[2], strides[1];
-    cuuint32_t box[2], estr[2] = {1, 1};
+    cuuint64_t dims[2];
+    cuuint32_t box[2];
     if (mn_major) {
         dims[0] = (cuuint64_t)rows; dims[1] = (cuuint64_t)kdim;
         box[0] = 64; box[1] = BK;
@@ -578,16 +542,10 @@ int make_operand_map(CUtensorMap* map, const void* ptr, long long rows, long lon
         dims[0] = (cuuint64_t)kdim; dims[1] = (cuuint64_t)rows;
         box[0] = BK; box[1] = (cuuint32_t)tile_rows;
     }
-    strides[0] = (cuuint64_t)ld * 2;
-    CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(ptr), dims, strides, box, estr,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-        spnet_set_error("gemm_bf16: cuTensorMapEncodeTiled failed (%d) rows=%lld k=%lld ld=%lld mn=%d", (int)r, rows,
-                        kdim, ld, (int)mn_major);
-        return SPNET_ERR_CUDA;
-    }
-    return SPNET_OK;
+    const cuuint64_t strides[1] = {(cuuint64_t)ld * 2};
+    return spnet_encode_tiled(map, "gemm_bf16", CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, ptr, dims, strides, box,
+                              CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
 }
 
 // CONV 0: tiles_m_conv / ntaps unused. CONV 1: tiles_m_conv = number of pixel tiles. CONV 2: ntaps = cg.ntaps.
@@ -600,17 +558,11 @@ int launch_gemm(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap&
     const size_t smem = (size_t)STAGES * (BM * BK * 2 + (BRES ? 0 : BN * BK * 2)) +
                         (BRES ? (size_t)((K + BK - 1) / BK) * BN * BK * 2 : 0) + 1024 + kEpiWarps * 2048 * (BN <= 128 ? 2 : 1);
     auto kern = gemm_tc_kernel<BN, A_MN, B_MN, STAGES, CL, CONV, BRES>;
-    // per (instantiation, device): the dynamic shared-memory opt-in is a per-device function attribute
     static bool configured[64] = {};
-    if (spnet_first_use_on_device(configured)) {
-        // (resident B: the size depends on K; opt in to the largest this mode is dispatched with)
-        const size_t smem_max = BRES ? (size_t)STAGES * BM * BK * 2 + (size_t)kMaxResidentKb * BN * BK * 2 + 1024 + kEpiWarps * 2048 * 2 : smem;
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_max);
-        if (e != cudaSuccess) {
-            spnet_set_error("gemm_bf16: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-            return SPNET_ERR_CUDA;
-        }
-    }
+    // (resident B: the size depends on K; opt in to the largest this mode is dispatched with)
+    const size_t smem_max = BRES ? (size_t)STAGES * BM * BK * 2 + (size_t)kMaxResidentKb * BN * BK * 2 + 1024 + kEpiWarps * 2048 * 2 : smem;
+    const int rc = spnet_smem_optin(configured, kern, smem_max, "gemm_bf16");
+    if (rc) return rc;
     const int total_kb = (K + BK - 1) / BK;
     if (splits < 1) splits = 1;
     if (splits > total_kb) splits = total_kb;
@@ -716,16 +668,15 @@ int spnet_gemm_bf16(const void* A, long long lda, int a_mn, const void* B, long 
     if (rc) return rc;
     CUtensorMap td;  // output boxes of the TMA-store epilogue: 32 x 32 bf16 or 32 x 16 fp32 (64-byte rows, SWIZZLE_64B)
     {
-        PFN_cuTensorMapEncodeTiled enc = spnet_get_tensormap_encoder();
         const bool ob = out_mode == OUT_BF16;
         const bool slabs = out_mode == OUT_SLAB_F32;
-        cuuint64_t dims[3] = {(cuuint64_t)N, (cuuint64_t)M, (cuuint64_t)n_slabs};
-        cuuint64_t strides[2] = {(cuuint64_t)ldd * (ob ? 2 : 4), (cuuint64_t)slab_stride * 4};
-        cuuint32_t box[3] = {ob ? 32u : 16u, 32u, 1u}, estr[3] = {1, 1, 1};
-        CUresult r = enc(&td, ob ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, slabs ? 3 : 2, D, dims,
-                         strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B,
-                         CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        SPNET_REQUIRE(r == CUDA_SUCCESS, "gemm_bf16: cuTensorMapEncodeTiled (output) failed (%d) M=%d N=%d ldd=%lld", (int)r, M, N, ldd);
+        const cuuint64_t dims[3] = {(cuuint64_t)N, (cuuint64_t)M, (cuuint64_t)n_slabs};
+        const cuuint64_t strides[2] = {(cuuint64_t)ldd * (ob ? 2 : 4), (cuuint64_t)slab_stride * 4};
+        const cuuint32_t box[3] = {ob ? 32u : 16u, 32u, 1u};
+        rc = spnet_encode_tiled(&td, "gemm_bf16 (output)", ob ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32,
+                                slabs ? 3 : 2, D, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_64B,
+                                CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+        if (rc) return rc;
     }
     GemmEpi epi = {D, ldd, out_mode, 0, colstats};
 #define SPNET_GEMM_DISPATCH(BN_, CL_)                                                                                       \
@@ -773,22 +724,11 @@ void pick_pixel_box(int log_rows, int OW, int OH, int NB, int* lw_out, int* lh_o
 int make_pixel_map(CUtensorMap* map, const void* ptr, int NB, int H, int W, int C, long long ld, int lw, int lh, int ln,
                    int box_c, CUtensorMapSwizzle swz, CUtensorMapL2promotion prom, long long row_ld = 0) {
     if (row_ld <= 0) row_ld = (long long)W * ld;
-    PFN_cuTensorMapEncodeTiled enc = spnet_get_tensormap_encoder();
-    if (!enc) {
-        spnet_set_error("conv_tc: cuTensorMapEncodeTiled entry point not available");
-        return SPNET_ERR_CUDA;
-    }
-    cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)NB};
-    cuuint64_t strides[3] = {(cuuint64_t)ld * 2, (cuuint64_t)row_ld * 2, (cuuint64_t)H * row_ld * 2};
-    cuuint32_t box[4] = {(cuuint32_t)box_c, 1u << lw, 1u << lh, 1u << ln}, estr[4] = {1, 1, 1, 1};
-    CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(ptr), dims, strides, box, estr,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, swz, prom, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-        spnet_set_error("conv_tc: cuTensorMapEncodeTiled failed (%d) NB=%d H=%d W=%d C=%d ld=%lld box=%d,%d,%d,%d", (int)r, NB,
-                        H, W, C, ld, box_c, 1 << lw, 1 << lh, 1 << ln);
-        return SPNET_ERR_CUDA;
-    }
-    return SPNET_OK;
+    const cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)NB};
+    const cuuint64_t strides[3] = {(cuuint64_t)ld * 2, (cuuint64_t)row_ld * 2, (cuuint64_t)H * row_ld * 2};
+    const cuuint32_t box[4] = {(cuuint32_t)box_c, 1u << lw, 1u << lh, 1u << ln};
+    return spnet_encode_tiled(map, "conv_tc", CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, ptr, dims, strides, box, swz, prom,
+                              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
 }
 
 // forward (dgrad = 0): out[n, y, x, :] = sum_taps in[n, y + ky - pt, x + kx - pl, :] . Wt[ky, kx, :, :]
@@ -867,12 +807,11 @@ int conv_tc_wgrad_impl(const void* X, long long ldx, int NB, int H, int W, int C
                         CU_TENSOR_MAP_L2_PROMOTION_L2_256B);
     if (rc) return rc;
     {
-        PFN_cuTensorMapEncodeTiled enc = spnet_get_tensormap_encoder();
-        cuuint64_t dims[2] = {(cuuint64_t)N, (cuuint64_t)cg.ntaps * M}, strides[1] = {(cuuint64_t)N * 4};
-        cuuint32_t box[2] = {16u, 32u}, estr[2] = {1, 1};
-        CUresult r = enc(&td, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, dW, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                         CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        SPNET_REQUIRE(r == CUDA_SUCCESS, "conv_tc_wgrad: cuTensorMapEncodeTiled (output) failed (%d)", (int)r);
+        const cuuint64_t dims[2] = {(cuuint64_t)N, (cuuint64_t)cg.ntaps * M}, strides[1] = {(cuuint64_t)N * 4};
+        const cuuint32_t box[2] = {16u, 32u};
+        rc = spnet_encode_tiled(&td, "conv_tc_wgrad (output)", CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, dW, dims, strides, box,
+                                CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+        if (rc) return rc;
     }
     // split the pixel reduction so that taps x tiles x splits fills the SMs about once; >= 4 pixel blocks per split
     const long long tiles = (long long)((M + BM - 1) / BM) * ((N + bn - 1) / bn) * cg.ntaps;

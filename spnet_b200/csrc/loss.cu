@@ -330,15 +330,14 @@ int spnet_yolo_ellipse_loss_ann(const double* ann, const int* counts, int max_ob
     const int xbin = (470 - 40) / nx, ybin = (350 - 40) / ny;
     SPNET_REQUIRE(xbin > 0 && ybin > 0, "yolo_ellipse_loss_ann: grid too fine");
     const int ncols = nx * ny * ppc * 8;
+    constexpr size_t kSmemMax = 200 * 1024;  // opted in to once; each launch asks for what its columns need
     int nwarps = kLossThreads / 32;
-    while (nwarps > 1 && (size_t)nwarps * (ncols * 4 + 256) > 200 * 1024) nwarps >>= 1;
+    while (nwarps > 1 && (size_t)nwarps * (ncols * 4 + 256) > kSmemMax) nwarps >>= 1;
     const size_t smem = (size_t)nwarps * (ncols * 4 + 256);
-    SPNET_REQUIRE(smem <= 200 * 1024, "yolo_ellipse_loss_ann: %d output columns do not fit shared memory", ncols);
-    cudaError_t e = cudaFuncSetAttribute(yolo_ellipse_loss_ann_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) {
-        spnet_set_error("yolo_ellipse_loss_ann: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-        return SPNET_ERR_CUDA;
-    }
+    SPNET_REQUIRE(smem <= kSmemMax, "yolo_ellipse_loss_ann: %d output columns do not fit shared memory", ncols);
+    static bool configured[64] = {};
+    const int rc = spnet_smem_optin(configured, yolo_ellipse_loss_ann_kernel, kSmemMax, "yolo_ellipse_loss_ann");
+    if (rc) return rc;
     yolo_ellipse_loss_ann_kernel<<<1, nwarps * 32, smem, stream>>>(ann, counts, max_obj, nx, ny, ppc, xbin, ybin, defaults, means,
                                                                   ranges, y_pred, batch, hybrid, sel_sigmoid, y_true_out, out6,
                                                                   grad, err);

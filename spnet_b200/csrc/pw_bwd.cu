@@ -94,12 +94,7 @@ __global__ void __launch_bounds__(kPwThreads, 1) pw_bwd_bn_kernel(
         mbar_init(bar(WACC_FULL), 1);
         mbar_fence_init();
     }
-    if (warp == 1) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_holder)),
-                     "r"(Cfg::TMEM_COLS)
-                     : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    if (warp == 1) tmem_alloc(smem_u32(&tmem_base_holder), Cfg::TMEM_COLS);
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
@@ -229,7 +224,7 @@ __global__ void __launch_bounds__(kPwThreads, 1) pw_bwd_bn_kernel(
                                  : "memory");
                 }
             // dz written by the generic proxy is read by tcgen05.mma (async proxy)
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+            fence_proxy_async_smem();
             __syncwarp();
             if (lane == 0) {
                 mbar_arrive(bar(Z_EMPTY + zs));
@@ -257,21 +252,14 @@ __global__ void __launch_bounds__(kPwThreads, 1) pw_bwd_bn_kernel(
                 for (int j = 0; j < 16; ++j) packed[j] = pack_bf16x2(__uint_as_float(v[2 * j]), __uint_as_float(v[2 * j + 1]));
                 if (row0 < M) {  // warp-uniform; rows >= M inside the box are clipped by the TMA unit
                     const uint32_t stg = out0 + ((uint32_t)ew * 2u + sbox) * 2048u;
-                    if (e_leader) asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");  // this box was read out
+                    if (e_leader) tma_store_wait_read<1>();  // this box was read out
                     __syncwarp();
-                    const uint32_t rowaddr = stg + (uint32_t)lane * 64u, sw = ((uint32_t)lane >> 1) & 3u;
-#pragma unroll
-                    for (int g = 0; g < 4; ++g)
-                        asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(rowaddr + (((uint32_t)g ^ sw) << 4)),
-                                     "r"(packed[4 * g]), "r"(packed[4 * g + 1]), "r"(packed[4 * g + 2]), "r"(packed[4 * g + 3])
-                                     : "memory");
-                    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+                    stage_box_row_sw64(stg, (uint32_t)lane, packed);
+                    fence_proxy_async_smem();
                     __syncwarp();
                     if (e_leader) {
-                        asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];" ::"l"(&tmGA),
-                                     "r"(stg), "r"(c * 32), "r"(row0)
-                                     : "memory");
-                        asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+                        tma_store_2d(&tmGA, stg, c * 32, row0);
+                        tma_store_commit();
                     }
                     sbox ^= 1u;
                 }
@@ -298,25 +286,20 @@ __global__ void __launch_bounds__(kPwThreads, 1) pw_bwd_bn_kernel(
                 }
             }
         }
-        if (e_leader) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");  // staging may not die under a store
+        if (e_leader) tma_store_wait_read<0>();  // staging may not die under a store
     }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
-    if (warp == 1)
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(Cfg::TMEM_COLS) : "memory");
+    if (warp == 1) tmem_dealloc(tmem_base, Cfg::TMEM_COLS);
 }
 
 int pw_map(CUtensorMap* map, const void* ptr, long long rows, int cols, int box_cols, int box_rows, bool bf16_out) {
-    PFN_cuTensorMapEncodeTiled enc = spnet_get_tensormap_encoder();
-    SPNET_REQUIRE(enc, "pw_bwd_bn: cuTensorMapEncodeTiled entry point not available");
-    cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows}, strides[1] = {(cuuint64_t)cols * 2};
-    cuuint32_t box[2] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows}, estr[2] = {1, 1};
-    CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(ptr), dims, strides, box, estr,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, bf16_out ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B,
-                     bf16_out ? CU_TENSOR_MAP_L2_PROMOTION_NONE : CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    SPNET_REQUIRE(r == CUDA_SUCCESS, "pw_bwd_bn: cuTensorMapEncodeTiled failed (%d) rows=%lld cols=%d", (int)r, rows, cols);
-    return SPNET_OK;
+    const cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows}, strides[1] = {(cuuint64_t)cols * 2};
+    const cuuint32_t box[2] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows};
+    return spnet_encode_tiled(map, "pw_bwd_bn", CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, ptr, dims, strides, box,
+                              bf16_out ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B,
+                              bf16_out ? CU_TENSOR_MAP_L2_PROMOTION_NONE : CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
 }
 
 template <int CIN>
@@ -325,10 +308,8 @@ int launch_pw_bwd(const CUtensorMap& tg, const CUtensorMap& tz, const CUtensorMa
                   const float* c2, float* gW, float* slabs, int M, int n_tiles, int grid, cudaStream_t stream) {
     auto kern = pw_bwd_bn_kernel<CIN>;
     static bool configured[64] = {};
-    if (spnet_first_use_on_device(configured)) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PwCfg<CIN>::SMEM);
-        SPNET_REQUIRE(e == cudaSuccess, "pw_bwd_bn: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-    }
+    const int rc = spnet_smem_optin(configured, kern, PwCfg<CIN>::SMEM, "pw_bwd_bn");
+    if (rc) return rc;
     kern<<<grid, kPwThreads, PwCfg<CIN>::SMEM, stream>>>(tg, tz, tt, tw, tga, a, mean, rstd, c1, c2, gW, slabs, M, n_tiles);
     return spnet_check_launch("pw_bwd_bn");
 }

@@ -984,11 +984,11 @@ int persist_grid_tiles(long long n_tiles, int ctas_per_sm) {
     return (int)(n_tiles < cap ? n_tiles : cap);
 }
 
-// dynamic shared memory above 48 KB is a per-device opt-in of the function
-// (set on every call: the kernels share one function-pointer type, so a per-type "done" flag would be wrong, and the
-// call is host-side only)
-template <typename K> void strip_smem_optin(K kern, size_t bytes) {
-    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+// dynamic shared memory above 48 KB is a per-device opt-in of each kernel: one flag array per kernel (the kernels
+// share one function-pointer type, so the kernel itself is the template argument)
+template <auto kern> int strip_smem_optin(size_t bytes, const char* who) {
+    static bool configured[64] = {};
+    return spnet_smem_optin(configured, kern, bytes, who);
 }
 
 }  // namespace
@@ -1019,10 +1019,11 @@ int spnet_conv_small_fwd(int which, const void* in, const float* w, const float*
     } else if (which == 1 && W % 8 == 0) {
         const int th = ceil_div(H, SK_TH), tw = ceil_div(W, SK_TW);
         const int grid = persist_grid_tiles((long long)B * th * tw, 2);
-        SPNET_DISPATCH_DTYPE(dtype, (strip_smem_optin(conv3c3_strip_kernel<T, 0>, StripWindow<T>::smem_bytes()),
-                                     conv3c3_strip_kernel<T, 0><<<grid, kThreads, StripWindow<T>::smem_bytes(), stream>>>(
+        SPNET_DISPATCH_DTYPE(dtype, const size_t smem = StripWindow<T>::smem_bytes();
+                                    if (int rc = strip_smem_optin<conv3c3_strip_kernel<T, 0>>(smem, "conv_small_fwd")) return rc;
+                                    conv3c3_strip_kernel<T, 0><<<grid, kThreads, smem, stream>>>(
                                         reinterpret_cast<const T*>(in), w, in_a, in_b, act, reinterpret_cast<T*>(out), stats,
-                                        nullptr, nullptr, nullptr, B, H, W, th, tw)));
+                                        nullptr, nullptr, nullptr, B, H, W, th, tw));
     } else if (which == 1) {
         const int th = ceil_div(H, C3_TH), tw = ceil_div(W, C3_TW);
         const int grid = persist_grid_tiles((long long)B * th * tw, 2);
@@ -1063,10 +1064,11 @@ int spnet_conv_small_wgrad(int which, const void* in, const float* in_a, const f
     } else if (which == 1 && W % 8 == 0) {
         const int th = ceil_div(H, SK_TH), tw = ceil_div(W, SK_TW);
         const int grid = persist_grid_tiles((long long)B * th * tw, 1);
-        SPNET_DISPATCH_DTYPE(dtype, (strip_smem_optin(conv3c3_wgrad_strip_kernel<T>, StripWindow<T>::smem_bytes()),
-                                     conv3c3_wgrad_strip_kernel<T><<<grid, kThreads, StripWindow<T>::smem_bytes(), stream>>>(
+        SPNET_DISPATCH_DTYPE(dtype, const size_t smem = StripWindow<T>::smem_bytes();
+                                    if (int rc = strip_smem_optin<conv3c3_wgrad_strip_kernel<T>>(smem, "conv_small_wgrad")) return rc;
+                                    conv3c3_wgrad_strip_kernel<T><<<grid, kThreads, smem, stream>>>(
                                         reinterpret_cast<const T*>(in), in_a, in_b, act, reinterpret_cast<const T*>(g), dw,
-                                        dw_acc, B, H, W, th, tw)));
+                                        dw_acc, B, H, W, th, tw));
     } else if (which == 1) {
         const int th = ceil_div(H, C3W_TH), tw = ceil_div(W, C3_TW);
         const int grid = persist_grid_tiles((long long)B * th * tw, 2);
@@ -1098,10 +1100,11 @@ int spnet_conv_small_dgrad(int which, const void* g, const float* w, const void*
     if (which == 1 && W % 8 == 0) {
         const int th = ceil_div(H, SK_TH), tw = ceil_div(W, SK_TW);
         const int grid = persist_grid_tiles((long long)B * th * tw, 2);
-        SPNET_DISPATCH_DTYPE(dtype, (strip_smem_optin(conv3c3_strip_kernel<T, 2>, StripWindow<T>::smem_bytes()),
-                                     conv3c3_strip_kernel<T, 2><<<grid, kThreads, StripWindow<T>::smem_bytes(), stream>>>(
+        SPNET_DISPATCH_DTYPE(dtype, const size_t smem = StripWindow<T>::smem_bytes();
+                                    if (int rc = strip_smem_optin<conv3c3_strip_kernel<T, 2>>(smem, "conv_small_dgrad")) return rc;
+                                    conv3c3_strip_kernel<T, 2><<<grid, kThreads, smem, stream>>>(
                                         reinterpret_cast<const T*>(g), w, nullptr, nullptr, act, reinterpret_cast<T*>(gin),
-                                        nullptr, reinterpret_cast<const T*>(mask_z), mask_a, mask_b, B, H, W, th, tw)));
+                                        nullptr, reinterpret_cast<const T*>(mask_z), mask_a, mask_b, B, H, W, th, tw));
     } else if (which == 1) {
         // 'same' 3x3 stride 1: the data gradient is the convolution of g with the flipped, transposed kernel
         const int th = ceil_div(H, C3_TH), tw = ceil_div(W, C3_TW);

@@ -16,12 +16,6 @@ __device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint6
         ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate), "r"(leader)
         : "memory");
 }
-// one lane of a converged warp (always the same one), in a form the compiler recognises as "one thread"
-__device__ __forceinline__ uint32_t elect_one() {
-    uint32_t leader;
-    asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(leader));
-    return leader;
-}
 __device__ __forceinline__ void umma_commit(uint32_t bar, uint32_t leader) {
     asm volatile(
         "{\n\t.reg .pred q;\n\t"
@@ -43,6 +37,14 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
     asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 }
 
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
+// One warp allocates `ncols` TMEM columns (a power of two >= 32) for the CTA and writes their base address to the
+// shared-memory word at `holder`, then gives up the CTA's right to allocate more.
+__device__ __forceinline__ void tmem_alloc(uint32_t holder, uint32_t ncols) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(holder), "r"(ncols)
+                 : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+}
+// by the warp that allocated, once every tcgen05 access of the CTA is complete
+__device__ __forceinline__ void tmem_dealloc(uint32_t base, uint32_t ncols) {
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(base), "r"(ncols) : "memory");
 }
