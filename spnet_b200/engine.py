@@ -219,13 +219,17 @@ class SPNetEngineBase:
         n = int(np.prod(shape))
         return buf[:n].view(*shape)
 
+    def _uses_moving(self, bn):
+        """Whether bn normalises with its moving statistics inside a training step (see bn_use_moving)."""
+        return self.bn_use_moving == "all" or (self.bn_use_moving == "frozen" and bn.name in self.frozen_layers)
+
     def _bn_ready(self, bn, count, training):
         if training:
             # a frozen BatchNormalization (layer.trainable = False under Keras 2.1.3) still normalises with the batch
             # statistics in the training phase; what stops is the update of its moving averages (Layer.updates is
             # empty for a non-trainable layer) and of gamma / beta (Adam mask)
             frozen = bn.name in self.frozen_layers
-            moving = self.bn_use_moving == "all" or (frozen and self.bn_use_moving == "frozen")
+            moving = self._uses_moving(bn)
             ops.bn_finalize(bn.stats, count, bn.gamma, bn.beta, bn.a, bn.b, bn.mean, bn.rstd, None if (frozen or moving) else bn.mm,
                             None if (frozen or moving) else bn.mv, eps=arch.BN_EPS, momentum=arch.BN_MOMENTUM, unbiased=self.unbiased)
             if moving:
@@ -258,19 +262,18 @@ class SPNetEngineBase:
     def _pw_bwd(self, A, Wl, gW, gz, gA, M, K, N):
         """gz [M,N] -> gW [K,N] += A^T gz ;  gA [M,K] = gz W^T. gW None: the weight gradient is computed elsewhere
         (the batched launch over the middle flow)."""
-        if gW is None:
-            pass
-        elif self.deterministic:
-            # fixed-order split-K: partial products to slabs, added in split order (bit-identical run to run)
-            sp = self._wgrad_splits(K, N, M)
-            slabs = self._slab_buf(sp, K, N)
-            if sp > 1:
-                slabs[:sp * K * N].zero_()  # a slab the GEMM does not need must read as zero
-            ops.gemm(A, True, gz, True, slabs, K, N, M, out_mode=ops.OUT_SLAB, splits=sp, lda=K, ldb=N)
-            ops.slab_reduce(slabs, sp, K, N, gW, accumulate=True)
-        else:
-            sp = 0 if self.lowp else self._wgrad_splits(K, N, M)  # 0 = let the tcgen05 GEMM pick (fills the SMs once)
-            ops.gemm(A, True, gz, True, gW, K, N, M, out_mode=ops.OUT_ATOMIC, splits=sp, lda=K, ldb=N)
+        if gW is not None:
+            if self.deterministic:
+                # fixed-order split-K: partial products to slabs, added in split order (bit-identical run to run)
+                sp = self._wgrad_splits(K, N, M)
+                slabs = self._slab_buf(sp, K, N)
+                if sp > 1:
+                    slabs[:sp * K * N].zero_()  # a slab the GEMM does not need must read as zero
+                ops.gemm(A, True, gz, True, slabs, K, N, M, out_mode=ops.OUT_SLAB, splits=sp, lda=K, ldb=N)
+                ops.slab_reduce(slabs, sp, K, N, gW, accumulate=True)
+            else:
+                sp = 0 if self.lowp else self._wgrad_splits(K, N, M)  # 0 = let the tcgen05 GEMM pick (fills the SMs once)
+                ops.gemm(A, True, gz, True, gW, K, N, M, out_mode=ops.OUT_ATOMIC, splits=sp, lda=K, ldb=N)
         if gA is not None:
             ops.gemm(gz, False, Wl, False, gA, M, K, N, out_mode=ops.OUT_T, ldb=N)
 
@@ -278,12 +281,17 @@ class SPNetEngineBase:
         """The BatchNorm backward and both pointwise GEMMs of a K -> N layer run as one kernel (csrc/pw_bwd.cu)."""
         return self.lowp and N == 128 and K in (64, 128)
 
-    def _bn_pw_bwd(self, g, z, bn, A, Wl, gW, gA, M, K, N):
-        """g = grad wrt the output of the BatchNorm of z = A W -> gA [M,K] = dz W^T, gW [K,N] += A^T dz, with
-        dz = _bn_bwd(g, z, bn, M, reduced=True) never leaving the chip (g is left as it is)."""
-        ops.bn_bwd_finalize(bn.stats, self._bwd_count(bn, M), bn.ggamma, bn.gbeta, bn.c1, bn.c2)
-        slabs = self._slab_buf(ops.pw_bwd_bn_slabs(M, self.device), K, N) if self.deterministic else None
-        ops.pw_bwd_bn(g, z, A, Wl, bn.a, bn.mean, bn.rstd, bn.c1, bn.c2, gA, gW, M, K, N, slabs=slabs)
+    def _bn_pw_bwd(self, g, z, bn, A, Wl, gW, gA, M, K, N, dz=None):
+        """g = grad wrt the output of BatchNorm bn of z = A W, its sums already in bn.stats -> gA [M,K] = dz W^T and
+        gW [K,N] += A^T dz (gW None: computed elsewhere from the stored dz). One kernel where _pw_bwd_fusable, dz never
+        leaving the chip and g left as it is; otherwise dz is stored in dz, or over g when dz is None."""
+        if gW is not None and self._pw_bwd_fusable(K, N):
+            ops.bn_bwd_finalize(bn.stats, self._bwd_count(bn, M), bn.ggamma, bn.gbeta, bn.c1, bn.c2)
+            slabs = self._slab_buf(ops.pw_bwd_bn_slabs(M, self.device), K, N) if self.deterministic else None
+            ops.pw_bwd_bn(g, z, A, Wl, bn.a, bn.mean, bn.rstd, bn.c1, bn.c2, gA, gW, M, K, N, slabs=slabs)
+        else:
+            dz = self._bn_bwd(g, z, bn, M, out=dz)
+            self._pw_bwd(A, Wl, gW, dz.view(M, N), gA, M, K, N)
 
     def _sep_fwd(self, s, x, in_bn, relu, training):
         B = self.B
@@ -292,15 +300,20 @@ class SPNetEngineBase:
         self._pw_fwd(s.t, s.pwl, s.z, M, s.cin, s.cout, s.bn, training)
 
     def _bwd_count(self, bn, rows):
-        moving = self.bn_use_moving == "all" or (self.bn_use_moving == "frozen" and bn.name in self.frozen_layers)
-        return 0 if moving else rows  # count 0: bn_bwd_finalize drops the batch-statistics terms (c1 = c2 = 0)
+        # count 0: bn_bwd_finalize drops the batch-statistics terms (c1 = c2 = 0)
+        return 0 if self._uses_moving(bn) else rows
 
-    def _bn_bwd(self, g, z, bn, rows, relu_mask=False, out=None, reduced=False):
-        """g = grad wrt BN output (or wrt relu(BN output) when relu_mask) -> grad wrt z.
-        reduced=True: the sums were already accumulated into bn.stats by the producer of g."""
-        if not reduced:
-            ops.bn_bwd_reduce(g, z, bn.mean, bn.rstd, bn.stats, relu_a=bn.a if relu_mask else None,
-                              relu_b=bn.b if relu_mask else None, act=1)
+    def _bn_bwd_sums(self, g, z, bn, act=None):
+        """Accumulates bn's backward sums over g into bn.stats: the step for a gradient whose producer does not. g = grad
+        wrt the BN output; with act (1 = ReLU, 3 = ReLU6) g = grad wrt act(BN output), masked in place by act' first."""
+        if act is None:
+            ops.bn_bwd_reduce(g, z, bn.mean, bn.rstd, bn.stats)
+        else:
+            ops.bn_bwd_reduce(g, z, bn.mean, bn.rstd, bn.stats, relu_a=bn.a, relu_b=bn.b, act=act)
+
+    def _bn_bwd(self, g, z, bn, rows, out=None):
+        """g = grad wrt the BN output, its backward sums already in bn.stats (accumulated by the producer of g or by
+        _bn_bwd_sums) -> grad wrt z, stored in out (default: over g)."""
         ops.bn_bwd_finalize(bn.stats, self._bwd_count(bn, rows), bn.ggamma, bn.gbeta, bn.c1, bn.c2)
         return ops.bn_bwd_dz(g, z, bn.a, bn.mean, bn.rstd, bn.c1, bn.c2, out=out if out is not None else g)
 
@@ -355,21 +368,19 @@ class SPNetEngineBase:
             ops.acc_to_f32(self.l2_acc, self.l2_out)
 
     # ------------------------------------------------------------------ backward
-    def _sep_bwd(self, s, gz, x, in_bn, relu, g_t, g_in, add_src=None, add_strided=None, wgrad=True, out_bn=None,
-                 gz_bn=False):
-        """gz: grad wrt s.z [B,H,W,cout] (gz_bn: grad wrt the output of s.bn, its sums already accumulated; the
-        BatchNorm backward then runs inside the pointwise backward). Produces the gradient wrt the sepconv's input tensor x
-        (before its on-load BN/ReLU transform) in g_in; for a BN'd input this is still the grad wrt
-        the BN OUTPUT (masked by relu'), to be pushed through _bn_bwd by the caller.
+    def _sep_bwd(self, s, g, x, in_bn, relu, g_t, g_in, add_src=None, add_strided=None, wgrad=True, out_bn=None,
+                 dz=None):
+        """g: grad wrt the output of s.bn [M,cout], its backward sums already in s.bn.stats. The BatchNorm and pointwise
+        backward run as _bn_pw_bwd (grad wrt s.t in g_t; dz as there; wgrad=False: the pointwise weight gradient is
+        computed elsewhere from dz). Produces the gradient wrt the sepconv's input tensor x (before its on-load BN/ReLU
+        transform) in g_in; for a BN'd input in_bn this is the grad wrt in_bn's OUTPUT (masked by relu'), with in_bn's
+        backward sums accumulated.
         out_bn = (z, bn, relu_mask): x = [relu](bn(z)) [+ ...], the BN that produced the UNtransformed input x. The
         depthwise backward then accumulates that BN's backward sums on the final g_in (masked by the ReLU when
-        relu_mask), so the caller's _bn_bwd on g_in runs with reduced=True."""
+        relu_mask), so the caller can go straight to _bn_bwd on g_in's residual path."""
         B = self.B
         M = B * s.H * s.W
-        if gz_bn:
-            self._bn_pw_bwd(gz, s.z, s.bn, s.t, s.pwl, s.gpw, g_t, M, s.cin, s.cout)
-        else:
-            self._pw_bwd(s.t, s.pwl, s.gpw if wgrad else None, gz, g_t, M, s.cin, s.cout)
+        self._bn_pw_bwd(g, s.z, s.bn, s.t, s.pwl, s.gpw if wgrad else None, g_t, M, s.cin, s.cout, dz=dz)
         gt4 = g_t.view(B, s.H, s.W, s.cin)
         zo, zbn, zmask = out_bn if out_bn else (None, None, False)
         ops.dwconv3x3_bwd_fused(gt4, x, s.dwk, s.gdwk, in_a=in_bn.a if in_bn else None, in_b=in_bn.b if in_bn else None,
@@ -381,8 +392,9 @@ class SPNetEngineBase:
                                 mask_b=zbn.b if zmask else None)
 
     def _entry_bwd(self, e, x, g_out, bufs, x_bn):
-        """g_out: grad wrt block output [B,oh,ow,c], its residual BN's backward sums already accumulated (by the
-        producer of g_out). Returns grad wrt block input x, with the sums of x's BN x_bn = (z, bn, relu_mask)."""
+        """g_out: grad wrt block output [B,oh,ow,c], the backward sums of its residual BN already accumulated (by the
+        producer of g_out); it is left as it is. Returns grad wrt block input x, with the sums of x's BN
+        x_bn = (z, bn, relu_mask) accumulated."""
         B = self.B
         (H, W), (oh, ow) = e["hw"], e["ohw"]
         cin, c = e["cin"], e["c"]
@@ -390,26 +402,18 @@ class SPNetEngineBase:
         Mo = B * oh * ow
         M = B * H * W
         s1, s2 = e["sep1"], e["sep2"]
-        # residual branch (g_out is read again by the max-pool backward: the unfused route writes dz to G1)
+        # residual branch (g_out is read again by the max-pool backward: dz goes to G1, not over g_out)
         g_xs = self._view(S, Mo, cin)
-        xs, Wr, gWr = e["xs"].view(Mo, cin), self.wl[e["res"] + "/kernel"].view(cin, c), self.g[e["res"] + "/kernel"].view(cin, c)
-        if self._pw_bwd_fusable(cin, c):
-            self._bn_pw_bwd(g_out, e["zr"], e["res_bn"], xs, Wr, gWr, g_xs, Mo, cin, c)
-        else:
-            g_zr = self._bn_bwd(g_out, e["zr"], e["res_bn"], Mo, out=self._view(G1, B, oh, ow, c), reduced=True)
-            self._pw_bwd(xs, Wr, gWr, g_zr.view(Mo, c), g_xs, Mo, cin, c)
+        self._bn_pw_bwd(g_out, e["zr"], e["res_bn"], e["xs"].view(Mo, cin), self.wl[e["res"] + "/kernel"].view(cin, c),
+                        self.g[e["res"] + "/kernel"].view(cin, c), g_xs, Mo, cin, c, dz=self._view(G1, Mo, c))
         # main branch
         g_y2 = ops.maxpool3s2_bwd(g_out, e["argmax"], H, W, out=self._view(G1, B, H, W, c), z=s2.z, mean=s2.bn.mean,
                                   rstd=s2.bn.rstd, stats=s2.bn.stats)
         g_y1 = self._view(G3, B, H, W, s2.cin)
-        fuse2 = self._pw_bwd_fusable(s2.cin, c)
-        g_z2 = g_y2 if fuse2 else self._bn_bwd(g_y2, s2.z, s2.bn, M, reduced=True)
-        self._sep_bwd(s2, g_z2.view(M, c), s1.z, s1.bn, True, self._view(G2, M, s2.cin), g_y1, gz_bn=fuse2)
-        fuse1 = self._pw_bwd_fusable(cin, s1.cout)
-        g_z1 = g_y1 if fuse1 else self._bn_bwd(g_y1, s1.z, s1.bn, M, reduced=True)
+        self._sep_bwd(s2, g_y2.view(M, c), s1.z, s1.bn, True, self._view(G2, M, s2.cin), g_y1)
         g_x = self._view(R, B, H, W, cin)
-        self._sep_bwd(s1, g_z1.view(M, s1.cout), x, None, e["relu_in"], self._view(G1, M, cin), g_x,
-                      add_strided=g_xs.view(B, oh, ow, cin), out_bn=x_bn, gz_bn=fuse1)
+        self._sep_bwd(s1, g_y1.view(M, s1.cout), x, None, e["relu_in"], self._view(G1, M, cin), g_x,
+                      add_strided=g_xs.view(B, oh, ow, cin), out_bn=x_bn)
         return g_x
 
     def backward_head(self):
@@ -724,15 +728,19 @@ class XceptionSPNetEngine(SPNetEngineBase):
             e["argmax"] = A(B, oh, ow, e["c"], dtype=torch.uint8) if train else None
         mh, mw = sh["middle"]
         # the depthwise outputs t (the A operand of every pointwise weight gradient) of the 24 identical middle-flow
-        # layers are ONE contiguous [24, B*mh*mw, 728] tensor, and so are the gradients dz reaching their pointwise
+        # layers are ONE contiguous [24, Mpad, 728] tensor, and so are the gradients dz reaching their pointwise
         # convolutions: the 24 weight gradients dW_i = t_i^T dz_i are then a single GEMM launch whose K range is cut
-        # into 24 slabs (ops.gemm out_mode OUT_SLAB), each stored straight into the flat gradient buffer
-        nmid = 3 * len(self.middle)
-        self.mid_t = A(nmid, B, mh, mw, 728)
-        self.mid_dz = A(nmid, B, mh, mw, 728) if train else None
+        # into 24 slabs (ops.gemm out_mode OUT_SLAB), each stored straight into the flat gradient buffer. Each layer's
+        # M = B*mh*mw rows are padded to Mpad, a multiple of the GEMM's k-block (64 rows bf16, 16 fp32), so that no
+        # k-block straddles two layers; the pad rows are zero (nothing writes them) and add nothing to dW_i
+        nmid, M = 3 * len(self.middle), B * mh * mw
+        kb = 64 if self.lowp else 16
+        Mpad = -(-M // kb) * kb
+        self.mid_t = torch.zeros(nmid, Mpad, 728, device=self.device, dtype=self.adt)
+        self.mid_dz = torch.zeros(nmid, Mpad, 728, device=self.device, dtype=self.adt) if train else None
         for bi, blk in enumerate(self.middle):
             for j, s in enumerate(blk):
-                s.t = self.mid_t[3 * bi + j]
+                s.t = self.mid_t[3 * bi + j, :M].view(B, mh, mw, 728)
                 s.z = A(B, mh, mw, 728)
         self.mid_out = [A(B, mh, mw, 728) for _ in self.middle]
         fh, fw = sh["out13"]
@@ -743,15 +751,12 @@ class XceptionSPNetEngine(SPNetEngineBase):
         if train:
             self.gcol = None if self.lowp else A(B * h2 * w2, 288)  # bf16: the data gradient is an implicit GEMM
             self.scratch = [A(maxel) for _ in range(6)]
-            # batched middle-flow weight gradient: needs the 24 pointwise kernels equally spaced in the flat gradient
-            # buffer (they are: every layer contributes dw kernel + pw kernel + gamma + beta) and k-blocks that do
-            # not straddle two layers (rows per layer a multiple of the GEMM's 64 / 16-row k-block)
+            # batched middle-flow weight gradient: the 24 pointwise kernels are equally spaced in the flat gradient
+            # buffer (every layer contributes dw kernel + pw kernel + gamma + beta, 728 * 739 parameters)
             o0 = self.offsets["block5_sepconv1/pointwise_kernel"][0]
             stride = self.offsets["block5_sepconv2/pointwise_kernel"][0] - o0
             names = ["block%d_sepconv%d/pointwise_kernel" % (b, j) for b in arch.MIDDLE_BLOCKS for j in (1, 2, 3)]
-            even = all(self.offsets[n][0] == o0 + i * stride for i, n in enumerate(names))
-            rows = B * mh * mw
-            self.mid_batched = even and rows % (64 if self.lowp else 16) == 0
+            assert all(self.offsets[n][0] == o0 + i * stride for i, n in enumerate(names))
             self.mid_gw_off, self.mid_gw_stride = o0, stride
 
     def _backbone_fwd(self, training):
@@ -799,12 +804,12 @@ class XceptionSPNetEngine(SPNetEngineBase):
         fh, fw = sh["out13"]
         M = B * fh * fw
         x13 = self.exit13["out"]
-        g_z = self._bn_bwd(self.gfeat.view(B, fh, fw, 2048), s2.z, s2.bn, M, relu_mask=True)
+        g_feat = self.gfeat.view(M, 2048)
+        self._bn_bwd_sums(g_feat, s2.z, s2.bn, act=1)
         g_y = self._view(G3, B, fh, fw, 1536)
-        self._sep_bwd(s2, g_z.view(M, 2048), s1.z, s1.bn, True, self._view(G2, M, 1536), g_y)
-        g_z = self._bn_bwd(g_y, s1.z, s1.bn, M, reduced=True)
+        self._sep_bwd(s2, g_feat, s1.z, s1.bn, True, self._view(G2, M, 1536), g_y)
         g_x = self._view(R0, B, fh, fw, 1024)
-        self._sep_bwd(s1, g_z.view(M, 1536), x13, None, False, self._view(G1, M, 1024), g_x,
+        self._sep_bwd(s1, g_y.view(M, 1536), x13, None, False, self._view(G1, M, 1024), g_x,
                       out_bn=(self.exit13["zr"], self.exit13["res_bn"], False))
         # ---- exit block 13
         R_cur, R_nxt = R0, R1
@@ -815,35 +820,31 @@ class XceptionSPNetEngine(SPNetEngineBase):
         # ---- middle blocks 12..5
         mh, mw = sh["middle"]
         M = B * mh * mw
-        bat = self.mid_batched
         for i in range(len(self.middle) - 1, -1, -1):
             blk = self.middle[i]
             x_in = self.mid_out[i - 1] if i > 0 else self.entry[-1]["out"]
             # the BN on x_in's residual path: the previous middle block's sepconv3 BN or entry block 4's residual BN
             x_bn = (self.middle[i - 1][2].z, self.middle[i - 1][2].bn, False) if i > 0 else \
                 (self.entry[-1]["zr"], self.entry[-1]["res_bn"], False)
-            # with the batched weight gradient every dz is kept (mid_dz) until the end of the middle flow
-            dz3, dz2, dz1 = (self.mid_dz[3 * i + 2], self.mid_dz[3 * i + 1], self.mid_dz[3 * i]) if bat else (None, None, None)
-            g3 = self._bn_bwd(g_x, blk[2].z, blk[2].bn, M, out=dz3 if bat else self._view(G1, B, mh, mw, 728), reduced=True)
-            gy2 = self._view(G3, B, mh, mw, 728)
-            self._sep_bwd(blk[2], g3.view(M, 728), blk[1].z, blk[1].bn, True, self._view(G2, M, 728), gy2, wgrad=not bat)
-            g2 = self._bn_bwd(gy2, blk[1].z, blk[1].bn, M, reduced=True, out=dz2)
-            gy1 = self._view(G1, B, mh, mw, 728)
-            self._sep_bwd(blk[1], g2.view(M, 728), blk[0].z, blk[0].bn, True, self._view(G2, M, 728), gy1, wgrad=not bat)
-            g1 = self._bn_bwd(gy1, blk[0].z, blk[0].bn, M, reduced=True, out=dz1)
+            # every dz is kept (mid_dz) for the batched weight gradient at the end of the middle flow (g_x is read again
+            # as blk[0]'s add_src)
+            dz = [self.mid_dz[3 * i + j, :M] for j in range(3)]
+            g_t = self._view(G2, M, 728)
+            gy2, gy1 = self._view(G3, B, mh, mw, 728), self._view(G1, B, mh, mw, 728)
+            self._sep_bwd(blk[2], g_x.view(M, 728), blk[1].z, blk[1].bn, True, g_t, gy2, wgrad=False, dz=dz[2])
+            self._sep_bwd(blk[1], gy2.view(M, 728), blk[0].z, blk[0].bn, True, g_t, gy1, wgrad=False, dz=dz[1])
             g_new = self._view(R_nxt, B, mh, mw, 728)
-            self._sep_bwd(blk[0], g1.view(M, 728), x_in, None, True, self._view(G2, M, 728), g_new, add_src=g_x, wgrad=not bat,
-                          out_bn=x_bn)
+            self._sep_bwd(blk[0], gy1.view(M, 728), x_in, None, True, g_t, g_new, add_src=g_x, wgrad=False, out_bn=x_bn,
+                          dz=dz[0])
             g_x = g_new
             R_cur, R_nxt = R_nxt, R_cur
-        if bat:
-            # dW_i = t_i^T dz_i for the 24 layers in ONE launch: both operands stacked along K (pixel rows), split s of the
-            # K range = layer s, its [728, 728] product stored at the layer's place in the flat gradient buffer. No
-            # split-K reduce-adds (every output tile has ONE writer: also bit-identical run to run), 192 k-blocks per
-            # tile instead of 24 launches with ~10 k-blocks per CTA each
-            n = len(self.middle) * 3
-            ops.gemm(self.mid_t.view(n * M, 728), True, self.mid_dz.view(n * M, 728), True, self.grads[self.mid_gw_off:], 728, 728,
-                     n * M, out_mode=ops.OUT_SLAB, splits=n, lda=728, ldb=728, ldd=728, slab_stride=self.mid_gw_stride)
+        # dW_i = t_i^T dz_i for the 24 layers in ONE launch: both operands stacked along K (pixel rows, Mpad per layer),
+        # split s of the K range = layer s, its [728, 728] product stored at the layer's place in the flat gradient
+        # buffer. No split-K reduce-adds (every output tile has ONE writer: also bit-identical run to run), 192 k-blocks
+        # per tile instead of 24 launches with ~10 k-blocks per CTA each
+        n, Mpad = self.mid_t.shape[:2]
+        ops.gemm(self.mid_t.view(n * Mpad, 728), True, self.mid_dz.view(n * Mpad, 728), True, self.grads[self.mid_gw_off:], 728,
+                 728, n * Mpad, out_mode=ops.OUT_SLAB, splits=n, lda=728, ldb=728, ldd=728, slab_stride=self.mid_gw_stride)
         self._bwd_state = (g_x, R_cur, R_nxt)
 
     def _backbone_bwd_b(self, ga):
@@ -864,7 +865,7 @@ class XceptionSPNetEngine(SPNetEngineBase):
         h1, w1 = sh["b1c1"]
         M2 = B * h2 * w2
         # masked by the block-1 ReLU, with its sums, by block2_sepconv1's depthwise backward
-        g_z12 = self._bn_bwd(g_x, self.z12, self.b1_bn2, M2, reduced=True)
+        g_z12 = self._bn_bwd(g_x, self.z12, self.b1_bn2, M2)
         W2l = self.wl["block1_conv2/kernel"].view(288, 64)
         g_y11 = self._view(G1, B, h1, w1, 32)
         if self.b1_fold:
@@ -878,7 +879,8 @@ class XceptionSPNetEngine(SPNetEngineBase):
         else:
             ops.col2im(self.gcol, g_y11, 3, 3, 1, 0, 0, h2, w2)
         # the ReLU mask of block1_conv1_act is applied by the BatchNorm-backward reduction
-        g_z11 = self._bn_bwd(g_y11, self.z11, self.b1_bn1, B * h1 * w1, relu_mask=True)
+        self._bn_bwd_sums(g_y11, self.z11, self.b1_bn1, act=1)
+        g_z11 = self._bn_bwd(g_y11, self.z11, self.b1_bn1, B * h1 * w1)
         ops.conv_small_wgrad(2, self.d, g_z11, g["block1_conv1/kernel"], acc=self._gacc)
         ops.conv_small_dgrad(2, g_z11, w["block1_conv1/kernel"], ga)
 
@@ -962,8 +964,7 @@ class MobileNetSPNetEngine(SPNetEngineBase):
         fh, fw, fc = self.feat_dims
         # gradient w.r.t. relu6(BN(zp13)) -> masked in place, BN-backward sums accumulated
         g_y = self.gfeat.view(B, fh, fw, fc)
-        ops.bn_bwd_reduce(g_y, last["zp"], last["bn_pw"].mean, last["bn_pw"].rstd, last["bn_pw"].stats,
-                          relu_a=last["bn_pw"].a, relu_b=last["bn_pw"].b, act=3)
+        self._bn_bwd_sums(g_y, last["zp"], last["bn_pw"], act=3)
         cur = None  # scratch buffer holding g_y (None: self.gfeat)
         for idx in range(len(self.blocks) - 1, -1, -1):
             b = self.blocks[idx]
@@ -973,13 +974,12 @@ class MobileNetSPNetEngine(SPNetEngineBase):
             x, xbn = (self.blocks[idx - 1]["zp"], self.blocks[idx - 1]["bn_pw"]) if idx > 0 else (self.zc1, self.c1_bn)
             tb, fb, nb = [i for i in range(4) if i != cur][:3]
             # pointwise BN + 1x1 (g_y already carries the ReLU6 mask and this BN's backward sums)
-            g_zp = self._bn_bwd(g_y, b["zp"], b["bn_pw"], M, reduced=True)
+            g_zp = self._bn_bwd(g_y, b["zp"], b["bn_pw"], M)
             g_t = self._view(bufs[tb], B, oh, ow, cin)
             self._pw_bwd(b["t"].view(M, cin), b["pwl"], b["gpw"], g_zp.view(M, cout), g_t.view(M, cin), M, cin, cout)
             # depthwise BN (+ReLU6 mask)
-            ops.bn_bwd_reduce(g_t, b["zd"], b["bn_dw"].mean, b["bn_dw"].rstd, b["bn_dw"].stats, relu_a=b["bn_dw"].a,
-                              relu_b=b["bn_dw"].b, act=3)
-            g_zd = self._bn_bwd(g_t, b["zd"], b["bn_dw"], M, reduced=True)
+            self._bn_bwd_sums(g_t, b["zd"], b["bn_dw"], act=3)
+            g_zd = self._bn_bwd(g_t, b["zd"], b["bn_dw"], M)
             g_full = ops.scatter_s2(g_zd, self._view(bufs[fb], B, h, wd, cin), off=b["off"]) if b["s"] == 2 else g_zd
             # depthwise 3x3: gradient w.r.t. relu6(BN_prev(x)) (masked) + BN_prev backward sums + dk
             g_y = self._view(bufs[nb], B, h, wd, cin)
@@ -987,7 +987,7 @@ class MobileNetSPNetEngine(SPNetEngineBase):
                                     bn_rstd=xbn.rstd, stats=xbn.stats, out=g_y, acc=self._gacc)
             cur = nb
         h, wd = self.shapes["conv1"]
-        g_zc1 = self._bn_bwd(g_y, self.zc1, self.c1_bn, B * h * wd, reduced=True)
+        g_zc1 = self._bn_bwd(g_y, self.zc1, self.c1_bn, B * h * wd)
         ops.conv_small_wgrad(3, self.d, g_zc1, g["conv1/kernel"], acc=self._gacc)
         ops.conv_small_dgrad(3, g_zc1, w["conv1/kernel"], ga)
 
@@ -1132,11 +1132,8 @@ class InceptionResNetV2SPNetEngine(SPNetEngineBase):
             M = B * o.h * o.w
             if kind == "conv_bn":
                 bn, z = op["bnrec"], op["z"]
-                if op["act"]:
-                    ops.bn_bwd_reduce(gy, z, bn.mean, bn.rstd, bn.stats, relu_a=bn.a, relu_b=bn.b, act=1)
-                else:
-                    ops.bn_bwd_reduce(gy, z, bn.mean, bn.rstd, bn.stats)
-                dz = self._bn_bwd(gy, z, bn, M, reduced=True)
+                self._bn_bwd_sums(gy, z, bn, act=1 if op["act"] else None)
+                dz = self._bn_bwd(gy, z, bn, M)
                 gW = g_[op["name"] + "/kernel"]
                 if op["cin"] == 3:
                     ops.conv_small_wgrad(2, xs[0], dz, gW, acc=self._gacc)
