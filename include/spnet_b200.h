@@ -68,6 +68,11 @@ int spnet_yolo_ellipse_loss_ann(const double* ann, const int* counts, int max_ob
 /* load_X_one_proc's (v/255 - 0.5)*2 (spnet/utils.py:340-342) on the device: uint8 frames cross PCIe, lut [256] fp32
  * holds the 256 possible results as numpy computes them (bit-exact by construction). */
 int spnet_normalize_u8(const unsigned char* in, const float* lut, float* out, long long n, cudaStream_t stream);
+/* load_X_one_proc's LANCZOS resize to force_dim (spnet/utils.py:325-349, PIL Image.resize) fused with the normalisation
+ * above: in uint8 [n,H,W] -> out fp32 [n,OH,OW] = lut[resized byte], the bytes bit-identical to Pillow's 8-bit resample.
+ * xbounds [OW,2] / ybounds [OH,2] int32 = (first input index, tap count), xcoeffs [OW,kx] / ycoeffs [OH,ky] int32 in
+ * units of 2^-22: Pillow's tables for (W -> OW) and (H -> OH) (spnet_b200/ops.py lanczos_tables). */
+int spnet_resize_lanczos_u8(const unsigned char* in, int n, int H, int W, const int* xbounds, const int* xcoeffs, int kx, const int* ybounds, const int* ycoeffs, int ky, const float* lut, float* out, int OH, int OW, cudaStream_t stream);
 
 /* ---- Evaluation metrics (spnet/diagnostics.py: calc_errors :13-60; compute_iou :85-120 for every (image, slot)
  *      pair, analytic ellipse raster with an anti-aliasing margin instead of cv2). yp / yt: denormalised fp32

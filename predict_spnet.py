@@ -36,8 +36,9 @@ def predict_network(weights_file="spnet.model", datapath=default_image_dir, frac
     # ALONE (the other ranks have left), so it must not wait for their CSV parts
     rank, world = ranks if ranks is not None else _ranks()
     shard_lo = 0
-    streaming = stream_chunk is not None and isinstance(X_pred, str) and "" == X_pred
-    if isinstance(X_pred, str) and "" == X_pred:
+    from_dir = isinstance(X_pred, str) and "" == X_pred
+    streaming = stream_chunk is not None and from_dir
+    if from_dir:
         print(f"Getting data from {datapath}, fraction = {fraction}.")
         if cf.model_type == "simple":
             grayscale, force_dim = False, 224
@@ -61,32 +62,52 @@ def predict_network(weights_file="spnet.model", datapath=default_image_dir, frac
             img_file_list = img_file_list[shard_lo:shard_lo + per + (1 if rank < extra else 0)]
             total_load = len(img_file_list)
             print("      rank %d / %d: frames [%d, %d)" % (rank, world, shard_lo, shard_lo + total_load))
-        if streaming:
-            chunks = utils.stream_X(img_file_list, int(stream_chunk), force_dim=force_dim, grayscale=grayscale, raw_u8=raw_u8)
-            first_lo, X_pred = next(chunks)  # the model is set up from the first chunk's frame shape
-        else:
-            X_pred, img_dims = utils.build_X(total_load, img_file_list, force_dim=force_dim, grayscale=grayscale, raw_u8=raw_u8)
-        print("")
     if model is None:
         print("Loading model from", weights_file)
         if ".hdf5" in weights_file:
             print("   Defining model, then loading weights")
+            if from_dir:  # setup_model reads only X[0].shape: the frame shape the loaders will deliver
+                if force_dim is None:
+                    from PIL import Image
+                    w, h = Image.open(img_file_list[0]).size
+                    X_pred = np.zeros((1, h, w, 1 if grayscale else 3), np.float32)
+                else:
+                    X_pred = np.zeros((1, force_dim, force_dim, 1 if grayscale else 3), np.float32)
             model, serial_model = models.setup_model(X_pred, try_checkpoint=True, no_cp_fatal=True,
                                                      weights_file=weights_file, parallel=False, freeze_fac=0.0,
                                                      quick_setup=True)
         else:
             print("   Loading whole model")
             model = models.load_model(weights_file)
+    # frames whose model input is the force_dim square travel at their decoded size and are resized on the GPU, the
+    # same bytes as PIL's LANCZOS (a directory of mixed frame sizes is resized on the host, as the loaders fall back)
+    defer = (from_dir and raw_u8 and grayscale and force_dim is not None
+             and (getattr(model, "H", None), getattr(model, "W", None)) == (force_dim, force_dim))
+
+    def predict(X):
+        if defer:
+            return model.predict(X, batch_size=batch_size, resize=tuple(X.shape[1:3]) != (force_dim, force_dim))
+        return model.predict(X, batch_size=batch_size)
+
+    if from_dir:
+        if streaming:
+            chunks = utils.stream_X(img_file_list, int(stream_chunk), force_dim=force_dim, grayscale=grayscale, raw_u8=raw_u8,
+                                    defer_resize=defer)
+            first_lo, X_pred = next(chunks)
+        else:
+            X_pred, img_dims = utils.build_X(total_load, img_file_list, force_dim=force_dim, grayscale=grayscale,
+                                             raw_u8=raw_u8, defer_resize=defer)
+        print("")
     m = len(img_file_list) if streaming else X_pred.shape[0]
     print("    Predicting... (m = ", m, " frames in dataset)", sep="")
     start_time = time.time()
     if streaming:
-        parts = [model.predict(X_pred, batch_size=batch_size)]
+        parts = [predict(X_pred)]
         for _, Xc in chunks:
-            parts.append(model.predict(Xc, batch_size=batch_size))
+            parts.append(predict(Xc))
         Y_pred = np.concatenate(parts, axis=0)
     else:
-        Y_pred = model.predict(X_pred, batch_size=batch_size)
+        Y_pred = predict(X_pred)
     elapsed = time.time() - start_time
     print("    ...elapsed time to predict = ", elapsed, "s.   FPS = ", m * 1.0 / elapsed)
 

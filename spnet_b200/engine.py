@@ -603,8 +603,8 @@ class SPNetEngineBase:
         self._ensure_stage()
         cs = self._copy_stream
         u8 = x_host.dtype == torch.uint8
-        if u8 and self._xs_u8 is None:
-            self._xs_u8 = torch.empty(self.x0.shape, device=self.device, dtype=torch.uint8)
+        if u8 and (self._xs_u8 is None or self._xs_u8.shape[1:3] != x_host.shape[1:3]):
+            self._xs_u8 = torch.empty((self.B,) + tuple(x_host.shape[1:3]), device=self.device, dtype=torch.uint8)
         with torch.cuda.stream(cs):
             cs.wait_event(self._stage_free)  # the previous staged batch has been taken
             if u8:
@@ -625,18 +625,32 @@ class SPNetEngineBase:
         main = torch.cuda.current_stream()
         main.wait_event(self._stage_ready)
         if self._staged_u8:
-            ops.normalize_u8(self._xs_u8, self.x0)  # (v/255 - 0.5)*2, spnet/utils.py:340-342
+            self.frames_to_x0(self._xs_u8)
         else:
             self.x0.copy_(self._xs)
         if self._has_y:
             self.y_true.copy_(self._ys)
         self._stage_free.record(main)
 
+    def frames_to_x0(self, x_u8):
+        """uint8 frames [m, h, w(, 1)] on the device -> self.x0[:m]: (v/255 - 0.5)*2 of spnet/utils.py:340-342, after a
+        LANCZOS resize to the engine's (H, W) when (h, w) differs - the bytes of the host's PIL resize (:325-349)."""
+        m = x_u8.shape[0]
+        if m > self.B or x_u8.dim() < 3 or x_u8.numel() != m * x_u8.shape[1] * x_u8.shape[2]:
+            raise ValueError("frames %s for an engine of batch %d: want [<= %d, h, w(, 1)] uint8" % (tuple(x_u8.shape), self.B, self.B))
+        if tuple(x_u8.shape[1:3]) == (self.H, self.W):
+            if x_u8.data_ptr() % 16:  # normalize_u8 reads 16-byte vectors; a slice of odd-sized frames may start anywhere
+                x_u8 = x_u8.clone()
+            ops.normalize_u8(x_u8, self.x0[:m])
+        else:
+            ops.resize_lanczos_u8(x_u8, self.H, self.W, out=self.x0[:m])
+
     def load_batch(self, x_host, y_host=None):
-        """H2D copy of one batch (numpy or pinned torch tensors; uint8 frames are normalised on the device)."""
+        """H2D copy of one batch (numpy or pinned torch tensors; uint8 frames are normalised - and resized when their size
+        is not the engine's - on the device)."""
         if (torch.is_tensor(x_host) and x_host.dtype == torch.uint8) or (not torch.is_tensor(x_host) and np.asarray(x_host).dtype == np.uint8):
             xt = x_host if torch.is_tensor(x_host) else torch.from_numpy(np.ascontiguousarray(x_host))
-            ops.normalize_u8(xt.view(self.x0.shape).to(self.device, non_blocking=True), self.x0)
+            self.frames_to_x0(xt.to(self.device, non_blocking=True).contiguous())
         else:
             xt = x_host if torch.is_tensor(x_host) else torch.from_numpy(np.ascontiguousarray(x_host, dtype=np.float32))
             self.x0.copy_(xt.view(self.x0.shape), non_blocking=True)

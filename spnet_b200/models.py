@@ -329,14 +329,19 @@ class SPNetModel:
         return eng
 
     # ---- inference ----------------------------------------------------------------------------
-    def predict(self, X, batch_size=32, verbose=0):
+    def predict(self, X, batch_size=32, verbose=0, resize=False):
         """Keras Model.predict (reference call site predict_spnet.py:85): inference-mode forward over X in batches.
         X: numpy / torch array (n, H, W, 1), float32 already normalised, or uint8 raw pixel values (normalised on the
         device, (v/255 - 0.5)*2 of spnet/utils.py:340-342 bit for bit; a quarter of the host->device bytes).
+        resize=True: X holds uint8 frames (n, h, w, 1) as decoded (utils.build_X(..., defer_resize=True)), on the host
+        or the device; each is LANCZOS-resized to the model's (H, W) on the device, the bytes of the host's PIL resize
+        (:325-349), so the result is predict() of the frames utils.build_X(force_dim=...) returns.
         The forward pass of a batch is one CUDA-graph replay; batch k+1 travels host -> device on a copy stream
         (from X itself when X is a pinned torch tensor, through a pinned staging pair filled by a helper thread
         otherwise) while batch k computes, and the results come back through one pinned buffer."""
         torch = _torch()
+        if resize and (X.dtype != torch.uint8 if torch.is_tensor(X) else np.asarray(X).dtype != np.uint8):
+            raise ValueError("predict(resize=True) takes uint8 frames as decoded, got %s" % (X.dtype,))
         if torch.is_tensor(X):
             Xt = X if X.dtype in (torch.uint8, torch.float32) else X.float()
         else:
@@ -345,6 +350,9 @@ class SPNetModel:
                 Xn = Xn.astype(np.float32)
             Xt = torch.from_numpy(np.ascontiguousarray(Xn))
         n = Xt.shape[0]
+        if Xt.dtype == torch.uint8 and not resize and tuple(Xt.shape[1:3]) != (self.H, self.W):
+            raise ValueError("predict: %s frames for a %dx%d model (resize=True resizes them on the device)"
+                             % ("x".join(map(str, Xt.shape[1:3])), self.H, self.W))
         out = np.empty((n, self.Y0size), np.float32)
         if n == 0:
             return out
@@ -366,11 +374,7 @@ class SPNetModel:
                     eng.x0.zero_()
                 src = Xt[j * bs:j * bs + m]
                 if src.dtype == torch.uint8:
-                    from . import ops
-                    if m == bs:
-                        ops.normalize_u8(src.contiguous().view(eng.x0.shape), eng.x0)
-                    else:
-                        eng.x0[:m].copy_(ops.normalize_u8(src.contiguous()).view((m,) + tuple(eng.x0.shape[1:])))
+                    eng.frames_to_x0(src.contiguous())
                 else:
                     eng.x0[:m].copy_(src.reshape((m,) + tuple(eng.x0.shape[1:])))
                 res[j * bs:(j + 1) * bs].copy_(eng.infer(), non_blocking=True)

@@ -4,6 +4,8 @@ PyTorch is used only as the owner of device memory and streams: every function h
 forwards raw device pointers and shapes to libspnet_b200.so on the current CUDA stream.
 Nothing in this module computes with torch ops, and nothing falls back to them.
 """
+import math
+
 import torch
 
 from ._lib import lib
@@ -474,19 +476,97 @@ _U8_LUT = {}
 def normalize_u8(x_u8, out=None):
     """(v/255 - 0.5)*2 of spnet/utils.py:340-342 on uint8 frames, bit-exact to numpy's fp32 arithmetic (the 256
     possible results are computed by numpy itself and looked up on the device)."""
-    import numpy as np
     _chk(x_u8, out)
     assert x_u8.dtype == torch.uint8
-    key = str(x_u8.device)
+    if out is None:
+        out = torch.empty(x_u8.shape, device=x_u8.device, dtype=torch.float32)
+    lib().normalize_u8(_p(x_u8), _p(_u8_lut(x_u8.device)), _p(out), x_u8.numel(), _s())
+    return out
+
+
+def _u8_lut(device):
+    """The 256 values of (v/255 - 0.5)*2 as numpy computes them in fp32, one device copy per device."""
+    import numpy as np
+    key = str(device)
     if key not in _U8_LUT:
         lut = np.arange(256, dtype=np.float32)
         lut = lut / 255.0
         lut -= 0.5
         lut *= 2.0
-        _U8_LUT[key] = torch.from_numpy(lut.astype(np.float32)).to(x_u8.device)
+        _U8_LUT[key] = torch.from_numpy(lut.astype(np.float32)).to(device)
+    return _U8_LUT[key]
+
+
+_PB_ONE = float(1 << 22)  # Pillow's PRECISION_BITS = 32 - 8 - 2
+
+
+def _lanczos(t):
+    """Pillow's lanczos_filter (libImaging/Resample.c): sinc(t) * sinc(t/3) on [-3, 3), sinc(x) = sin(pi x) / (pi x)."""
+    def sinc(x):
+        if x == 0.0:
+            return 1.0
+        x = x * math.pi
+        return math.sin(x) / x
+    return sinc(t) * sinc(t / 3.0) if -3.0 <= t < 3.0 else 0.0
+
+
+def lanczos_tables(in_size, out_size):
+    """Pillow's LANCZOS coefficients for one axis in its 8-bit fixed point (precompute_coeffs + normalize_coeffs_8bpc
+    of libImaging/Resample.c, float64 in Pillow's operation order): bounds int32 [out_size, 2] = (first input index,
+    tap count), coeffs int32 [out_size, ksize] in units of 2^-22. Host only; resize_lanczos_u8 applies them."""
+    import numpy as np
+    if in_size < 1 or out_size < 1:
+        raise ValueError("lanczos_tables: sizes must be positive, got %r -> %r" % (in_size, out_size))
+    scale = in_size / out_size
+    fs = max(scale, 1.0)
+    support = 3.0 * fs
+    ss = 1.0 / fs  # Pillow multiplies by 1/filterscale; dividing by filterscale can differ in the last bit
+    ksize = int(math.ceil(support)) * 2 + 1
+    bounds = np.zeros((out_size, 2), np.int32)
+    coeffs = np.zeros((out_size, ksize), np.int32)
+    for xx in range(out_size):
+        center = (xx + 0.5) * scale
+        xmin = max(int(center - support + 0.5), 0)
+        count = min(int(center + support + 0.5), in_size) - xmin
+        w = [_lanczos((x + xmin - center + 0.5) * ss) for x in range(count)]
+        ww = 0.0
+        for v in w:
+            ww += v
+        if ww != 0.0:
+            w = [v / ww for v in w]
+        bounds[xx] = (xmin, count)
+        coeffs[xx, :count] = [int(v * _PB_ONE + (0.5 if v >= 0 else -0.5)) for v in w]
+    return bounds, coeffs
+
+
+_LANCZOS = {}
+
+
+def resize_lanczos_u8(x_u8, OH, OW, out=None):
+    """LANCZOS resize of uint8 frames [n, H, W] (or [n, H, W, 1]) to [n, OH, OW], fused with normalize_u8's
+    (v/255 - 0.5)*2: out fp32 [n, OH, OW] (or any contiguous tensor of that many elements) = lut[resized byte]. The
+    bytes are those of PIL's Image.resize((OW, OH), Image.LANCZOS) on each frame (spnet/utils.py:325-349)."""
+    _chk(x_u8, out)
+    if x_u8.dtype != torch.uint8:
+        raise TypeError("resize_lanczos_u8 takes uint8 frames, got %s" % x_u8.dtype)
+    if x_u8.dim() == 4 and x_u8.shape[3] == 1:
+        x_u8 = x_u8.view(x_u8.shape[:3])
+    if x_u8.dim() != 3:
+        raise ValueError("resize_lanczos_u8 takes frames [n, H, W] or [n, H, W, 1], got %s" % (tuple(x_u8.shape),))
+    n, H, W = x_u8.shape
+    OH, OW = int(OH), int(OW)
     if out is None:
-        out = torch.empty(x_u8.shape, device=x_u8.device, dtype=torch.float32)
-    lib().normalize_u8(_p(x_u8), _p(_U8_LUT[key]), _p(out), x_u8.numel(), _s())
+        out = torch.empty((n, OH, OW), device=x_u8.device, dtype=torch.float32)
+    if out.dtype != torch.float32 or out.numel() != n * OH * OW:
+        raise ValueError("resize_lanczos_u8: out must be fp32 with %d elements" % (n * OH * OW))
+    key = (H, W, OH, OW, str(x_u8.device))
+    if key not in _LANCZOS:
+        xb, xc = lanczos_tables(W, OW)
+        yb, yc = lanczos_tables(H, OH)
+        _LANCZOS[key] = tuple(torch.from_numpy(a).to(x_u8.device) for a in (xb, xc, yb, yc))
+    xb, xc, yb, yc = _LANCZOS[key]
+    lib().resize_lanczos_u8(_p(x_u8), n, H, W, _p(xb), _p(xc), xc.shape[1], _p(yb), _p(yc), yc.shape[1],
+                            _p(_u8_lut(x_u8.device)), _p(out), OH, OW, _s())
     return out
 
 

@@ -201,35 +201,50 @@ def _load_one(args):
     return arr[:, :, 0:1] if grayscale else arr
 
 
-def build_X(total_load, img_file_list, force_dim=224, grayscale=False, raw_u8=False):
+def build_X(total_load, img_file_list, force_dim=224, grayscale=False, raw_u8=False, defer_resize=False):
     """Images -> X float32 NHWC in [-1,1] (spnet/utils.py:325-421): PIL decode, optional LANCZOS
     resize to a force_dim square, (v/255 - 0.5)*2, channel 0 only when grayscale.
     raw_u8 (B200 build only): return the uint8 pixel values instead; SPNetModel.predict / the engine apply the
-    same normalisation on the device, bit for bit, and a quarter of the bytes cross PCIe."""
+    same normalisation on the device, bit for bit, and a quarter of the bytes cross PCIe.
+    defer_resize (B200 build only; with raw_u8, grayscale and a force_dim): leave the LANCZOS resize to the device
+    (SPNetModel.predict(X, resize=True), the same bytes as PIL's) and return the frames at their decoded size - unless
+    one frame's size differs from the first's, in which case the whole call returns the host-resized frames."""
     print("      Reading images and assigning as input X...")
-    first = _load_one((img_file_list[0], force_dim, grayscale, raw_u8))
+    defer = defer_resize and raw_u8 and grayscale and force_dim is not None
+    dim = None if defer else force_dim
+    first = _load_one((img_file_list[0], dim, grayscale, raw_u8))
     img_dims = first.shape if not grayscale else (first.shape[0], first.shape[1], 3)
     X = np.zeros((total_load,) + first.shape, dtype=np.uint8 if raw_u8 else cf.dtype)
     nproc = os.cpu_count() or 1
+    ragged = False
     with ThreadPoolExecutor(nproc) as ex:
-        for i, arr in enumerate(ex.map(_load_one, [(f, force_dim, grayscale, raw_u8) for f in img_file_list[:total_load]])):
+        for i, arr in enumerate(ex.map(_load_one, [(f, dim, grayscale, raw_u8) for f in img_file_list[:total_load]])):
+            if defer and arr.shape != first.shape:
+                ragged = True
+                break
             X[i] = arr
+    if ragged:
+        return build_X(total_load, img_file_list, force_dim=force_dim, grayscale=grayscale, raw_u8=raw_u8)
     return X, img_dims
 
 
-def stream_X(img_file_list, chunk, force_dim=224, grayscale=False, raw_u8=False):
+def stream_X(img_file_list, chunk, force_dim=224, grayscale=False, raw_u8=False, defer_resize=False):
     """Generator over (start, X_chunk): the frames of build_X in chunks of `chunk` files, the NEXT chunk being
     decoded by the worker threads while the caller consumes the current one (SURVEY.md section 8(f) rank 1: at
     B200 inference rates PIL decode, not the network, bounds predict_spnet over tens of thousands of frames, and
-    the whole set no longer has to fit in host memory). Values are identical to build_X's."""
+    the whole set no longer has to fit in host memory). Values are identical to build_X's, chunk by chunk
+    (defer_resize: native-size frames, or the host-resized ones for a chunk whose frames differ in size)."""
     nproc = os.cpu_count() or 1
     n = len(img_file_list)
+    defer = defer_resize and raw_u8 and grayscale and force_dim is not None
 
     def decode(lo):
         files = img_file_list[lo:lo + chunk]
         with ThreadPoolExecutor(nproc) as ex:
-            return np.stack(list(ex.map(_load_one, [(f, force_dim, grayscale, raw_u8) for f in files]))).astype(
-                np.uint8 if raw_u8 else cf.dtype)
+            frames = list(ex.map(_load_one, [(f, None if defer else force_dim, grayscale, raw_u8) for f in files]))
+            if defer and any(a.shape != frames[0].shape for a in frames):
+                frames = list(ex.map(_load_one, [(f, force_dim, grayscale, raw_u8) for f in files]))
+        return np.stack(frames).astype(np.uint8 if raw_u8 else cf.dtype)
 
     with ThreadPoolExecutor(1) as bg:
         fut = bg.submit(decode, 0) if n else None
