@@ -73,6 +73,20 @@ int spnet_normalize_u8(const unsigned char* in, const float* lut, float* out, lo
  * xbounds [OW,2] / ybounds [OH,2] int32 = (first input index, tap count), xcoeffs [OW,kx] / ycoeffs [OH,ky] int32 in
  * units of 2^-22: Pillow's tables for (W -> OW) and (H -> OH) (spnet_b200/ops.py lanczos_tables). */
 int spnet_resize_lanczos_u8(const unsigned char* in, int n, int H, int W, const int* xbounds, const int* xcoeffs, int kx, const int* ybounds, const int* ycoeffs, int ky, const float* lut, float* out, int OH, int OW, cudaStream_t stream);
+/* PNG pixel data (the concatenated IDAT payload: one zlib stream of filtered scanlines) -> channel 0 of each frame,
+ * the bytes of np.asarray(Image.open(f).convert("RGB"))[:, :, 0] for bit depth 8, not interlaced, no palette.
+ * streams: the n frames' zlib streams back to back; offsets int64 [n+1] (clamped to [0, stream_bytes]); all frames
+ * H x W with bpp bytes per pixel (1, 2, 3, 4 = colour type 0, 4, 2, 6); scratch: n*H*(1 + W*bpp) bytes for the
+ * inflated scanlines; out uint8 [n, H, W]; status int32 [n] = 0 or one SPNET_PNG_ERR_* per frame (out undefined then).
+ * Stricter than zlib / Pillow: the inflated length must be exactly H*(1 + W*bpp) and the Adler-32 trailer present. */
+#define SPNET_PNG_OK 0
+#define SPNET_PNG_ERR_HEADER (-1)    /* zlib CMF/FLG header invalid, or a preset dictionary */
+#define SPNET_PNG_ERR_DATA (-2)      /* invalid block type, stored length, code set, symbol or distance */
+#define SPNET_PNG_ERR_TRUNCATED (-3) /* the stream ends inside a block */
+#define SPNET_PNG_ERR_SIZE (-4)      /* inflated length is not H*(1 + W*bpp) */
+#define SPNET_PNG_ERR_ADLER (-5)     /* Adler-32 trailer missing, wrong, or followed by more bytes */
+#define SPNET_PNG_ERR_FILTER (-6)    /* a scanline's filter type is above 4 */
+int spnet_png_decode_u8(const unsigned char* streams, long long stream_bytes, const long long* offsets, int n, int H, int W, int bpp, unsigned char* scratch, long long scratch_bytes, unsigned char* out, int* status, cudaStream_t stream);
 
 /* ---- Evaluation metrics (spnet/diagnostics.py: calc_errors :13-60; compute_iou :85-120 for every (image, slot)
  *      pair, analytic ellipse raster with an anti-aliasing margin instead of cv2). yp / yt: denormalised fp32

@@ -26,7 +26,8 @@ def predict_network(weights_file="spnet.model", datapath=default_image_dir, frac
                     batch_size=16, model=None, X_pred="", draw_images=True, stream_chunk=None, raw_u8=True, ranks=None):
     """stream_chunk (B200 build only): decode / predict the directory in chunks of that many frames, decoding chunk
     k+1 on the host threads while chunk k is on the GPU, instead of loading every frame into memory first.
-    raw_u8: frames read from `datapath` travel to the GPU as uint8 and are normalised there (same values bit for bit).
+    raw_u8: frames read from `datapath` travel to the GPU as uint8 and are normalised there (same values bit for bit);
+    grayscale PNG frames used at their decoded size are also decoded there (utils.build_X(..., device=True)).
 
     Under `torchrun --nproc-per-node N` the sorted file list is cut into N contiguous shards, rank r predicts shard r on
     GPU r (no collective on the data path) and writes hawley_spnet.csv.part<r>; rank 0 then concatenates the parts in
@@ -83,6 +84,9 @@ def predict_network(weights_file="spnet.model", datapath=default_image_dir, frac
     # same bytes as PIL's LANCZOS (a directory of mixed frame sizes is resized on the host, as the loaders fall back)
     defer = (from_dir and raw_u8 and grayscale and force_dim is not None
              and (getattr(model, "H", None), getattr(model, "W", None)) == (force_dim, force_dim))
+    # frames used at their decoded size are decoded on this process's GPU (spnet_b200.png: the bytes PIL decodes; files
+    # outside the PNG subset it takes, and frames it rejects, are decoded by PIL)
+    device = from_dir and raw_u8 and grayscale and (defer or force_dim is None)
 
     def predict(X):
         if defer:
@@ -92,11 +96,11 @@ def predict_network(weights_file="spnet.model", datapath=default_image_dir, frac
     if from_dir:
         if streaming:
             chunks = utils.stream_X(img_file_list, int(stream_chunk), force_dim=force_dim, grayscale=grayscale, raw_u8=raw_u8,
-                                    defer_resize=defer)
+                                    defer_resize=defer, device=device)
             first_lo, X_pred = next(chunks)
         else:
             X_pred, img_dims = utils.build_X(total_load, img_file_list, force_dim=force_dim, grayscale=grayscale,
-                                             raw_u8=raw_u8, defer_resize=defer)
+                                             raw_u8=raw_u8, defer_resize=defer, device=device)
         print("")
     m = len(img_file_list) if streaming else X_pred.shape[0]
     print("    Predicting... (m = ", m, " frames in dataset)", sep="")

@@ -570,6 +570,25 @@ def resize_lanczos_u8(x_u8, OH, OW, out=None):
     return out
 
 
+def png_decode_u8(streams, offsets, H, W, bpp, out, scratch=None):
+    """Channel 0 of n PNG frames of one size and colour type (csrc/png.cu): streams uint8 = the frames' zlib streams
+    (concatenated IDAT payloads) back to back, offsets int64 [n + 1], bpp bytes per pixel (1, 2, 3, 4 for colour
+    types 0, 4, 2, 6), out uint8 [n, H, W] (or [n, H, W, 1]). Returns the int32 status per frame (0, or one of the
+    header's SPNET_PNG_ERR_* codes; that frame's out bytes are then undefined). spnet_b200.png hides the container."""
+    _chk(streams, offsets, out, scratch)
+    if streams.dtype != torch.uint8 or out.dtype != torch.uint8 or offsets.dtype != torch.int64:
+        raise TypeError("png_decode_u8 takes uint8 streams and out and int64 offsets")
+    n = offsets.numel() - 1
+    if n < 1 or out.numel() != n * H * W:
+        raise ValueError("png_decode_u8: %d offsets for out %s of %dx%d frames" % (offsets.numel(), tuple(out.shape), H, W))
+    if scratch is None:
+        scratch = torch.empty(n * H * (1 + W * bpp), dtype=torch.uint8, device=out.device)
+    status = torch.empty(n, dtype=torch.int32, device=out.device)
+    lib().png_decode_u8(_p(streams), streams.numel(), _p(offsets), n, H, W, bpp, _p(scratch), scratch.numel(), _p(out),
+                        _p(status), _s())
+    return status
+
+
 def cast_f32_to_bf16(src, dst):
     lib().cast_f32_to_bf16(_p(src), _p(dst), src.numel(), _s())
 

@@ -201,15 +201,22 @@ def _load_one(args):
     return arr[:, :, 0:1] if grayscale else arr
 
 
-def build_X(total_load, img_file_list, force_dim=224, grayscale=False, raw_u8=False, defer_resize=False):
+def build_X(total_load, img_file_list, force_dim=224, grayscale=False, raw_u8=False, defer_resize=False, device=False):
     """Images -> X float32 NHWC in [-1,1] (spnet/utils.py:325-421): PIL decode, optional LANCZOS
     resize to a force_dim square, (v/255 - 0.5)*2, channel 0 only when grayscale.
     raw_u8 (B200 build only): return the uint8 pixel values instead; SPNetModel.predict / the engine apply the
     same normalisation on the device, bit for bit, and a quarter of the bytes cross PCIe.
     defer_resize (B200 build only; with raw_u8, grayscale and a force_dim): leave the LANCZOS resize to the device
     (SPNetModel.predict(X, resize=True), the same bytes as PIL's) and return the frames at their decoded size - unless
-    one frame's size differs from the first's, in which case the whole call returns the host-resized frames."""
+    one frame's size differs from the first's, in which case the whole call returns the host-resized frames.
+    device (B200 build only; with raw_u8, grayscale, and force_dim None or defer_resize): decode the PNGs on the
+    current CUDA device (spnet_b200.png, the bytes PIL decodes) and return X as a CUDA uint8 tensor; frames of
+    different sizes, or a file PIL fails on, make the call return (or raise) what it does without `device`."""
     print("      Reading images and assigning as input X...")
+    if device and raw_u8 and grayscale and (force_dim is None or defer_resize):
+        X = _device_frames(img_file_list[:total_load])
+        if X is not None:
+            return X, (X.shape[1], X.shape[2], 3)
     defer = defer_resize and raw_u8 and grayscale and force_dim is not None
     dim = None if defer else force_dim
     first = _load_one((img_file_list[0], dim, grayscale, raw_u8))
@@ -228,24 +235,48 @@ def build_X(total_load, img_file_list, force_dim=224, grayscale=False, raw_u8=Fa
     return X, img_dims
 
 
-def stream_X(img_file_list, chunk, force_dim=224, grayscale=False, raw_u8=False, defer_resize=False):
+def _device_frames(files, items=None, decoder=None):
+    """uint8 frames [n, H, W, 1] decoded on the current CUDA device (spnet_b200.png), or None when the host route
+    must run instead (frames of different sizes, or a file PIL fails on). items: png.read of each file, when the caller
+    has read them already; decoder: the png.Decoder to reuse (stream_X keeps one per generator)."""
+    import torch
+    from . import png
+    if items is None:
+        with ThreadPoolExecutor(os.cpu_count() or 1) as ex:
+            items = list(ex.map(png.read, files))
+    dev = torch.device("cuda", torch.cuda.current_device())
+    return (decoder or png.Decoder()).frames(files, items, dev)
+
+
+def stream_X(img_file_list, chunk, force_dim=224, grayscale=False, raw_u8=False, defer_resize=False, device=False):
     """Generator over (start, X_chunk): the frames of build_X in chunks of `chunk` files, the NEXT chunk being
     decoded by the worker threads while the caller consumes the current one (SURVEY.md section 8(f) rank 1: at
     B200 inference rates PIL decode, not the network, bounds predict_spnet over tens of thousands of frames, and
     the whole set no longer has to fit in host memory). Values are identical to build_X's, chunk by chunk
-    (defer_resize: native-size frames, or the host-resized ones for a chunk whose frames differ in size)."""
+    (defer_resize: native-size frames, or the host-resized ones for a chunk whose frames differ in size; device: CUDA
+    uint8 frames decoded on the device, the worker threads reading and parsing the next chunk's files while the
+    caller consumes this one, or the host route's values for a chunk whose frames differ in size)."""
     nproc = os.cpu_count() or 1
     n = len(img_file_list)
     defer = defer_resize and raw_u8 and grayscale and force_dim is not None
+    on_device = device and raw_u8 and grayscale and (force_dim is None or defer_resize)
 
-    def decode(lo):
-        files = img_file_list[lo:lo + chunk]
+    def host(files):
         with ThreadPoolExecutor(nproc) as ex:
             frames = list(ex.map(_load_one, [(f, None if defer else force_dim, grayscale, raw_u8) for f in files]))
             if defer and any(a.shape != frames[0].shape for a in frames):
                 frames = list(ex.map(_load_one, [(f, force_dim, grayscale, raw_u8) for f in files]))
         return np.stack(frames).astype(np.uint8 if raw_u8 else cf.dtype)
 
+    def decode(lo):
+        files = img_file_list[lo:lo + chunk]
+        if not on_device:
+            return host(files)
+        with ThreadPoolExecutor(nproc) as ex:
+            return list(ex.map(png.read, files))
+
+    from . import png
+    decoder = png.Decoder() if on_device else None
     with ThreadPoolExecutor(1) as bg:
         fut = bg.submit(decode, 0) if n else None
         lo = 0
@@ -253,6 +284,10 @@ def stream_X(img_file_list, chunk, force_dim=224, grayscale=False, raw_u8=False,
             X = fut.result()
             nxt = lo + chunk
             fut = bg.submit(decode, nxt) if nxt < n else None
+            if on_device:  # the copy and the launch are issued here, on the caller's thread and current stream
+                files = img_file_list[lo:lo + chunk]
+                Xd = _device_frames(files, X, decoder)
+                X = Xd if Xd is not None else host(files)
             yield lo, X
             lo = nxt
 
