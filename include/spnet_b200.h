@@ -89,11 +89,12 @@ int spnet_resize_lanczos_u8(const unsigned char* in, int n, int H, int W, const 
 int spnet_png_decode_u8(const unsigned char* streams, long long stream_bytes, const long long* offsets, int n, int H, int W, int bpp, unsigned char* scratch, long long scratch_bytes, unsigned char* out, int* status, cudaStream_t stream);
 
 /* ---- Evaluation metrics (spnet/diagnostics.py: calc_errors :13-60; compute_iou :85-120 for every (image, slot)
- *      pair, analytic ellipse raster with an anti-aliasing margin instead of cv2). yp / yt: denormalised fp32
- *      [n, ncols]; counters int32 [7] (caller zeroes), pix_err fp32 [n]; iou fp32 [n, ncols/8] (-1 = skipped pair),
- *      counts nullable int32 [n, ncols/8, 2]. ---- */
+ *      pair, through an integer port of cv2's anti-aliased filled-ellipse raster on the reference's 512 x 384 canvas).
+ *      yp / yt: denormalised fp32 [n, ncols]; counters int32 [7] (caller zeroes), pix_err fp32 [n]; counts int32
+ *      [n, ncols/8, 2] = (intersection, union) pixel counts, intersection / union = the reference's IoU bit for bit,
+ *      union = 0 where the reference returns -1 (empty true slot, or nothing drawn). ---- */
 int spnet_calc_errors(const float* yp, const float* yt, int n, int ncols, int* counters, float* pix_err, cudaStream_t stream);
-int spnet_ellipse_iou(const float* yp, const float* yt, int n, int ncols, int nx, int ny, float margin, float* iou, int* counts, cudaStream_t stream);
+int spnet_ellipse_iou(const float* yp, const float* yt, int n, int ncols, int* counts, cudaStream_t stream);
 
 /* ---- AugmentOnTheFly on the device (spnet/callbacks.py:272-341; cutout_inplace / salt_n_pepa_inplace of
  *      spnet/augmentation.py:117-135,159-180): x = augmented copy of the pristine frames x_orig, fp32 [n,H,W,C],

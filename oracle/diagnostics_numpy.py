@@ -9,14 +9,12 @@ spnet_b200/csrc/diagnostics.cu:
   shift=10) on a 512 x 384 canvas and counts non-zero pixels, i.e. every pixel the ANTI-ALIASED filled polygon
   touches. That rasteriser (third-party: OpenCV drawing.cpp) is restated in integers in oracle/cv2_raster.py and
   pinned pixel for pixel against cv2 itself; the IoUs here are therefore the reference's own, bit for bit
-  (tests/test_diagnostics.py compares with tests/golden/ref_diagnostics.npz). The earlier analytic approximation
-  (semi-axes enlarged by AA_MARGIN) is kept as ellipse_mask_analytic for the device kernel's fast mode.
+  (tests/test_diagnostics.py compares with tests/golden/ref_diagnostics.npz).
 * precision (:125-150) and calc_map (:153-162): exact restatements on top of the IoU matrix.
 """
 import numpy as np
 
 VARS = 8  # spnet/config.py:30
-AA_MARGIN = np.float32(1.35)
 THRESHES = (0.5, 0.55, 0.6, 0.65, 0.7, 0.75, 0.8, 0.85, 0.9, 0.95)  # diagnostics.py:156
 
 
@@ -61,22 +59,6 @@ def ellipse_mask(args, nx=512, ny=384):
         return np.zeros((ny, nx), bool)
     angle = np.rad2deg(np.arctan2(s2, c2) / 2.0)   # float32 arithmetic, as the reference's numpy scalars
     return cv2_raster.ellipse_mask(cx, cy, a, b, angle, nx, ny)
-
-
-def ellipse_mask_analytic(args, nx=512, ny=384):
-    """The analytic approximation (device kernel's `margin >= 0` mode): ellipse test with both semi-axes enlarged by
-    AA_MARGIN pixels standing in for cv2's anti-aliased edge (create_ellipse_image :68-80; draw_ellipse utils.py:35-53
-    passes -angle to cv2, whose angles run clockwise on the y-down canvas)."""
-    cx, cy, a, b, c2, s2, noobj = [np.float32(v) for v in args[:7]]
-    if not noobj < 0.5:
-        return np.zeros((ny, nx), bool)
-    th = -np.arctan2(s2, c2) / np.float32(2.0)
-    ct, st = np.cos(th), np.sin(th)
-    ys, xs = np.mgrid[0:ny, 0:nx].astype(np.float32)
-    dx, dy = xs - cx, ys - cy
-    u = (dx * ct + dy * st) / (a + AA_MARGIN)
-    v = (dy * ct - dx * st) / (b + AA_MARGIN)
-    return (u * u + v * v) <= np.float32(1.0)
 
 
 def ellipse_image(args, nx=512, ny=384):

@@ -5,9 +5,8 @@
 //    ellipses with cv2 on a 512 x 384 canvas per pair and counts pixels on the CPU (calc_map does that for
 //    2 x 72 x N masks x 10 thresholds). Here one CTA per pair rasterises both ellipses EXACTLY as cv2 does (integer
 //    port of its polygon / anti-aliased line / convex fill code, pixel VALUES included: ellipse_iou_exact_kernel) and
-//    counts - the IoUs are the reference's, bit for bit (margin < 0). margin >= 0 selects the earlier analytic
-//    approximation (bounding-box scan of the ellipse test, semi-axes enlarged by `margin`; within 0.04 IoU).
-//    IoU = -1 where the reference returns -1.
+//    writes the intersection and union pixel counts - intersection / union is the reference's IoU, bit for bit.
+//    union = 0 where the reference returns -1.
 #include "common.cuh"
 
 namespace {
@@ -45,74 +44,6 @@ __global__ void __launch_bounds__(256) calc_errors_kernel(const float* __restric
         if ((threadIdx.x & 31) == 0 && m) atomicAdd(counters + c, __popc(m));
     }
 }
-
-struct Ell { float cx, cy, ia, ib, ct, st; bool drawn; int x0, x1, y0, y1; };
-
-__device__ __forceinline__ Ell make_ell(const float* a, float margin, int nx, int ny) {
-    Ell e;
-    e.drawn = a[6] < 0.5f;
-    e.cx = a[0]; e.cy = a[1];
-    const float sa = a[2] + margin, sb = a[3] + margin;
-    e.ia = 1.0f / sa; e.ib = 1.0f / sb;
-    const float th = -0.5f * atan2f(a[5], a[4]);
-    e.ct = cosf(th); e.st = sinf(th);
-    const float r = fmaxf(fabsf(sa), fabsf(sb)) + 1.0f;
-    e.x0 = max(0, (int)floorf(e.cx - r)); e.x1 = min(nx - 1, (int)ceilf(e.cx + r));
-    e.y0 = max(0, (int)floorf(e.cy - r)); e.y1 = min(ny - 1, (int)ceilf(e.cy + r));
-    return e;
-}
-__device__ __forceinline__ bool inside(const Ell& e, float x, float y) {
-    const float dx = x - e.cx, dy = y - e.cy;
-    const float u = (dx * e.ct + dy * e.st) * e.ia, v = (dy * e.ct - dx * e.st) * e.ib;
-    return u * u + v * v <= 1.0f;
-}
-
-__global__ void __launch_bounds__(256) ellipse_iou_kernel(const float* __restrict__ yp, const float* __restrict__ yt,
-                                                          int ncols, int nx, int ny, float margin,
-                                                          float* __restrict__ iou, int* __restrict__ counts) {
-    const int slots = ncols / VARS;
-    const int pair = blockIdx.x, j = pair / slots, an = pair - j * slots;
-    const float* p = yp + (size_t)j * ncols + an * VARS;
-    const float* t = yt + (size_t)j * ncols + an * VARS;
-    __shared__ int red[2][8];
-    if (t[6] > 0.99f) {  // empty true slot: the reference skips the pair
-        if (threadIdx.x == 0) {
-            iou[pair] = -1.0f;
-            if (counts) { counts[2 * pair] = 0; counts[2 * pair + 1] = 0; }
-        }
-        return;
-    }
-    const Ell ep = make_ell(p, margin, nx, ny), et = make_ell(t, margin, nx, ny);
-    int x0 = nx, x1 = -1, y0 = ny, y1 = -1;
-    if (ep.drawn) { x0 = min(x0, ep.x0); x1 = max(x1, ep.x1); y0 = min(y0, ep.y0); y1 = max(y1, ep.y1); }
-    if (et.drawn) { x0 = min(x0, et.x0); x1 = max(x1, et.x1); y0 = min(y0, et.y0); y1 = max(y1, et.y1); }
-    int ni = 0, nu = 0;
-    const int bw = x1 - x0 + 1, bh = y1 - y0 + 1;
-    if (bw > 0 && bh > 0) {
-        const int npx = bw * bh;
-        for (int i = threadIdx.x; i < npx; i += blockDim.x) {
-            const int yy = i / bw, xx = i - yy * bw;
-            const float x = (float)(x0 + xx), y = (float)(y0 + yy);
-            const bool a = ep.drawn && inside(ep, x, y), b = et.drawn && inside(et, x, y);
-            ni += a && b;
-            nu += a || b;
-        }
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-        ni += __shfl_xor_sync(0xffffffffu, ni, o);
-        nu += __shfl_xor_sync(0xffffffffu, nu, o);
-    }
-    if ((threadIdx.x & 31) == 0) { red[0][threadIdx.x >> 5] = ni; red[1][threadIdx.x >> 5] = nu; }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        int si = 0, su = 0;
-        for (int w = 0; w < 8; ++w) { si += red[0][w]; su += red[1][w]; }
-        iou[pair] = su > 0 ? (float)si / (float)su : -1.0f;  // nothing drawn at all: -1 like the reference
-        if (counts) { counts[2 * pair] = si; counts[2 * pair + 1] = su; }
-    }
-}
-
 
 // =================================================================================================
 // EXACT rasterisation: the pixels cv2.ellipse(canvas, centre, axes, -angle, 0, 360, 255, thickness = -1, LINE_AA,
@@ -396,17 +327,14 @@ struct RasterSmem {
 };
 
 __global__ void __launch_bounds__(256) ellipse_iou_exact_kernel(const float* __restrict__ yp, const float* __restrict__ yt,
-                                                                int ncols, float* __restrict__ iou, int* __restrict__ counts) {
+                                                                int ncols, int* __restrict__ counts) {
     extern __shared__ __align__(16) unsigned char raster_raw[];
     RasterSmem& S = *reinterpret_cast<RasterSmem*>(raster_raw);
     const int slots = ncols / VARS;
     const int pair = blockIdx.x, jimg = pair / slots, an = pair - jimg * slots;
     const float* pe[2] = {yp + (size_t)jimg * ncols + an * VARS, yt + (size_t)jimg * ncols + an * VARS};
     if (pe[1][6] > 0.99f) {  // empty true slot: the reference skips the pair (compute_iou :98-99)
-        if (threadIdx.x == 0) {
-            iou[pair] = -1.0f;
-            if (counts) { counts[2 * pair] = 0; counts[2 * pair + 1] = 0; }
-        }
+        if (threadIdx.x == 0) { counts[2 * pair] = 0; counts[2 * pair + 1] = 0; }
         return;
     }
     const bool drawn[2] = {pe[0][6] < 0.5f, pe[1][6] < 0.5f};   // create_ellipse_image: noobj < 0.5
@@ -494,8 +422,8 @@ __global__ void __launch_bounds__(256) ellipse_iou_exact_kernel(const float* __r
     if (threadIdx.x == 0) {
         int si = 0, su = 0;
         for (int w = 0; w < 8; ++w) { si += S.red[0][w]; su += S.red[1][w]; }
-        iou[pair] = su > 0 ? (float)((double)si / (double)su) : -1.0f;  // nothing drawn at all: -1 like the reference
-        if (counts) { counts[2 * pair] = si; counts[2 * pair + 1] = su; }
+        counts[2 * pair] = si;
+        counts[2 * pair + 1] = su;  // 0 when nothing is drawn at all: the reference returns -1
     }
 }
 
@@ -513,20 +441,13 @@ int spnet_calc_errors(const float* yp, const float* yt, int n, int ncols, int* c
     return spnet_check_launch("calc_errors");
 }
 
-// iou: fp32 [n, ncols/8]; counts: nullable int32 [n, ncols/8, 2] (intersection, union pixel counts)
-int spnet_ellipse_iou(const float* yp, const float* yt, int n, int ncols, int nx, int ny, float margin, float* iou,
-                      int* counts, cudaStream_t stream) {
-    SPNET_REQUIRE(yp && yt && iou && n > 0 && ncols > 0 && ncols % VARS == 0 && nx > 0 && ny > 0, "ellipse_iou: bad args");
-    if (margin < 0.0f) {
-        // exact: the reference's own raster (cv2's anti-aliased filled polygon), pixel for pixel; 512 x 384 canvas only
-        SPNET_REQUIRE(nx == RX && ny == RY, "ellipse_iou: the exact raster is built for the reference's 512 x 384 canvas");
-        static bool configured[64] = {};
-        const int rc = spnet_smem_optin(configured, ellipse_iou_exact_kernel, sizeof(RasterSmem), "ellipse_iou");
-        if (rc) return rc;
-        ellipse_iou_exact_kernel<<<n * (ncols / VARS), 256, sizeof(RasterSmem), stream>>>(yp, yt, ncols, iou, counts);
-        return spnet_check_launch("ellipse_iou");
-    }
-    ellipse_iou_kernel<<<n * (ncols / VARS), 256, 0, stream>>>(yp, yt, ncols, nx, ny, margin, iou, counts);
+// counts: int32 [n, ncols/8, 2] = (intersection, union) pixel counts of the reference's raster on its 512 x 384 canvas
+int spnet_ellipse_iou(const float* yp, const float* yt, int n, int ncols, int* counts, cudaStream_t stream) {
+    SPNET_REQUIRE(yp && yt && counts && n > 0 && ncols > 0 && ncols % VARS == 0, "ellipse_iou: bad args");
+    static bool configured[64] = {};
+    const int rc = spnet_smem_optin(configured, ellipse_iou_exact_kernel, sizeof(RasterSmem), "ellipse_iou");
+    if (rc) return rc;
+    ellipse_iou_exact_kernel<<<n * (ncols / VARS), 256, sizeof(RasterSmem), stream>>>(yp, yt, ncols, counts);
     return spnet_check_launch("ellipse_iou");
 }
 

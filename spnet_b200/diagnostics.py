@@ -6,14 +6,10 @@ thresholds; here every (image, slot) pair's IoU comes out of one kernel launch a
 counted from that matrix. The rasteriser is an integer port of cv2's own (polygon of the ellipse, anti-aliased
 edges with their pixel values, convex fill): intersection and union are the reference's pixel counts, so IoU,
 precision and mAP are the reference's numbers bit for bit (tests/test_diagnostics.py against
-tests/golden/ref_diagnostics.npz). `fast=True` selects the earlier analytic approximation (ellipse test with a
-1.35-pixel margin; within 0.04 IoU / 0.03 mAP of the reference). calc_errors is exact."""
+tests/golden/ref_diagnostics.npz). calc_errors is exact."""
 import numpy as np
 
 from . import config as cf
-
-AA_MARGIN = 1.35
-CANVAS = (512, 384)  # create_ellipse_image(nx=512, ny=384), diagnostics.py:68
 
 
 def _dev(a):
@@ -36,16 +32,15 @@ def calc_errors(Yp, Yt):
     return c[0], c[1], c[2], c[3], c[4], c[5], c[6], pe, int(np.argmax(pe))
 
 
-def iou_matrix(Yp, Yt, fast=False):
-    """IoU of every (image, predictor slot) pair, -1 where the reference's compute_iou returns -1. The exact mode returns
-    intersection / union of the reference's pixel counts in float64."""
+def iou_matrix(Yp, Yt):
+    """IoU of every (image, predictor slot) pair: intersection / union of the reference's pixel counts in float64, and
+    -1 where the reference's compute_iou returns -1 (union = 0)."""
     from . import ops
-    if fast:
-        return ops.ellipse_iou(_dev(Yp), _dev(Yt), CANVAS[0], CANVAS[1], AA_MARGIN).cpu().numpy().astype(np.float64)
-    iou, counts = ops.ellipse_iou(_dev(Yp), _dev(Yt), CANVAS[0], CANVAS[1], -1.0, counts=True)
-    iou, counts = iou.cpu().numpy().astype(np.float64), counts.cpu().numpy().astype(np.float64)
-    live = iou >= 0
-    iou[live] = counts[..., 0][live] / counts[..., 1][live]   # num_i / num_u in double, as the reference divides
+    counts = ops.ellipse_iou(_dev(Yp), _dev(Yt)).cpu().numpy().astype(np.float64)
+    inter, union = counts[..., 0], counts[..., 1]
+    iou = np.full(union.shape, -1.0)
+    live = union > 0
+    iou[live] = inter[live] / union[live]   # num_i / num_u in double, as the reference divides
     return iou
 
 

@@ -284,14 +284,14 @@ def calc_errors(yp, yt):
     return counters, pix_err
 
 
-def ellipse_iou(yp, yt, nx=512, ny=384, margin=1.35, counts=False):
-    """-> iou fp32 [n, ncols/8] (-1 = pair skipped by the reference); counts=True also returns int32 [n, ncols/8, 2]."""
+def ellipse_iou(yp, yt):
+    """-> int32 [n, ncols/8, 2] = (intersection, union) pixel counts of the reference's raster; union = 0 marks a pair
+    the reference scores -1."""
     _chk(yp, yt)
     n, ncols = yp.shape
-    iou = torch.empty(n, ncols // 8, device=yp.device, dtype=torch.float32)
-    cnt = torch.empty(n, ncols // 8, 2, device=yp.device, dtype=torch.int32) if counts else None
-    lib().ellipse_iou(_p(yp), _p(yt), n, ncols, nx, ny, margin, _p(iou), _p(cnt), _s())
-    return (iou, cnt) if counts else iou
+    cnt = torch.empty(n, ncols // 8, 2, device=yp.device, dtype=torch.int32)
+    lib().ellipse_iou(_p(yp), _p(yt), n, ncols, _p(cnt), _s())
+    return cnt
 
 
 # ----------------------------------------------------------------------------- pooling

@@ -38,7 +38,7 @@ for i in range(N):
         P[i, s * 8:(s + 1) * 8] = Tt[i, s * 8:(s + 1) * 8] + rng.normal(0, 3, 8).astype(np.float32) * [1, 1, 1, 1, 0.02, 0.02, 0, 0.1]
 Pd, Td = torch.from_numpy(P).to(dev), torch.from_numpy(Tt).to(dev)
 for _ in range(2):
-    ops.ellipse_iou(Pd, Td, margin=-1.0, counts=True)
+    ops.ellipse_iou(Pd, Td)
 # (4) 3-channel stem passes (vectorised), uint8 normalisation, device grid assignment, fused annotation loss
 px = 64 * 192 * 256
 g3 = torch.randn(px * 3, device=dev).to(torch.bfloat16); z3 = torch.randn(px * 3, device=dev).to(torch.bfloat16)
