@@ -166,7 +166,8 @@ int spnet_bn3_bwd_dz(const void* g, const void* z, const float* a, const float* 
 /* ---- dense-convolution backbone pieces (keras.applications.InceptionResNetV2 via spnet/models.py:18,357-359):
  *      generic im2col / col2im around the GEMMs (also Xception's block1_conv2 in the fp32 and deterministic modes),
  *      'valid' max-pool, AveragePooling2D(3,1,'same'), channel-slice copies (Concatenate), the scaled residual of the
- *      Inception-ResNet blocks, bias gradient ---- */
+ *      Inception-ResNet blocks, bias gradient (acc nullable: order-independent accumulators, C entries, for the
+ *      deterministic mode; spnet_acc_to_f32 then adds them into out) ---- */
 int spnet_im2col(const void* in, void* col, int dtype, int B, int H, int W, int C, int KH, int KW, int sh, int sw, int pt, int pl, int OH, int OW, cudaStream_t stream);
 int spnet_col2im(const void* gcol, void* gin, int accumulate, int dtype, int B, int H, int W, int C, int KH, int KW, int sh, int sw, int pt, int pl, int OH, int OW, cudaStream_t stream);
 int spnet_maxpool3s2_valid_fwd(const void* z, void* out, unsigned char* argmax, int dtype, int B, int H, int W, int C, cudaStream_t stream);
@@ -175,7 +176,7 @@ int spnet_avgpool3s1(const void* in, void* out, int bwd, int accumulate, int dty
 int spnet_copy2d(const void* src, long long ld_src, void* dst, long long ld_dst, int accumulate, int dtype, long long rows, int cols, cudaStream_t stream);
 int spnet_residual_fwd(const void* x, const void* u, const float* bias, float scale, int relu, void* y, int dtype, long long rows, int C, cudaStream_t stream);
 int spnet_residual_bwd(const void* gy, const void* y, float scale, int relu, void* gx, int accumulate_gx, void* gu, int dtype, long long rows, int C, cudaStream_t stream);
-int spnet_colsum_rows(const void* g, float* out, int dtype, long long rows, int C, cudaStream_t stream);
+int spnet_colsum_rows(const void* g, float* out, long long* acc, int dtype, long long rows, int C, cudaStream_t stream);
 
 /* ---- optimiser: keras Adam (spnet/models.py:494) + L2 of add_regularization (:47-71) ---- */
 /* frozen8 (nullable): one byte per 8 parameters, non-zero = not trainable (layer.trainable = False, spnet/models.py:361-372);

@@ -131,11 +131,16 @@ __device__ __forceinline__ float warp_colsum32(float (&v)[32], int lane) {
 // added with integer atomics: exact for any fp32 partial of magnitude >= 2^-32, rounded down to the
 // quantum below that, and bit-identical for every arrival order. Entry i occupies words [2i, 2i+1] of
 // a zero-initialised int64 buffer; stat_get() reassembles the double.
-__device__ __forceinline__ void stat_add(long long* acc, long long i, double v) {
+__device__ __forceinline__ void stat_limbs(double v, long long& hi, unsigned long long& lo) {
     const double t = v * 16777216.0;  // units of 2^-24
     const double fh = floor(t);
-    const long long hi = __double2ll_rd(t);
-    const unsigned long long lo = __double2ull_rz((t - fh) * 4294967296.0);  // [0, 2^32)
+    hi = __double2ll_rd(t);
+    lo = __double2ull_rz((t - fh) * 4294967296.0);  // [0, 2^32)
+}
+__device__ __forceinline__ void stat_add(long long* acc, long long i, double v) {
+    long long hi;
+    unsigned long long lo;
+    stat_limbs(v, hi, lo);
     unsigned long long* p = reinterpret_cast<unsigned long long*>(acc) + 2 * i;
     atomicAdd(p, (unsigned long long)hi);
     if (lo) atomicAdd(p + 1, lo);

@@ -195,13 +195,43 @@ __global__ void __launch_bounds__(kT) residual_bwd_kernel(const T* __restrict__ 
 
 // out[c] += sum_r g[r, c]   (bias gradient; out is fp32 and zeroed by the caller)
 // blockIdx.y = chunk of cvb channel vectors; thread t -> vector t % cvb of row lane t / cvb
+// acc == nullptr: fp32 partial sums per thread, added into out with float atomics (order of the adds not fixed).
+// acc != nullptr: every element is split into the fixed-point limbs of the order-independent accumulators
+// (common.cuh stat_limbs), summed as integers per thread and added into acc[c] with integer atomics: the result
+// does not depend on the order of the rows or of the CTAs (spnet_acc_to_f32 then adds acc into out)
 template <typename T>
-__global__ void __launch_bounds__(kT) colsum_rows_kernel(const T* __restrict__ g, float* __restrict__ out, long long rows,
-                                                         int C, int cvb, int per) {
+__global__ void __launch_bounds__(kT) colsum_rows_kernel(const T* __restrict__ g, float* __restrict__ out,
+                                                         long long* __restrict__ acc_out, long long rows, int C, int cvb,
+                                                         int per) {
     constexpr int V = VecN<T>::N;
     const int CV = C / V;
     const int cv = blockIdx.y * cvb + threadIdx.x % cvb, rl = threadIdx.x / cvb;
     if (rl >= per || cv >= CV) return;
+    if (acc_out) {
+        long long hi[V];
+        unsigned long long lo[V];
+#pragma unroll
+        for (int i = 0; i < V; ++i) hi[i] = 0, lo[i] = 0;
+        for (long long r = (long long)blockIdx.x * per + rl; r < rows; r += (long long)gridDim.x * per) {
+            float v[V];
+            load_vec(g + r * C + cv * V, v);
+#pragma unroll
+            for (int i = 0; i < V; ++i) {
+                long long h;
+                unsigned long long l;
+                stat_limbs((double)v[i], h, l);
+                hi[i] += h;
+                lo[i] += l;
+            }
+        }
+        unsigned long long* p = reinterpret_cast<unsigned long long*>(acc_out) + 2 * (cv * V);
+#pragma unroll
+        for (int i = 0; i < V; ++i) {
+            atomicAdd(p + 2 * i, (unsigned long long)hi[i]);
+            if (lo[i]) atomicAdd(p + 2 * i + 1, lo[i]);
+        }
+        return;
+    }
     float acc[V];
     zero_vec<T>(acc);
     for (long long r = (long long)blockIdx.x * per + rl; r < rows; r += (long long)gridDim.x * per) {
@@ -313,8 +343,9 @@ int spnet_residual_bwd(const void* gy, const void* y, float scale, int relu, voi
     return spnet_check_launch("residual_bwd");
 }
 
-// out[c] += sum over rows of g[r, c]   (fp32 out, zeroed by the caller)
-int spnet_colsum_rows(const void* g, float* out, int dtype, long long rows, int C, cudaStream_t stream) {
+// out[c] += sum over rows of g[r, c]   (fp32 out, zeroed by the caller). acc (nullable): the sums go to these
+// order-independent accumulators instead (C entries, zero; spnet_acc_to_f32 adds them into out and clears them)
+int spnet_colsum_rows(const void* g, float* out, long long* acc, int dtype, long long rows, int C, cudaStream_t stream) {
     int rc = chk("colsum_rows", dtype, C);
     if (rc) return rc;
     const int CV = C / (dtype == SPNET_BF16 ? 8 : 4);
@@ -326,7 +357,7 @@ int spnet_colsum_rows(const void* g, float* out, int dtype, long long rows, int 
     if (gx > 64) gx = 64;                                                    // end serialise per address (64-deep at most)
     if (gx < 1) gx = 1;
     SPNET_DISPATCH_DTYPE(dtype, (colsum_rows_kernel<T><<<dim3((unsigned)gx, chunks), kT, 0, stream>>>(
-                                    reinterpret_cast<const T*>(g), out, rows, C, cvb, per)));
+                                    reinterpret_cast<const T*>(g), out, acc, rows, C, cvb, per)));
     return spnet_check_launch("colsum_rows");
 }
 

@@ -1074,8 +1074,10 @@ class InceptionResNetV2SPNetEngine(SPNetEngineBase):
     # ---- helpers
     def _implicit(self, op):
         """k x k stride-1 convolutions of the bf16 engine run as implicit GEMM (csrc/gemm_tc.cu CONV modes): no
-        im2col / col2im buffers. fp32 and the few stride-2 convolutions keep the im2col + GEMM route."""
-        return self.lowp and op["stride"] == 1 and (op["kh"] > 1 or op["kw"] > 1) and op["cin"] != 3
+        im2col / col2im buffers. fp32, the few stride-2 convolutions and the deterministic mode (the implicit weight
+        gradient reduce-adds fp32 partials from many CTAs) keep the im2col + GEMM route."""
+        return (self.lowp and not self.deterministic and op["stride"] == 1 and (op["kh"] > 1 or op["kw"] > 1)
+                and op["cin"] != 3)
 
     def _conv_operand(self, op, x):
         """GEMM A operand [M, K] of a convolution: the activation itself for 1x1, an im2col buffer otherwise."""
@@ -1176,7 +1178,8 @@ class InceptionResNetV2SPNetEngine(SPNetEngineBase):
                 self._pw_bwd(xs[0].view(M, K), wl[op["name"] + "/kernel"].view(K, o.c), g_[op["name"] + "/kernel"].view(K, o.c),
                              gy.view(M, o.c), tgt.view(M, K), M, K, o.c)
                 self._merge(ins[0], op["first"][0])
-                ops.colsum_rows(gy.view(M, o.c), g_[op["name"] + "/bias"])
+                assert self._gacc is None or o.c <= self._gacc.numel() // 2
+                ops.colsum_rows(gy.view(M, o.c), g_[op["name"] + "/bias"], acc=self._gacc)
             elif kind == "maxpool":
                 tgt = self._into(ins[0], op["first"][0])
                 ops.maxpool3s2_valid_bwd(gy, op["argmax"], tgt)

@@ -655,7 +655,13 @@ def residual_bwd(gy, y, scale, relu, gx, accumulate_gx, gu):
                        y.numel() // C, C, _s())
 
 
-def colsum_rows(g, out):
-    _chk(g, out)
+def colsum_rows(g, out, acc=None):
+    """out[C] += column sums of g [rows, C]. acc: accumulator scratch (stats_alloc, >= C entries, all zero): the sums
+    then go through the order-independent accumulators (bit-identical whatever the order of the rows) and are added
+    into out afterwards."""
+    _chk(g, out, acc)
     C = g.shape[-1]
-    lib().colsum_rows(_p(g), _p(out), dtype_code(g), g.numel() // C, C, _s())
+    lib().colsum_rows(_p(g), _p(out), _p(acc), dtype_code(g), g.numel() // C, C, _s())
+    if acc is not None:
+        lib().acc_to_f32(_p(acc), _p(out), C, 1, 1, _s())
+    return out
